@@ -3,6 +3,7 @@
 supervised + unsupervised ELBO step).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+                    [--dump-outputs DIR]
 
 One "step" = one supervised train_step + one unsupervised train_step (forward, backward, gradient
 all-reduce, Adam), each on `--batch` images per GPU (default: BASELINE.json configs[1], fixed-inferred
@@ -61,7 +62,14 @@ def parse():
                                                           "(fused_chain, wgrad_streams, post_chain_stream)")
     ap.add_argument("--e2e-input", default="uint8", choices=["uint8", "fp32"],
                     help="host image dtype of the headline e2e run (the other one is reported as e2e_alt)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (sup/unsup loss and c) and the parameters after it "
+                         "as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.ref_batch is None:
         args.ref_batch = args.batch
     return args
@@ -203,6 +211,17 @@ def dp_equivalence_check(G, cfg, dev, rank, world, exchange, b_local=8, K=10):
     return out
 
 
+def dump_outputs(path, lrn, last):
+    """The last timed step's results as float32 .npy files: what its train_steps returned (loss_sup, c_sup, loss_unsup,
+    c_unsup) and the parameters it left (params, the flat store of the model, ~4 MB)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"params": lrn.store.flat}
+    for kind, (loss, c) in last.items():
+        arrays["loss_" + kind], arrays["c_" + kind] = loss, c
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------------
@@ -245,12 +264,14 @@ def run_ours(args, rank, world, local_rank):
     dev_x = [(t if precision == "bf16" else f).to(dev) for t, f in zip(host_u8, host_x)]
     dev_y = [t.to(dev) for t in host_y]
 
+    last = {}   # (loss, c) of the latest supervised / unsupervised train_step, for --dump-outputs
+
     def step_resident(i):
         j = i % NBUF
         # (the resident ring was written once, before the warm-up: nothing that produces these tensors is pending)
-        out = lrn.train_step(dev_x[j], dev_y[j], True, inputs_ready=True)
+        out = last["sup"] = lrn.train_step(dev_x[j], dev_y[j], True, inputs_ready=True)
         for u in range(U):
-            out = lrn.train_step(dev_x[(j + 1 + u) % NBUF], None, False, inputs_ready=True)
+            out = last["unsup"] = lrn.train_step(dev_x[(j + 1 + u) % NBUF], None, False, inputs_ready=True)
         return out
 
     def barrier():
@@ -282,6 +303,9 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     ms_total, launches = timed(step_resident, args.steps, max(3, args.warmup))
+    if args.dump_outputs and rank == 0:
+        # now: the returned tensors are ring slots that later steps overwrite, and the e2e runs below train on
+        dump_outputs(args.dump_outputs, lrn, last)
     ms_step = ms_total / args.steps
     value = imgs_per_step * world / (ms_step / 1e3)
 
