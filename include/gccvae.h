@@ -166,6 +166,16 @@ int gccvae_convt_recon_bf16(int batch, const void* g4, const void* Wp8, const fl
                             const float* coef, float* log_pxz, void* D2, float* xhat, float* db, int log_pxz_ready,
                             void* stream);
 int gccvae_fill_f32(float* p, long long n, float v, void* stream);
+/* Image of the decoder (no counterpart in the reference: the generation path of gated_ccvae.py's Learner.generate /
+ * reconstruct / intervene): conv5t forward (Conv2DTranspose 32 -> 3, k4, s2, same, networks.py:49,58) + sigmoid, with
+ * nothing else - no likelihood, no gradient.
+ *   g4: [B,32,32,32] bf16, the decoder's conv4t output (after ReLU); Wp8: pack kind 8 ([16][4][32] bf16); bias: [3].
+ *   out: [B,64,64,3] NHWC, contiguous, 16-byte aligned;
+ *        out_u8 = 0: fp32 sigmoid values xhat;
+ *        out_u8 = 1: uint8 u = min(255, rint(255.0f * xhat)) (fp32 product, round half to even).
+ *   The uint8 output is the fp32 output of the same call converted by that rule, bit for bit. */
+int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp8, const float* bias, void* out, int out_u8,
+                            void* stream);
 /* S -> L "halo" kernel for 16x16 / 32x32 S planes with 32 or 64 channels and C_L <= 64: all four output-parity
  * phases per CTA from three column-shifted halo boxes (3.6x less L2 traffic than gccvae_sl_bf16), one MMA per
  * shifted view with N = 4*C_L.  Weights packed "sl9" = [9 views][4 phases][C_L padded to 16][C_S]
@@ -261,6 +271,45 @@ typedef struct {
 } gccvae_latent_bwd_args;
 int gccvae_latent_bwd_partials(int batch);
 int gccvae_latent_bwd(const gccvae_latent_bwd_args* a, void* stream);
+
+/* ---- latent code of the generation path (no counterpart in the reference) ------------------------------------
+ * One warp per image writes the z the decoder turns into an image, in one of three modes.  Notation: c is the gate
+ * sample of gate_ws (gccvae_gate_fwd); loc_p(y,c), scale_p(y,c) are the conditional prior of networks.py:118-127
+ * (scale after softplus and the [1e-3, 1e3] clip); eps [B,45] is N(0,1) with the layout of gccvae_latent_fwd
+ * (columns 0..26 style dims, 27..44 classify dims).  Labels are nonzero -> 1.
+ *   GCCVAE_GEN_GENERATE:     z_s = eps_s, z_c = loc_p(y_tgt,c) + scale_p(y_tgt,c) eps_c;
+ *                            sample = 0: z_s = 0, z_c = loc_p(y_tgt,c).
+ *   GCCVAE_GEN_RECONSTRUCT:  z = loc (posterior mean: relu / clipped softplus of the heads, networks.py:17-18,33-34);
+ *                            sample = 1: z = loc + scale eps.
+ *   GCCVAE_GEN_INTERVENE:    z as for RECONSTRUCT, then the classify dims move from y_src to y_tgt by the Gaussian
+ *                            counterfactual  e = (z_c - loc_p(y_src,c)) / scale_p(y_src,c),
+ *                            z_c' = z_c + (loc_p(y_tgt,c) - loc_p(y_src,c)) + (scale_p(y_tgt,c) - scale_p(y_src,c)) e
+ *                            (y_src == y_tgt leaves z_c bit-identical); z_s is never touched.  y_src = NULL: the
+ *                            classifier's decision on z_c, sigmoid(logit) > 0.5 (as gccvae_accuracy_f32 decides).
+ * Only RECONSTRUCT and INTERVENE read loc_pre / scale_pre; only GENERATE and INTERVENE read y_tgt; eps is read only when
+ * sampling (eps = NULL: the Philox stream of gccvae_latent_fwd, which gccvae_draw_noise_f32 kind 0 reproduces). */
+#define GCCVAE_GEN_GENERATE 1
+#define GCCVAE_GEN_RECONSTRUCT 2
+#define GCCVAE_GEN_INTERVENE 3
+typedef struct {
+  int batch;
+  int mode;                /* GCCVAE_GEN_* */
+  int sample;              /* 0: means, 1: draw with eps (see above) */
+  int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
+  const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu (RECONSTRUCT, INTERVENE) */
+  const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip */
+  const long long* y_tgt;  /* [B,18] int64 target labels (GENERATE, INTERVENE) */
+  const long long* y_src;  /* [B,18] int64 source labels (INTERVENE) or NULL */
+  const float* eps;        /* [B,45] N(0,1) or NULL -> Philox */
+  uint64_t seed, offset;   /* Philox key / counter base */
+  const int* step_dev;     /* optional device int added to `offset` */
+  const float* gate_ws;    /* from gccvae_gate_fwd */
+  /* outputs */
+  float* z;                /* [B,45] fp32 */
+  void* z16;               /* optional bf16 [B,64] copy of z, columns 45..63 zero (operand of the tensor-core fc1) */
+  int* y_src_out;          /* optional [B,18] int32: the y_src used (INTERVENE) */
+} gccvae_gen_latent_args;
+int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
 
 /* reduce the partials; chain through c to mu (clip / pow / ratio of gated_ccvae.py:103-109) and
  * add the L1 term gating_reg*mean|mu| (gated_ccvae.py:229-230,297-298) scaled by l1_scale

@@ -34,6 +34,19 @@ class LatentFwdArgs(C.Structure):
     ]
 
 
+GEN_GENERATE, GEN_RECONSTRUCT, GEN_INTERVENE = 1, 2, 3
+
+
+class GenLatentArgs(C.Structure):
+    """gccvae_gen_latent_args (include/gccvae.h)."""
+    _fields_ = [
+        ("batch", C.c_int), ("mode", C.c_int), ("sample", C.c_int), ("ld_pre", C.c_int),
+        ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y_tgt", C.c_void_p), ("y_src", C.c_void_p),
+        ("eps", C.c_void_p), ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p),
+        ("gate_ws", C.c_void_p), ("z", C.c_void_p), ("z16", C.c_void_p), ("y_src_out", C.c_void_p),
+    ]
+
+
 class LatentBwdArgs(C.Structure):
     _fields_ = [
         ("batch", C.c_int), ("batch_global", C.c_int), ("supervised", C.c_int), ("K", C.c_int),
@@ -143,10 +156,12 @@ SIGNATURES = {
     "gccvae_wg_s2d_bf16": (_I, [_I, _I, _I, _I, _P, _P, _I, _P, _P]),
     "gccvae_tap4_wg_bf16": (_I, [_I, _P, _P, _I, _P, _P, _P]),
     "gccvae_convt_recon_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _I, _P]),
+    "gccvae_convt_image_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P]),
     "gccvae_fill_f32": (_I, [_P, _LL, _F, _P]),
     "gccvae_gate_fwd": (_I, [_P, _P, _P, _P, _U64, _U64, _P, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gccvae_latent_fwd": (_I, [C.POINTER(LatentFwdArgs), _P]),
     "gccvae_latent_bwd_partials": (_I, [_I]),
+    "gccvae_gen_latent": (_I, [C.POINTER(GenLatentArgs), _P]),
     "gccvae_latent_bwd": (_I, [C.POINTER(LatentBwdArgs), _P]),
     "gccvae_chain_rows": (_I, [_I]),
     "gccvae_chain_partials": (_I, [_I]),

@@ -1801,6 +1801,158 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
   }
 }
 
+// conv5t forward + sigmoid into the image [B,64,64,3] (fp32, or uint8 when U8) - the generation path's last layer.
+// TMA box, taps as descriptor row offsets, barriers, phases and MMA issue are those of convt_recon_kernel with an fp32
+// image operand (XM = 0); only the epilogue differs: it stores the sigmoid of every in-image pixel and nothing else.
+struct alignas(64) CtiParams {
+  CUtensorMap tmA, tmB;
+  const float* bias;   // [3]
+  void* out;           // [B,64,64,3] fp32 or uint8
+  int batch, total_tiles, stages;
+};
+
+template <bool U8>
+__global__ void __launch_bounds__(TG_THREADS, 4) convt_image_kernel(const __grid_constant__ CtiParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
+  constexpr int B_TAP = 1024;
+  constexpr int STAGE = CTR_A_STAGE;
+  uint8_t* sB = smem;                 // 4 taps x [16 rows x 64 B]
+  uint8_t* sA = smem + 4 * B_TAP;
+  uint64_t* full = reinterpret_cast<uint64_t*>(sA + p.stages * STAGE);
+  uint64_t* empty = full + p.stages;
+  uint64_t* tfull = empty + p.stages;
+  uint64_t* tempty = tfull + 2;
+  uint64_t* bfull = tempty + 2;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  pdl_launch_dependents();
+  const int per_cta = (p.total_tiles + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int tile_beg = blockIdx.x * per_cta;
+  const int tile_end = min(tile_beg + per_cta, p.total_tiles);
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&p.tmA);
+    tma_prefetch_desc(&p.tmB);
+    for (int s = 0; s < p.stages; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], 1);
+    }
+    for (int s = 0; s < 2; ++s) {
+      mbar_init(&tfull[s], 1);
+      mbar_init(&tempty[s], 4);
+    }
+    mbar_init(bfull, 1);
+    fence_mbar_init();
+  }
+  if (warp == 2) tmem_alloc(tmem_slot, 64);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  pdl_wait();
+
+  if (warp == 0) {
+    if (elect_one() && tile_beg < tile_end) {
+      mbar_expect_tx(bfull, 4 * B_TAP);
+      for (int t = 0; t < 4; ++t) tma_load_2d(sB + t * B_TAP, &p.tmB, bfull, t * 32, 0);
+      int stage = 0;
+      uint32_t ph = 0;
+      int n = tile_beg / 9, k = tile_beg - n * 9;
+      for (int tile = tile_beg; tile < tile_end; ++tile) {
+        const int i_first = (k * 128) / 33;
+        mbar_wait_relaxed(&empty[stage], ph ^ 1);
+        mbar_expect_tx(&full[stage], CTR_BOX_ROWS * 64);
+        tma_load_4d(sA + stage * STAGE, &p.tmA, &full[stage], 0, -1, i_first - 1, n);
+        if (++stage == p.stages) { stage = 0; ph ^= 1; }
+        if (++k == 9) { k = 0; ++n; }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0 && tile_beg < tile_end) {
+      const uint32_t idesc = instr_desc_bf16(128, 16, 0, 0);
+      const uint64_t dproto = smem_desc(0, 16, 8u * 64u, SW_64);
+      const uint64_t adesc0 = dproto + (uint64_t)(smem_u32(sA) >> 4), bdesc0 = dproto + (uint64_t)(smem_u32(sB) >> 4);
+      int stage = 0;
+      uint32_t ph = 0;
+      int k = tile_beg % 9;
+      mbar_wait(bfull, 0);
+      for (int tile = tile_beg; tile < tile_end; ++tile) {
+        const int li = tile - tile_beg, as = li & 1;
+        const int f0 = k * 128, d0 = f0 - (f0 / 33) * 33;
+        mbar_wait(&tempty[as], ((uint32_t)(li >> 1) & 1u) ^ 1u);
+        mbar_wait(&full[stage], ph);
+        tc_fence_after();
+        const uint64_t a_st = adesc0 + (uint64_t)((uint32_t)stage * (STAGE >> 4) + (uint32_t)(d0 + 34) * 4u);
+        const uint32_t tacc = tmem_base + (uint32_t)as * 32u;
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const uint32_t row_off = (uint32_t)(33 * (t >> 1) + (t & 1)) * 4u;   // tap (a, b) = (t >> 1, t & 1)
+#pragma unroll
+          for (int kk = 0; kk < 2; ++kk)
+            umma_bf16(tacc, a_st - (uint64_t)row_off + (uint64_t)(2 * kk), bdesc0 + (uint64_t)(t * (B_TAP >> 4) + 2 * kk),
+                      idesc, (t > 0 || kk > 0) ? 1u : 0u);
+        }
+        umma_commit(&empty[stage]);
+        umma_commit(&tfull[as]);
+        if (++stage == p.stages) { stage = 0; ph ^= 1; }
+        if (++k == 9) k = 0;
+      }
+    }
+  } else {
+    const int q = warp & 3;
+    const int m = q * 32 + lane;
+    constexpr float LOG2E = 1.4426950408889634f;
+    const float nb0 = -LOG2E * __ldg(p.bias), nb1 = -LOG2E * __ldg(p.bias + 1), nb2 = -LOG2E * __ldg(p.bias + 2);
+    int n = tile_beg / 9, k = tile_beg - n * 9;
+    for (int tile = tile_beg; tile < tile_end; ++tile) {
+      const int li = tile - tile_beg, as = li & 1;
+      const int f = k * 128 + m, i = f / 33, j = f - i * 33;
+      const bool row_ok = f < 33 * 33;
+      const int n_cur = n;
+      if (++k == 9) { k = 0; ++n; }
+      mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
+      tc_fence_after();
+      uint32_t acc[16];
+      tmem_ld16(tmem_base + (uint32_t)as * 32u + ((uint32_t)(q * 32) << 16), acc);
+      tmem_ld_wait();
+      tc_fence_before();
+      if (lane == 0) mbar_arrive(&tempty[as]);
+      // the sigmoid of convt_recon_kernel: xhat = 1 / (1 + 2^(-(a + b) log2 e))
+      float xh[12];
+#pragma unroll
+      for (int k2 = 0; k2 < 12; ++k2) {
+        const int qq = k2 / 3, c = k2 % 3;
+        const float t = fmaf(__uint_as_float(acc[4 * qq + c]), -LOG2E, c == 0 ? nb0 : (c == 1 ? nb1 : nb2));
+        xh[k2] = rcp_approx(1.0f + ex2_approx(t));
+      }
+      // pixel (dy, dx) of block (i, j) lies in the image unless the block touches that border
+      const bool oky[2] = {row_ok && i > 0, row_ok && i < 32}, okx[2] = {j > 0, j < 32};
+#pragma unroll
+      for (int qq = 0; qq < 4; ++qq) {
+        if (!(oky[qq >> 1] && okx[qq & 1])) continue;
+        const int Yp = 2 * i - 1 + (qq >> 1), Xp = 2 * j - 1 + (qq & 1);
+        const size_t o = (((size_t)n_cur * 64 + Yp) * 64 + Xp) * 3;
+        if constexpr (U8) {
+          uint8_t* dst = static_cast<uint8_t*>(p.out) + o;
+#pragma unroll
+          for (int c = 0; c < 3; ++c) dst[c] = (uint8_t)min(255u, __float2uint_rn(__fmul_rn(255.0f, xh[3 * qq + c])));
+        } else {
+          float* dst = static_cast<float*>(p.out) + o;
+          dst[0] = xh[3 * qq]; dst[1] = xh[3 * qq + 1]; dst[2] = xh[3 * qq + 2];
+        }
+      }
+    }
+    tc_fence_before();
+  }
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 64);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // L -> S convolution of a 3-channel image in x2 block form (conv1 forward, conv5t dgrad) with the im2col tile
 // built by four producer warps instead of TMA: TMA moves one box row per ~1.3 cycles whatever its width, so
@@ -2885,6 +3037,53 @@ extern "C" int gccvae_convt_recon_bf16(int batch, const void* g4, const void* Wp
   else if (x_u8) GCC_CUDA(launch_pdl(convt_recon_kernel<1>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
   else GCC_CUDA(launch_pdl(convt_recon_kernel<0>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
   GCC_CHECK_LAUNCH("convt_recon");
+  return GCCVAE_OK;
+}
+
+// conv5t forward + sigmoid into the image (generation path): g4 [B,32,32,32] bf16, Wp8 = pack kind 8, bias [3],
+// out [B,64,64,3] fp32 (out_u8 = 0) or uint8 min(255, rint(255 xhat)) (out_u8 = 1).
+extern "C" int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp8, const float* bias, void* out,
+                                       int out_u8, void* stream) {
+  GCC_REQUIRE(g4 && Wp8 && bias && out, "convt_image: null pointer");
+  GCC_REQUIRE(batch > 0 && batch <= (1 << 26), "convt_image: bad batch %d", batch);
+  GCC_REQUIRE(out_u8 == 0 || out_u8 == 1, "convt_image: out_u8 = %d (0 fp32, 1 uint8)", out_u8);
+  GCC_REQUIRE((uintptr_t)out % 16 == 0 && (uintptr_t)g4 % 16 == 0, "convt_image: out and g4 must be 16-byte aligned");
+  CtiParams p;
+  memset(&p, 0, sizeof(p));
+  EncodeTiledFn enc = get_encode();
+  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
+  {   // the A box of convt_recon: 6 image rows x (zero column + 32 pixels)
+    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)batch};
+    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
+    cuuint32_t box[4] = {32, 33, 6, 1};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    GCC_REQUIRE(r == CUDA_SUCCESS, "convt_image: cuTensorMapEncodeTiled failed: %d", (int)r);
+  }
+  int rc;
+  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
+  p.bias = bias; p.out = out; p.batch = batch; p.total_tiles = batch * 9;
+  // the launch shape of convt_recon's default: 4 CTAs per SM, 3 stages of the A box
+  const int per_sm = 4;
+  p.stages = 3;
+  const size_t smem = 4096 + (size_t)p.stages * CTR_A_STAGE + 1024 + 2048;
+  static bool attr_set = false;
+  if (!attr_set) {
+    GCC_CUDA(cudaFuncSetAttribute(convt_image_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GCC_CUDA(cudaFuncSetAttribute(convt_image_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_set = true;
+  }
+  int ctas = p.total_tiles < 148 * per_sm ? p.total_tiles : 148 * per_sm;
+  {
+    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
+    ctas = (p.total_tiles + per_cta - 1) / per_cta;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (out_u8) GCC_CUDA(launch_pdl(convt_image_kernel<true>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  else GCC_CUDA(launch_pdl(convt_image_kernel<false>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  GCC_CHECK_LAUNCH("convt_image");
   return GCCVAE_OK;
 }
 

@@ -691,6 +691,91 @@ __global__ void __launch_bounds__(256) accuracy_kernel(const float* __restrict__
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// latent code of the generation path (gccvae_gen_latent, include/gccvae.h): one warp per image, as latent_fwd
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_latent_args a) {
+  pdl_prologue();
+  __shared__ __align__(16) GateSmem g;
+  __shared__ float s_zc[WARPS][ZC];
+  load_gate_smem(g, a.gate_ws);
+  __syncthreads();
+  if (a.step_dev) a.offset += (uint64_t)(*a.step_dev);
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int ldp = a.ld_pre > 0 ? a.ld_pre : Z;
+  const bool from_image = a.mode != GCCVAE_GEN_GENERATE;
+  float* zcs = s_zc[wid];
+
+  for (int b = blockIdx.x * WARPS + wid; b < a.batch; b += gridDim.x * WARPS) {
+    // --- posterior (Reconstruct / Intervene) or N(0,1) style dims (Generate) ------------------------------------
+    float zv[2] = {0.0f, 0.0f};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int d = lane + 32 * h;
+      if (d >= Z) continue;
+      float z = 0.0f;
+      if (from_image) {
+        float loc, sc;
+        head_act(a.loc_pre[(size_t)b * ldp + d], a.scale_pre[(size_t)b * ldp + d], loc, sc);
+        z = a.sample ? fmaf(sc, draw_eps(a.eps, a.seed, a.offset, b, d), loc) : loc;
+      } else if (d < ZS && a.sample) {
+        z = draw_eps(a.eps, a.seed, a.offset, b, d);
+      }
+      zv[h] = z;
+      if (d >= ZS) zcs[d - ZS] = z;
+    }
+    __syncwarp();
+    // --- labels: target, and (Intervene) source = given or the classifier's decision on z_c -------------------------
+    bool yt = false, ys = false;
+    if (lane < Y) {
+      if (a.mode != GCCVAE_GEN_RECONSTRUCT) yt = a.y_tgt[(size_t)b * Y + lane] != 0;
+      if (a.mode == GCCVAE_GEN_INTERVENE) {
+        if (a.y_src != nullptr) {
+          ys = a.y_src[(size_t)b * Y + lane] != 0;
+        } else {
+          float acc = g.b[lane];
+#pragma unroll
+          for (int i = 0; i < ZC; ++i) acc = fmaf(zcs[i], g.M[i * Y + lane], acc);
+          ys = sigmoid_f(acc) > 0.5f;
+        }
+        if (a.y_src_out != nullptr) a.y_src_out[(size_t)b * Y + lane] = ys ? 1 : 0;
+      }
+    }
+    const uint32_t tmask = __ballot_sync(0xffffffffu, yt), smask = __ballot_sync(0xffffffffu, ys);
+    // --- classify dims through the conditional prior (lane i < ZC: classify dim i) -------------------------------------
+    if (lane < ZC && a.mode != GCCVAE_GEN_RECONSTRUCT) {
+      float mt, st;
+      prior_i(g, tmask, lane, mt, st);
+      const float spt = clip_f(softplus_f(st), 1e-3f, 1e3f);
+      float zc;
+      if (a.mode == GCCVAE_GEN_GENERATE) {
+        zc = a.sample ? fmaf(spt, draw_eps(a.eps, a.seed, a.offset, b, ZS + lane), mt) : mt;
+      } else {
+        float ms, ss;
+        prior_i(g, smask, lane, ms, ss);
+        const float sps = clip_f(softplus_f(ss), 1e-3f, 1e3f);
+        const float z0 = zcs[lane];
+        const float e = (z0 - ms) / sps;
+        zc = fmaf(spt - sps, e, z0 + (mt - ms));   // incremental form: an unchanged prior leaves z_c bit-identical
+      }
+      zcs[lane] = zc;
+    }
+    __syncwarp();
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int d = lane + 32 * h;
+      if (d < Z) {
+        const float z = d >= ZS ? zcs[d - ZS] : zv[h];
+        a.z[(size_t)b * Z + d] = z;
+        if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)b * 64 + d] = __float2bfloat16(z);
+      } else if (d < 64 && a.z16 != nullptr) {
+        reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)b * 64 + d] = __float2bfloat16(0.0f);
+      }
+    }
+    __syncwarp();
+  }
+}
+
 }  // namespace gccvae
 
 using namespace gccvae;
@@ -755,6 +840,24 @@ extern "C" int gccvae_latent_fwd(const gccvae_latent_fwd_args* a, void* stream) 
   else
     GCC_CUDA(launch_pdl_k(latent_fwd_kernel<false>, dim3(grid), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   GCC_CHECK_LAUNCH("latent_fwd");
+  return GCCVAE_OK;
+}
+
+extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) {
+  GCC_REQUIRE(a, "gen_latent: null args");
+  GCC_REQUIRE(a->batch > 0, "gen_latent: bad batch %d", a->batch);
+  GCC_REQUIRE(a->mode >= GCCVAE_GEN_GENERATE && a->mode <= GCCVAE_GEN_INTERVENE,
+              "gen_latent: mode %d (1 generate, 2 reconstruct, 3 intervene)", a->mode);
+  GCC_REQUIRE(a->gate_ws && a->z, "gen_latent: null pointer");
+  GCC_REQUIRE(a->mode == GCCVAE_GEN_GENERATE || (a->loc_pre && a->scale_pre && a->ld_pre >= 0),
+              "gen_latent: reconstruct / intervene need loc_pre and scale_pre");
+  GCC_REQUIRE(a->mode == GCCVAE_GEN_RECONSTRUCT || a->y_tgt, "gen_latent: generate / intervene need y_tgt");
+  GCC_REQUIRE((uintptr_t)a->z % 4 == 0 && (uintptr_t)a->eps % 4 == 0 && (uintptr_t)a->loc_pre % 4 == 0 &&
+                  (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y_tgt % 8 == 0 && (uintptr_t)a->y_src % 8 == 0 &&
+                  (uintptr_t)a->y_src_out % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
+              "gen_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
+  GCC_CUDA(launch_pdl_k(gen_latent_kernel, dim3(latent_grid(a->batch)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+  GCC_CHECK_LAUNCH("gen_latent");
   return GCCVAE_OK;
 }
 

@@ -48,6 +48,12 @@ def out_shape(layer):
     return layer[3] if layer[1] == "LS" else layer[2]
 
 
+def image_u8(xhat):
+    """fp32 image in [0,1] -> uint8 min(255, rint(255 x)): fp32 product, round half to even (the rule of
+    gccvae_convt_image_bf16)."""
+    return torch.clamp(torch.round(xhat * 255.0), max=255.0).to(torch.uint8)
+
+
 def _stream():
     return torch.cuda.current_stream().cuda_stream
 
@@ -127,6 +133,9 @@ class Engine:
     def zero_grads(self):
         """the fp32 kernels overwrite every gradient; nothing to clear."""
 
+    def pack_weights(self, part=None):
+        """the fp32 kernels read the fp32 master weights; nothing to pack."""
+
     def recon(self, x, b, coef, log_pxz, backward):
         """utils.py:101-105 (+ gradient w.r.t. the decoder's pre-sigmoid logits when backward)."""
         B = x.shape[0]
@@ -154,6 +163,12 @@ class Engine:
             self.layer_fwd(lay, B, h, b[lay[0] + ".out"])
             h = b[lay[0] + ".out"]
         return h
+
+    def image_fwd(self, z, b, batch, out_u8):
+        """generation path: the decoder from the latent code z [B,45] -> a fresh [B,64,64,3] image, the fp32 sigmoid
+        values or (out_u8) uint8 min(255, rint(255 xhat)) with the product and the rounding in fp32."""
+        xhat = self.decoder_fwd(z, b)
+        return image_u8(xhat) if out_u8 else xhat.clone()
 
     def decoder_bwd(self, z, b, want_dz=True):
         """expects b['dec.conv5t.dout'] = dLoss/d(pre-sigmoid logits); returns dz."""

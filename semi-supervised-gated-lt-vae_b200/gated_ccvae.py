@@ -7,15 +7,19 @@ sm_100a kernels.  Same class names, constructor arguments, method names and retu
     lqx     = learner.classifier_loss(x, y, c, k=100)   # :167-182
     loss, c = learner.train_step(x, y, supervised)      # :302-311  (fwd + bwd + Adam)
     acc     = learner.classifier_accuracy(x, y)         # :421-446
+    img     = learner.generate(y) / .reconstruct(x) / .intervene(x, y_new)   # extension, see below
 
-Extensions the reference lacks (needed for parity testing and for data parallelism):
+Extensions the reference lacks (for parity testing, data parallelism and image generation):
   * every stochastic call takes an optional `noise=` dict of explicit draws
     (eps [B,45], eps_k [K,B,45], U_y [B,18], U1/U2 [18,18]); without it noise comes from an
     in-kernel Philox4x32-10 keyed by (seed, step counter);
   * `Learner.last` exposes every per-image term of the last loss call;
   * if torch.distributed is initialised the step is data parallel: the batch given to each rank is
     its shard, gradients are all-reduced (sum) over the flat gradient buffer, the loss is the global
-    mean, and the gate sample c is identical on all ranks.
+    mean, and the gate sample c is identical on all ranks;
+  * a forward-only generation path with no counterpart in the reference: `generate(y)` decodes target labels through
+    the conditional prior, `reconstruct(x)` decodes an image's posterior, `intervene(x, y_new)` moves an image's classify
+    dims to new labels by a Gaussian counterfactual; each returns a [B,64,64,3] fp32 or uint8 image on the device.
 """
 from __future__ import annotations
 
@@ -30,7 +34,7 @@ import torch
 
 from . import _lib, dp
 from ._lib import (GATE_WS_FLOATS, LATENT_PARTIAL_FLOATS, RESULT_SLOT_FLOATS, ChainBwdArgs, ChainFwdArgs, DpArgs,
-                   LatentBwdArgs, LatentFwdArgs, ptr)
+                   GenLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
 from .engine import Engine, _stream
 from .networks import Classifier, Conditional_Prior, Decoder, Encoder, _default_device, as_device_f32
 from .params import ParamStore, keras_default_init
@@ -733,6 +737,85 @@ class Learner:
             xs, ys = next(iterator)
             acc += float(self.classifier_accuracy(xs, ys))
         return acc / num_batches
+
+    # ---- generation path (an extension: the reference has no call that turns labels into images) --------------------
+    def generate(self, y, sample=True, c=None, noise=None, dtype=torch.float32):
+        """Images for target labels y [B,18] (nonzero = 1): z_s = eps_s, z_c = loc_p(y,c) + scale_p(y,c) eps_c with the
+        conditional prior p(z_c|y,c) (networks.py:118-127); `sample=False`: z_s = 0, z_c = loc_p(y,c).
+        Returns a fresh [B,64,64,3] NHWC device tensor: fp32 sigmoid values (`dtype=torch.float32`) or uint8
+        min(255, rint(255 x)) (`dtype=torch.uint8`).  See `intervene` for c, noise and `last`."""
+        return self._generation(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype)
+
+    def reconstruct(self, x, sample=False, noise=None, dtype=torch.float32):
+        """Decoded posterior of images x [B,64,64,3] (fp32 in [0,1] or uint8 0..255): z = the posterior mean (heads after
+        relu / clipped softplus, networks.py:17-18,33-34); `sample=True`: z = loc + scale eps.  Returns the image as
+        `generate` does."""
+        return self._generation(_lib.GEN_RECONSTRUCT, x, None, None, sample, None, noise, dtype)
+
+    def intervene(self, x, y_new, y=None, sample=False, c=None, noise=None, dtype=torch.float32):
+        """Counterfactual of images x: z as in `reconstruct`, then the classify dims move from the labels y to y_new
+        ([B,18] each, nonzero = 1) by abduction - action - prediction under the conditional prior:
+            e = (z_c - loc_p(y,c)) / scale_p(y,c),  z_c' = z_c + (loc_p(y_new,c) - loc_p(y,c)) + (scale_p(y_new,c) - scale_p(y,c)) e.
+        y_new == y leaves z bit-identical (the result equals `reconstruct(x)`); the style dims are never touched.
+        y=None: the classifier's decision sigmoid(logit) > 0.5 on the z_c being moved.  Returns the image as `generate`.
+
+        Common to the three calls: c [18,18] is a fresh gate sample at the current `gating_sampler_temp` unless given
+        (pass the same c to a series of edits); `noise={"eps": [B,45], "U1": [18,18], "U2": [18,18]}` makes the draws
+        explicit (eps layout: style dims 0..26, classify dims 27..44); without it every call draws new noise.
+        `self.last` = {"z": [B,45], "c": [18,18], "y_src": [B,18] int32 labels moved from (intervene) or None}.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        return self._generation(_lib.GEN_INTERVENE, x, y_new, y, sample, c, noise, dtype)
+
+    def _gen_labels(self, y, B, what):
+        t = torch.as_tensor(y) if not torch.is_tensor(y) else y
+        if t.dim() != 2 or t.shape[1] != self.y_dim or t.shape[0] == 0 or (B is not None and t.shape[0] != B):
+            raise ValueError("{} must be [B,{}]{}, got {}".format(what, self.y_dim, "" if B is None else " with B={}".format(B),
+                                                                tuple(t.shape)))
+        return (t.to(self.device, non_blocking=True) != 0).to(torch.int64).contiguous()
+
+    def _generation(self, mode, x, y_tgt, y_src, sample, c, noise, dtype):
+        if dtype not in (torch.float32, torch.uint8):
+            raise ValueError("dtype must be torch.float32 or torch.uint8, got {}".format(dtype))
+        if x is not None:
+            x, _ = self._prep_inputs(x, None)
+            B = x.shape[0]
+            if B == 0:
+                raise ValueError("x holds no image")
+        else:
+            B = None
+        if y_tgt is not None:
+            y_tgt = self._gen_labels(y_tgt, B, "y" if x is None else "y_new")
+            B = y_tgt.shape[0]
+        if y_src is not None:
+            y_src = self._gen_labels(y_src, B, "y")
+        n = self._noise(noise, B, False, 0)
+        for k, shape in (("eps", (B, self.z_dim)), ("U1", (18, 18)), ("U2", (18, 18))):
+            if n[k] is not None and tuple(n[k].shape) != shape:
+                raise ValueError("noise[{!r}] must be {}, got {}".format(k, list(shape), tuple(n[k].shape)))
+        if c is not None:
+            c = as_device_f32(c, self.device)
+            if tuple(c.shape) != (18, 18):
+                raise ValueError("c must be [18,18], got {}".format(tuple(c.shape)))
+        b = self.engine.bufs(B)
+        z = torch.empty(B, self.z_dim, dtype=torch.float32, device=self.device)
+        y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if mode == _lib.GEN_INTERVENE else None
+        with self._fresh_noise():
+            self._gate(n, c_in=c)
+            if x is None:
+                self.engine.pack_weights()
+            else:
+                self.engine.encoder_fwd(x, b)
+            a, io = GenLatentArgs(), self.engine.latent_io(b)
+            a.batch, a.mode, a.sample = B, mode, int(bool(sample))
+            if x is not None:
+                a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
+            a.y_tgt, a.y_src, a.eps = ptr(y_tgt), ptr(y_src), ptr(n["eps"])
+            a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
+            a.gate_ws, a.z, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(z), io["z16"], ptr(y_used)
+            _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
+            img = self.engine.image_fwd(z, b, B, dtype == torch.uint8)
+        self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
+        return img
 
     # ---- checkpoints (gated_ccvae.py:146-165, 391-419) ---------------------------------------------------------------
     # file stem -> parameter prefix; inside a file the tensors follow Keras' own order (layer_names x weight_names),
