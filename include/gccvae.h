@@ -176,6 +176,16 @@ int gccvae_fill_f32(float* p, long long n, float v, void* stream);
  *   The uint8 output is the fp32 output of the same call converted by that rule, bit for bit. */
 int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp8, const float* bias, void* out, int out_u8,
                             void* stream);
+/* Likelihood of K decoded rows per source image (no counterpart in the reference: the importance-weighted estimate of
+ * gated_ccvae.py's Learner.log_likelihood): conv5t forward + sigmoid + the Laplace log-likelihood of utils.py:101-105,
+ * with no gradient, no reconstruction and no bias gradient.
+ *   g4: [rows,32,32,32] bf16, the decoder's conv4t output of `rows` decoded rows; Wp8, bias: as gccvae_convt_recon_bf16.
+ *   Decoded row r is scored against source image r / kc (rows = B * kc, image-major).  x / x_u8 as for
+ *   gccvae_convt_recon_bf16, over the B source images: 0 = fp32 [B,64,64,3], 1 = uint8 [B,64,64,3], 2 = the raw-byte
+ *   blocks XB [B,33,33,16] of gccvae_prep_x2_bf16 (16-byte aligned).
+ *   log_pxz [rows]: must hold -12288 ln 2 on entry (gccvae_fill_f32); -|x - xhat|_1 is added. */
+int gccvae_convt_ll_bf16(int rows, int kc, const void* g4, const void* Wp8, const float* bias, const void* x, int x_u8,
+                         float* log_pxz, void* stream);
 /* S -> L "halo" kernel for 16x16 / 32x32 S planes with 32 or 64 channels and C_L <= 64: all four output-parity
  * phases per CTA from three column-shifted halo boxes (3.6x less L2 traffic than gccvae_sl_bf16), one MMA per
  * shifted view with N = 4*C_L.  Weights packed "sl9" = [9 views][4 phases][C_L padded to 16][C_S]
@@ -310,6 +320,48 @@ typedef struct {
   int* y_src_out;          /* optional [B,18] int32: the y_src used (INTERVENE) */
 } gccvae_gen_latent_args;
 int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
+
+/* ---- importance-weighted log-likelihood (no counterpart in the reference) -------------------------------------
+ * log p(x [, y]) >= log p_hat = logsumexp_k log w_k - ln K over K samples per image, with proposal q(z|x) (labelled) or
+ * q(z|x) q(y|z_c) (unlabelled) and the gate sample c of gate_ws:
+ *   z_k = loc + scale eps_k (eps_k [45]: columns 0..26 style dims, 27..44 classify dims, as gccvae_latent_fwd);
+ *   y_k = y (labelled) or [U_k < sigmoid(logit(z_c,k))] (unlabelled, U_k [18] uniform: the rule of gated_ccvae.py:206);
+ *   log w_k = log p(x|z_k) + log p(z_s) + log p(z_c,k|y_k) + log p(y_k) - log q(z_k|x) [- log q(y_k|z_c,k) unlabelled]
+ * with N(0,1) style prior, the conditional prior of networks.py:118-127, log p(y) = 18 ln 0.5, log q(z|x) computed from
+ * eps_k itself (not from (z - loc) / scale) and log p(x|z) = the Laplace likelihood of utils.py:101-105.
+ *
+ * The K samples are processed in chunks of kc samples per image; rows of a chunk are image-major, r = b * kc + j for
+ * sample k0 + j of image b.  The Philox draws of (image b, sample k) depend on (seed, offset, b, k) only - never on the
+ * chunking or on B - and gccvae_draw_noise_f32 kinds 4 / 5 reproduce them.
+ *
+ * gccvae_iw_latent: one warp per row; writes the decoder operand of every row of the chunk and lw_part[row] = every
+ * term of log w_k except log p(x|z_k). */
+typedef struct {
+  int batch;               /* B source images */
+  int K;                   /* samples per image of the whole estimate (the explicit noise is [K,B,...]) */
+  int k0, kc;              /* this chunk: samples k0 .. k0 + kc - 1 of every image, rows = B * kc */
+  int labelled;            /* 1: y given; 0: y_k drawn from the classifier */
+  int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
+  const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu */
+  const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip */
+  const long long* y;      /* [B,18] int64 labels, nonzero = 1 (labelled) */
+  const float* eps;        /* [K,B,45] N(0,1) or NULL -> Philox */
+  const float* U_y;        /* [K,B,18] uniforms (unlabelled) or NULL -> Philox */
+  uint64_t seed, offset;   /* Philox key / counter base */
+  const int* step_dev;     /* optional device int added to `offset` */
+  const float* gate_ws;    /* from gccvae_gate_fwd */
+  /* outputs */
+  float* lw_part;          /* [rows] */
+  float* z;                /* optional [rows,45] fp32 (operand of the fp32 decoder) */
+  void* z16;               /* optional bf16 [rows,64], columns 45..63 zero (operand of the tensor-core fc1) */
+} gccvae_iw_latent_args;
+int gccvae_iw_latent(const gccvae_iw_latent_args* a, void* stream);
+/* Online log-sum-exp over the chunks: for every image b the chunk's log w = lw_part[r] + log_pxz[r] of its kc rows
+ * r = b * kc + j is folded into state[b] = {max m, sum e^(lw - m), sum e^(2 (lw - m))} (first != 0: the state is
+ * started, not read).  log_w (optional): [K,B], log_w[k0 + j][b] = log w.  finalize != 0 (the last chunk):
+ * est[b] = m + ln(sum e^(lw - m)) - ln K and ess[b] = (sum w)^2 / sum w^2. */
+int gccvae_iw_accumulate(int batch, int kc, int k0, int K, const float* lw_part, const float* log_pxz, float* state,
+                         float* log_w, int first, int finalize, float* est, float* ess, void* stream);
 
 /* reduce the partials; chain through c to mu (clip / pow / ratio of gated_ccvae.py:103-109) and
  * add the L1 term gating_reg*mean|mu| (gated_ccvae.py:229-230,297-298) scaled by l1_scale
@@ -473,7 +525,8 @@ int gccvae_head_act_f32(const float* loc_pre, const float* scale_pre, long long 
 int gccvae_accuracy_f32(const float* logits, const long long* y, int n, float* out, void* stream);
 
 /* test/debug aid: write the noise the kernels would draw in Philox mode.
- * kind 0: eps [B,45]; 1: eps_k [K,B,18]; 2: U_y [B,18]; 3: U1|U2 [2,18,18]. */
+ * kind 0: eps [B,45]; 1: eps_k [K,B,18]; 2: U_y [B,18]; 3: U1|U2 [2,18,18];
+ * 4: eps [K,B,45] and 5: U_y [K,B,18] of gccvae_iw_latent. */
 int gccvae_draw_noise_f32(int kind, uint64_t seed, uint64_t offset, int batch, int K, float* out, void* stream);
 
 /* ---- tiled module API (networks.py:72-74,83-86,104-106,118-127) --------------------------------------

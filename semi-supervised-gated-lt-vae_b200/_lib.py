@@ -47,6 +47,16 @@ class GenLatentArgs(C.Structure):
     ]
 
 
+class IwLatentArgs(C.Structure):
+    """gccvae_iw_latent_args (include/gccvae.h)."""
+    _fields_ = [
+        ("batch", C.c_int), ("K", C.c_int), ("k0", C.c_int), ("kc", C.c_int), ("labelled", C.c_int), ("ld_pre", C.c_int),
+        ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y", C.c_void_p), ("eps", C.c_void_p), ("U_y", C.c_void_p),
+        ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p), ("gate_ws", C.c_void_p),
+        ("lw_part", C.c_void_p), ("z", C.c_void_p), ("z16", C.c_void_p),
+    ]
+
+
 class LatentBwdArgs(C.Structure):
     _fields_ = [
         ("batch", C.c_int), ("batch_global", C.c_int), ("supervised", C.c_int), ("K", C.c_int),
@@ -157,11 +167,14 @@ SIGNATURES = {
     "gccvae_tap4_wg_bf16": (_I, [_I, _P, _P, _I, _P, _P, _P]),
     "gccvae_convt_recon_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _I, _P]),
     "gccvae_convt_image_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P]),
+    "gccvae_convt_ll_bf16": (_I, [_I, _I, _P, _P, _P, _P, _I, _P, _P]),
     "gccvae_fill_f32": (_I, [_P, _LL, _F, _P]),
     "gccvae_gate_fwd": (_I, [_P, _P, _P, _P, _U64, _U64, _P, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gccvae_latent_fwd": (_I, [C.POINTER(LatentFwdArgs), _P]),
     "gccvae_latent_bwd_partials": (_I, [_I]),
     "gccvae_gen_latent": (_I, [C.POINTER(GenLatentArgs), _P]),
+    "gccvae_iw_latent": (_I, [C.POINTER(IwLatentArgs), _P]),
+    "gccvae_iw_accumulate": (_I, [_I, _I, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P, _P]),
     "gccvae_latent_bwd": (_I, [C.POINTER(LatentBwdArgs), _P]),
     "gccvae_chain_rows": (_I, [_I]),
     "gccvae_chain_partials": (_I, [_I]),

@@ -44,7 +44,7 @@ void count_launch(int n = 1);
 // stream id, per-step offset); key = seed.  Forward and backward kernels regenerate identical
 // noise from identical counters, so no noise tensor ever touches HBM in RNG mode.
 // ---------------------------------------------------------------------------------------------
-enum PhiloxStream : uint32_t { PH_EPS = 0, PH_EPS_K = 1, PH_UY = 2, PH_GATE = 3 };
+enum PhiloxStream : uint32_t { PH_EPS = 0, PH_EPS_K = 1, PH_UY = 2, PH_GATE = 3, PH_IW_EPS = 4, PH_IW_UY = 5 };
 
 __host__ __device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
   const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u;

@@ -1953,6 +1953,198 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_image_kernel(const __grid
   }
 }
 
+// conv5t forward + sigmoid + Laplace log-likelihood of decoded row n against source image n / kc - the importance-
+// weighted likelihood's last layer.  Pipeline (TMA box, taps as descriptor row offsets, barriers, phases, MMA issue, the
+// XM = 2 bulk copy of the raw-byte blocks) and epilogue arithmetic are those of convt_recon_kernel; the only semantic
+// change is the source image of a row.  No gradient, no reconstruction, no bias gradient.
+struct alignas(64) CtlParams {
+  CUtensorMap tmA, tmB;
+  const void* x;       // the B source images (form XM)
+  const float* bias;   // [3]
+  float* log_pxz;      // [rows], pre-set to -12288 ln 2
+  int rows, kc, total_tiles, stages;
+};
+
+template <int XM>
+__global__ void __launch_bounds__(TG_THREADS, 4) convt_ll_kernel(const __grid_constant__ CtlParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
+  constexpr int B_TAP = 1024;
+  constexpr int STAGE = CTR_A_STAGE + (XM == 2 ? CTR_X_BYTES : 0);
+  uint8_t* sB = smem;
+  uint8_t* sA = smem + 4 * B_TAP;
+  uint64_t* full = reinterpret_cast<uint64_t*>(sA + p.stages * STAGE);
+  uint64_t* empty = full + p.stages;
+  uint64_t* tfull = empty + p.stages;
+  uint64_t* tempty = tfull + 2;
+  uint64_t* bfull = tempty + 2;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
+  float* s_lut = reinterpret_cast<float*>(tmem_slot + 4) + 4;   // [256] uint8 -> float(u) / 255
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  pdl_launch_dependents();
+  const int per_cta = (p.total_tiles + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int tile_beg = blockIdx.x * per_cta;
+  const int tile_end = min(tile_beg + per_cta, p.total_tiles);
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&p.tmA);
+    tma_prefetch_desc(&p.tmB);
+    for (int s = 0; s < p.stages; ++s) {
+      mbar_init(&full[s], 1);
+      mbar_init(&empty[s], XM == 2 ? 5 : 1);
+    }
+    for (int s = 0; s < 2; ++s) {
+      mbar_init(&tfull[s], 1);
+      mbar_init(&tempty[s], 4);
+    }
+    mbar_init(bfull, 1);
+    fence_mbar_init();
+  }
+  for (int i = threadIdx.x; i < 256; i += TG_THREADS) s_lut[i] = g_u8lut[i];
+  if (XM == 2)
+    for (int i = threadIdx.x; i < p.stages * (CTR_X_BYTES / 16); i += TG_THREADS)
+      reinterpret_cast<uint4*>(sA + (i / (CTR_X_BYTES / 16)) * STAGE + CTR_A_STAGE)[i % (CTR_X_BYTES / 16)] = make_uint4(0u, 0u, 0u, 0u);
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  if (warp == 2) tmem_alloc(tmem_slot, 64);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  pdl_wait();
+
+  if (warp == 0) {
+    if (elect_one() && tile_beg < tile_end) {
+      mbar_expect_tx(bfull, 4 * B_TAP);
+      for (int t = 0; t < 4; ++t) tma_load_2d(sB + t * B_TAP, &p.tmB, bfull, t * 32, 0);
+      int stage = 0;
+      uint32_t ph = 0;
+      int n = tile_beg / 9, k = tile_beg - n * 9;
+      for (int tile = tile_beg; tile < tile_end; ++tile) {
+        const int i_first = (k * 128) / 33;
+        const uint32_t xbytes = XM == 2 ? (uint32_t)min(128, 33 * 33 - k * 128) * 16u : 0u;
+        mbar_wait_relaxed(&empty[stage], ph ^ 1);
+        mbar_expect_tx(&full[stage], CTR_BOX_ROWS * 64 + xbytes);
+        tma_load_4d(sA + stage * STAGE, &p.tmA, &full[stage], 0, -1, i_first - 1, n);
+        if (XM == 2)   // the raw bytes of the SOURCE image of row n
+          bulk_load_1d(sA + stage * STAGE + CTR_A_STAGE,
+                       reinterpret_cast<const uint4*>(p.x) + ((size_t)(n / p.kc) * 1089 + (size_t)k * 128), xbytes,
+                       &full[stage]);
+        if (++stage == p.stages) { stage = 0; ph ^= 1; }
+        if (++k == 9) { k = 0; ++n; }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0 && tile_beg < tile_end) {
+      const uint32_t idesc = instr_desc_bf16(128, 16, 0, 0);
+      const uint64_t dproto = smem_desc(0, 16, 8u * 64u, SW_64);
+      const uint64_t adesc0 = dproto + (uint64_t)(smem_u32(sA) >> 4), bdesc0 = dproto + (uint64_t)(smem_u32(sB) >> 4);
+      int stage = 0;
+      uint32_t ph = 0;
+      int k = tile_beg % 9;
+      mbar_wait(bfull, 0);
+      for (int tile = tile_beg; tile < tile_end; ++tile) {
+        const int li = tile - tile_beg, as = li & 1;
+        const int f0 = k * 128, d0 = f0 - (f0 / 33) * 33;
+        mbar_wait(&tempty[as], ((uint32_t)(li >> 1) & 1u) ^ 1u);
+        mbar_wait(&full[stage], ph);
+        tc_fence_after();
+        const uint64_t a_st = adesc0 + (uint64_t)((uint32_t)stage * (STAGE >> 4) + (uint32_t)(d0 + 34) * 4u);
+        const uint32_t tacc = tmem_base + (uint32_t)as * 32u;
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const uint32_t row_off = (uint32_t)(33 * (t >> 1) + (t & 1)) * 4u;
+#pragma unroll
+          for (int kk = 0; kk < 2; ++kk)
+            umma_bf16(tacc, a_st - (uint64_t)row_off + (uint64_t)(2 * kk), bdesc0 + (uint64_t)(t * (B_TAP >> 4) + 2 * kk),
+                      idesc, (t > 0 || kk > 0) ? 1u : 0u);
+        }
+        umma_commit(&empty[stage]);
+        umma_commit(&tfull[as]);
+        if (++stage == p.stages) { stage = 0; ph ^= 1; }
+        if (++k == 9) k = 0;
+      }
+    }
+  } else {
+    const int q = warp & 3;
+    const int m = q * 32 + lane;
+    constexpr float LOG2E = 1.4426950408889634f;
+    const float nb0 = -LOG2E * __ldg(p.bias), nb1 = -LOG2E * __ldg(p.bias + 1), nb2 = -LOG2E * __ldg(p.bias + 2);
+    using XT = typename std::conditional<XM == 0, float, uint8_t>::type;
+    XT xn[XM == 2 ? 1 : 12];
+    auto fetch_x = [&](int n, int k) {   // the pixels of this thread's block of source image n / kc, one tile ahead
+      if constexpr (XM != 2) {
+        const int f = k * 128 + m;
+        const XT* xs = reinterpret_cast<const XT*>(p.x);
+        const int i = f / 33, j = f - i * 33;
+        const size_t src = (size_t)(n / p.kc);
+#pragma unroll
+        for (int qq = 0; qq < 4; ++qq) {
+          const int Y = min(max(2 * i - 1 + (qq >> 1), 0), 63), X = min(max(2 * j - 1 + (qq & 1), 0), 63);
+          const XT* px = xs + ((src * 64 + Y) * 64 + X) * 3;
+          xn[3 * qq] = __ldg(px); xn[3 * qq + 1] = __ldg(px + 1); xn[3 * qq + 2] = __ldg(px + 2);
+        }
+      }
+    };
+    int n = tile_beg / 9, k = tile_beg - n * 9;
+    if (tile_beg < tile_end) fetch_x(n, k);
+    float l1 = 0.0f;
+    int stage = 0;
+    uint32_t ph = 0;
+    for (int tile = tile_beg; tile < tile_end; ++tile) {
+      const int li = tile - tile_beg, as = li & 1;
+      const int f = k * 128 + m, i = f / 33, j = f - i * 33;
+      const bool row_ok = f < 33 * 33;
+      const int n_cur = n;
+      float xv[12];
+      uint4 xb = make_uint4(0u, 0u, 0u, 0u);
+      if constexpr (XM == 2) {
+        mbar_wait(&full[stage], ph);
+        xb = lds_u4(smem_u32(sA + stage * STAGE + CTR_A_STAGE) + (uint32_t)m * 16u);
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[stage]);
+        if (++stage == p.stages) { stage = 0; ph ^= 1; }
+      } else {
+#pragma unroll
+        for (int k2 = 0; k2 < 12; ++k2) xv[k2] = px_value<XT>(xn[k2], s_lut);
+      }
+      if (++k == 9) { k = 0; ++n; }
+      if (tile + 1 < tile_end) fetch_x(n, k);
+      mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
+      tc_fence_after();
+      uint32_t acc[16];
+      tmem_ld16(tmem_base + (uint32_t)as * 32u + ((uint32_t)(q * 32) << 16), acc);
+      tmem_ld_wait();
+      tc_fence_before();
+      if (lane == 0) mbar_arrive(&tempty[as]);
+      if constexpr (XM == 2) {
+        const uint32_t w[3] = {xb.x, xb.y, xb.z};
+#pragma unroll
+        for (int k2 = 0; k2 < 12; ++k2) xv[k2] = s_lut[(w[k2 >> 2] >> (8 * (k2 & 3))) & 0xffu];
+      }
+      const bool oky[2] = {row_ok && i > 0, row_ok && i < 32}, okx[2] = {j > 0, j < 32};
+#pragma unroll
+      for (int k2 = 0; k2 < 12; ++k2) {
+        const int qq = k2 / 3, c = k2 % 3;
+        const float t = fmaf(__uint_as_float(acc[4 * qq + c]), -LOG2E, c == 0 ? nb0 : (c == 1 ? nb1 : nb2));
+        const float xh = rcp_approx(1.0f + ex2_approx(t));
+        l1 = fmaf((oky[qq >> 1] && okx[qq & 1]) ? 1.0f : 0.0f, fabsf(xv[k2] - xh), l1);
+      }
+      if (k == 0 || tile + 1 == tile_end) {   // once per row (and at the end of the CTA's range)
+        l1 = warp_sum(l1);
+        if (lane == 0 && l1 != 0.0f) atomicAdd(p.log_pxz + n_cur, -l1);
+        l1 = 0.0f;
+      }
+    }
+    tc_fence_before();
+  }
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 64);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // L -> S convolution of a 3-channel image in x2 block form (conv1 forward, conv5t dgrad) with the im2col tile
 // built by four producer warps instead of TMA: TMA moves one box row per ~1.3 cycles whatever its width, so
@@ -3084,6 +3276,59 @@ extern "C" int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp
   if (out_u8) GCC_CUDA(launch_pdl(convt_image_kernel<true>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
   else GCC_CUDA(launch_pdl(convt_image_kernel<false>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
   GCC_CHECK_LAUNCH("convt_image");
+  return GCCVAE_OK;
+}
+
+// conv5t forward + sigmoid + Laplace log-likelihood of `rows` decoded rows, row r against source image r / kc
+// (importance-weighted likelihood): log_pxz[r] (pre-set to -12288 ln 2) += -|x - xhat|_1.
+extern "C" int gccvae_convt_ll_bf16(int rows, int kc, const void* g4, const void* Wp8, const float* bias, const void* x,
+                                    int x_u8, float* log_pxz, void* stream) {
+  GCC_REQUIRE(g4 && Wp8 && bias && x && log_pxz, "convt_ll: null pointer");
+  GCC_REQUIRE(rows > 0 && rows <= (1 << 26) && kc >= 1 && rows % kc == 0, "convt_ll: bad rows %d / kc %d", rows, kc);
+  GCC_REQUIRE(x_u8 >= 0 && x_u8 <= 2 && (x_u8 != 2 || (uintptr_t)x % 16 == 0),
+              "convt_ll: x_u8 = %d (0 fp32 image, 1 uint8 image, 2 raw-byte blocks, 16-byte aligned)", x_u8);
+  GCC_REQUIRE((uintptr_t)g4 % 16 == 0, "convt_ll: g4 must be 16-byte aligned");
+  CtlParams p;
+  memset(&p, 0, sizeof(p));
+  EncodeTiledFn enc = get_encode();
+  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
+  {   // the A box of convt_recon: 6 image rows x (zero column + 32 pixels)
+    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)rows};
+    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
+    cuuint32_t box[4] = {32, 33, 6, 1};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    GCC_REQUIRE(r == CUDA_SUCCESS, "convt_ll: cuTensorMapEncodeTiled failed: %d", (int)r);
+  }
+  int rc;
+  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
+  p.x = x; p.bias = bias; p.log_pxz = log_pxz; p.rows = rows; p.kc = kc; p.total_tiles = rows * 9;
+  // the launch shape of convt_recon's default: 4 CTAs per SM, 3 stages
+  const int per_sm = 4;
+  p.stages = 3;
+  const int stage_bytes = CTR_A_STAGE + (x_u8 == 2 ? CTR_X_BYTES : 0);
+  const size_t smem = 4096 + (size_t)p.stages * stage_bytes + 1024 + 2048;
+  if (int rc2 = ensure_u8lut()) return rc2;
+  static bool attr_set = false;
+  if (!attr_set) {
+    const int mx = 4096 + 3 * (CTR_A_STAGE + CTR_X_BYTES) + 1024 + 2048;
+    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
+    attr_set = true;
+  }
+  int ctas = p.total_tiles < 148 * per_sm ? p.total_tiles : 148 * per_sm;
+  {
+    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
+    ctas = (p.total_tiles + per_cta - 1) / per_cta;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (x_u8 == 2) GCC_CUDA(launch_pdl(convt_ll_kernel<2>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  else if (x_u8) GCC_CUDA(launch_pdl(convt_ll_kernel<1>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  else GCC_CUDA(launch_pdl(convt_ll_kernel<0>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  GCC_CHECK_LAUNCH("convt_ll");
   return GCCVAE_OK;
 }
 

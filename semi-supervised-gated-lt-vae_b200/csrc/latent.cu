@@ -776,13 +776,164 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// importance-weighted log-likelihood (gccvae_iw_latent / gccvae_iw_accumulate, include/gccvae.h)
+// ---------------------------------------------------------------------------------------------
+// Philox index of (image b, sample k): independent of B and of the chunking
+__device__ __forceinline__ uint64_t iw_index(int b, int k) { return ((uint64_t)b << 32) | (uint32_t)k; }
+
+__device__ __forceinline__ float draw_iw_eps(const float* __restrict__ eps, uint64_t seed, uint64_t offset, int B, int b,
+                                             int k, int d) {
+  if (eps != nullptr) return eps[((size_t)k * B + b) * Z + d];
+  float n[4];
+  philox_normal4(seed, offset, PH_IW_EPS, iw_index(b, k) * 12 + (d >> 2), n);
+  return n[d & 3];
+}
+
+__device__ __forceinline__ float draw_iw_uy(const float* __restrict__ U_y, uint64_t seed, uint64_t offset, int B, int b,
+                                            int k, int j) {
+  if (U_y != nullptr) return U_y[((size_t)k * B + b) * Y + j];
+  uint32_t r[4];
+  philox4x32(seed, offset, PH_IW_UY, iw_index(b, k) * 5 + (j >> 2), r);
+  return u32_to_unit(r[j & 3]);
+}
+
+// One warp per row.  The Normal normalisers cancel: log p(z_s) + log p(z_c|y) - log q(z|x) carries
+// (-27 - 18 + 45) * ln(2 pi) / 2 = 0, so none of the three terms adds it.
+__global__ void __launch_bounds__(WARPS * 32) iw_latent_kernel(gccvae_iw_latent_args a) {
+  pdl_prologue();
+  __shared__ __align__(16) GateSmem g;
+  __shared__ float s_zc[WARPS][ZC];
+  load_gate_smem(g, a.gate_ws);
+  __syncthreads();
+  if (a.step_dev) a.offset += (uint64_t)(*a.step_dev);
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int ldp = a.ld_pre > 0 ? a.ld_pre : Z;
+  const int rows = a.batch * a.kc;
+  float* zcs = s_zc[wid];
+
+  for (int r = blockIdx.x * WARPS + wid; r < rows; r += gridDim.x * WARPS) {
+    const int b = r / a.kc, k = a.k0 + (r - b * a.kc);
+    // --- z_k = loc + scale eps_k; -log q(z_k|x) and log p(z_s) ----------------------------------------------
+    float part = 0.0f;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int d = lane + 32 * h;
+      if (d < Z) {
+        float loc, sc;
+        head_act(a.loc_pre[(size_t)b * ldp + d], a.scale_pre[(size_t)b * ldp + d], loc, sc);
+        const float e = draw_iw_eps(a.eps, a.seed, a.offset, a.batch, b, k, d);
+        const float z = fmaf(sc, e, loc);
+        part += fmaf(0.5f * e, e, logf(sc));            // -log q(z_k|x), dimension d
+        if (d < ZS) part -= 0.5f * z * z;                 // log p(z_s)
+        else zcs[d - ZS] = z;
+        if (a.z != nullptr) a.z[(size_t)r * Z + d] = z;
+        if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(z);
+      } else if (d < 64 && a.z16 != nullptr) {
+        reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(0.0f);
+      }
+    }
+    __syncwarp();
+    // --- labels y_k: given, or drawn from the gated classifier (then -log q(y_k|z_c,k)) ----------------------------
+    bool y1 = false;
+    float lqy = 0.0f;
+    if (lane < Y) {
+      if (a.labelled) {
+        y1 = a.y[(size_t)b * Y + lane] != 0;
+      } else {
+        float acc = g.b[lane];
+#pragma unroll
+        for (int i = 0; i < ZC; ++i) acc = fmaf(zcs[i], g.M[i * Y + lane], acc);
+        y1 = draw_iw_uy(a.U_y, a.seed, a.offset, a.batch, b, k, lane) < sigmoid_f(acc);
+        lqy = bern_lp(acc, y1);
+      }
+    }
+    part -= lqy;
+    const uint32_t ymask = __ballot_sync(0xffffffffu, y1);
+    // --- log p(z_c,k|y_k) under the conditional prior ---------------------------------------------------------------
+    if (lane < ZC) {
+      float mp, spr;
+      prior_i(g, ymask, lane, mp, spr);
+      const float sp = clip_f(softplus_f(spr), 1e-3f, 1e3f);
+      const float t = (zcs[lane] - mp) / sp;
+      part -= fmaf(0.5f * t, t, logf(sp));
+    }
+    const float lw = warp_sum(part);
+    if (lane == 0) a.lw_part[r] = lw + (float)Y * logf(0.5f);   // + log p(y_k)
+    __syncwarp();
+  }
+}
+
+// one warp per image: the lanes stride over the chunk's kc rows with their own running (max, sums), joined by shuffles
+__global__ void __launch_bounds__(256) iw_accumulate_kernel(int B, int kc, int k0, int K,
+                                                            const float* __restrict__ lw_part,
+                                                            const float* __restrict__ log_pxz, float* __restrict__ state,
+                                                            float* __restrict__ log_w, int first, int finalize,
+                                                            float* __restrict__ est, float* __restrict__ ess) {
+  pdl_prologue();
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (b >= B) return;
+  float m = -INFINITY, s1 = 0.0f, s2 = 0.0f;
+  for (int j = lane; j < kc; j += 32) {
+    const size_t r = (size_t)b * kc + j;
+    const float lw = lw_part[r] + log_pxz[r];
+    if (log_w != nullptr) log_w[(size_t)(k0 + j) * B + b] = lw;
+    const float m_new = fmaxf(m, lw);
+    const float f = m == -INFINITY ? 0.0f : expf(m - m_new), e = expf(lw - m_new);
+    s1 = fmaf(s1, f, e);
+    s2 = fmaf(s2, f * f, e * e);
+    m = m_new;
+  }
+  // the warp's chunk result, then the state of the earlier chunks (lane 0)
+  const float mx = warp_max(m);
+  const float f = m == -INFINITY ? 0.0f : expf(m - mx);
+  s1 = warp_sum(s1 * f);
+  s2 = warp_sum(s2 * f * f);
+  if (lane != 0) return;
+  m = mx;
+  if (!first) {
+    const float mo = state[3 * (size_t)b], so1 = state[3 * (size_t)b + 1], so2 = state[3 * (size_t)b + 2];
+    const float m_new = fmaxf(mo, m);
+    const float fo = mo == -INFINITY ? 0.0f : expf(mo - m_new), fc = m == -INFINITY ? 0.0f : expf(m - m_new);
+    s1 = so1 * fo + s1 * fc;
+    s2 = so2 * fo * fo + s2 * fc * fc;
+    m = m_new;
+  }
+  state[3 * (size_t)b] = m;
+  state[3 * (size_t)b + 1] = s1;
+  state[3 * (size_t)b + 2] = s2;
+  if (finalize) {
+    est[b] = m + logf(s1) - logf((float)K);
+    ess[b] = s1 * s1 / s2;
+  }
+}
+
+// kinds 4 / 5 of gccvae_draw_noise_f32: eps [K,B,45] and U_y [K,B,18] of iw_latent_kernel
+__global__ void draw_iw_noise_kernel(int kind, uint64_t seed, uint64_t offset, int B, int K, float* __restrict__ out) {
+  const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  const int w = kind == 4 ? Z : Y;
+  if (t >= (long long)K * B * w) return;
+  const int d = (int)(t % w);
+  const long long kb = t / w;
+  const int b = (int)(kb % B), k = (int)(kb / B);
+  out[t] = kind == 4 ? draw_iw_eps(nullptr, seed, offset, B, b, k, d) : draw_iw_uy(nullptr, seed, offset, B, b, k, d);
+}
+
 }  // namespace gccvae
 
 using namespace gccvae;
 
 extern "C" int gccvae_draw_noise_f32(int kind, uint64_t seed, uint64_t offset, int batch, int K, float* out,
                                      void* stream) {
-  GCC_REQUIRE(out && kind >= 0 && kind <= 3 && batch > 0, "draw_noise: bad args");
+  GCC_REQUIRE(out && kind >= 0 && kind <= 5 && batch > 0, "draw_noise: bad args");
+  if (kind >= 4) {
+    GCC_REQUIRE(K >= 1, "draw_noise: kinds 4 / 5 need K >= 1");
+    const long long n4 = (long long)K * batch * (kind == 4 ? Z : Y);
+    draw_iw_noise_kernel<<<(int)((n4 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(kind, seed, offset, batch, K, out);
+    GCC_CHECK_LAUNCH("draw_noise");
+    return GCCVAE_OK;
+  }
   long long n = kind == 0 ? (long long)batch * Z : kind == 1 ? (long long)batch * K : kind == 2 ? (long long)batch * Y : NP;
   GCC_REQUIRE(n > 0, "draw_noise: empty");
   draw_noise_kernel<<<(int)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(kind, seed, offset, batch, K, out);
@@ -858,6 +1009,35 @@ extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) 
               "gen_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
   GCC_CUDA(launch_pdl_k(gen_latent_kernel, dim3(latent_grid(a->batch)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   GCC_CHECK_LAUNCH("gen_latent");
+  return GCCVAE_OK;
+}
+
+extern "C" int gccvae_iw_latent(const gccvae_iw_latent_args* a, void* stream) {
+  GCC_REQUIRE(a, "iw_latent: null args");
+  GCC_REQUIRE(a->batch > 0 && a->K >= 1 && a->kc >= 1 && a->k0 >= 0 && a->k0 + a->kc <= a->K,
+              "iw_latent: bad sizes B=%d K=%d k0=%d kc=%d", a->batch, a->K, a->k0, a->kc);
+  GCC_REQUIRE((long long)a->batch * a->kc < (1LL << 31), "iw_latent: too many rows");
+  GCC_REQUIRE(a->loc_pre && a->scale_pre && a->ld_pre >= 0 && a->gate_ws && a->lw_part, "iw_latent: null pointer");
+  GCC_REQUIRE(!a->labelled || a->y, "iw_latent: labelled needs y");
+  GCC_REQUIRE((uintptr_t)a->z % 4 == 0 && (uintptr_t)a->eps % 4 == 0 && (uintptr_t)a->U_y % 4 == 0 &&
+                  (uintptr_t)a->loc_pre % 4 == 0 && (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y % 8 == 0 &&
+                  (uintptr_t)a->lw_part % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
+              "iw_latent: misaligned pointer (fp32: 4 bytes, int64: 8, z16: 16)");
+  const int rows = a->batch * a->kc;
+  GCC_CUDA(launch_pdl_k(iw_latent_kernel, dim3(latent_grid(rows)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+  GCC_CHECK_LAUNCH("iw_latent");
+  return GCCVAE_OK;
+}
+
+extern "C" int gccvae_iw_accumulate(int batch, int kc, int k0, int K, const float* lw_part, const float* log_pxz,
+                                    float* state, float* log_w, int first, int finalize, float* est, float* ess,
+                                    void* stream) {
+  GCC_REQUIRE(batch > 0 && kc >= 1 && k0 >= 0 && k0 + kc <= K, "iw_accumulate: bad sizes B=%d K=%d k0=%d kc=%d", batch,
+              K, k0, kc);
+  GCC_REQUIRE(lw_part && log_pxz && state && (!finalize || (est && ess)), "iw_accumulate: null pointer");
+  GCC_CUDA(launch_pdl_k(iw_accumulate_kernel, dim3((batch + 7) / 8), dim3(256), 0, (cudaStream_t)stream, batch, kc, k0,
+                        K, lw_part, log_pxz, state, log_w, first, finalize, est, ess));
+  GCC_CHECK_LAUNCH("iw_accumulate");
   return GCCVAE_OK;
 }
 

@@ -71,6 +71,7 @@ class Engine:
             raise _lib.GccvaeError("the Gated-CCVAE kernels run on a CUDA device only (got {})".format(self.device))
         _lib.check(self.lib.gccvae_arch_check(self.device.index or 0), "arch_check")
         self._bufs = {}
+        self._dec_bufs = {}
 
     # ---- buffers -----------------------------------------------------------------------------------
     def bufs(self, batch):
@@ -97,6 +98,17 @@ class Engine:
             ws_bytes = max(ws_bytes, self.lib.gccvae_colsum_f32_workspace_bytes(B * oh * ow, oc))
         b["ws"] = torch.empty(ws_bytes // 4 + 16, dtype=f32, device=dev)
         b["ws_bytes"] = ws_bytes
+        return b
+
+    def dec_bufs(self, rows):
+        """forward-only decoder buffers for `rows` latent rows (importance-weighted likelihood): the decoder's
+        activations and its input z [rows,45], without the encoder's tensors or any gradient."""
+        b = self._dec_bufs.get(rows)
+        if b is None:
+            b = {lay[0] + ".out": torch.empty(rows, *out_shape(lay), dtype=torch.float32, device=self.device)
+                 for lay in DEC_LAYERS}
+            b["z"] = torch.empty(rows, 45, dtype=torch.float32, device=self.device)
+            self._dec_bufs[rows] = b
         return b
 
     # ---- single layer ops -------------------------------------------------------------------------------
@@ -169,6 +181,15 @@ class Engine:
         values or (out_u8) uint8 min(255, rint(255 xhat)) with the product and the rounding in fp32."""
         xhat = self.decoder_fwd(z, b)
         return image_u8(xhat) if out_u8 else xhat.clone()
+
+    def iw_decoder_ll(self, x, b, batch, kc, dec, log_pxz):
+        """importance-weighted likelihood: log_pxz[r] = log p(x_(r / kc) | z_r) for the batch * kc rows of dec["z"]
+        (the parity path: the generic decoder, then the reconstruction likelihood against the repeated images)."""
+        rows = batch * kc
+        xhat = self.decoder_fwd(dec["z"][:rows], dec)
+        xr = x.repeat_interleave(kc, 0) if kc > 1 else x
+        _lib.check(self.lib.gccvae_recon_f32(ptr(xr), ptr(xhat), rows, 64 * 64 * 3, None, ptr(log_pxz), None,
+                                             _stream()), "recon")
 
     def decoder_bwd(self, z, b, want_dz=True):
         """expects b['dec.conv5t.dout'] = dLoss/d(pre-sigmoid logits); returns dz."""

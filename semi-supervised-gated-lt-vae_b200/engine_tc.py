@@ -220,6 +220,19 @@ class EngineTC(Engine):
             b[tname] = e(B, H // 2 + 1, W // 2 + 1, 4 * Cc, dt=BF16)   # zero borders are never written
         return b
 
+    def dec_bufs(self, rows):
+        """forward-only decoder buffers for `rows` latent rows (importance-weighted likelihood): the z16 operand and the
+        bf16 activations of fc1 .. conv4t, about 92 KB per row - a fraction of `bufs`, which also holds the encoder's
+        tensors and every gradient."""
+        b = self._dec_bufs.get(rows)
+        if b is None:
+            b = {"z16": torch.zeros(rows, 64, dtype=BF16, device=self.device),
+                 "dec.fc1.out": torch.zeros(rows, 64, dtype=BF16, device=self.device)}
+            for name in ["dec.conv1t"] + TC_DEC:
+                b[name + ".out"] = torch.empty(rows, *out_shape(_DEC[name]), dtype=BF16, device=self.device)
+            self._dec_bufs[rows] = b
+        return b
+
     def _xhat4(self, b, B):
         if b["xhat4"] is None:     # only the stand-alone Decoder(z) call needs it in x2 mode
             b["xhat4"] = torch.zeros(B, 64, 64, 4, dtype=torch.float32, device=self.device)
@@ -499,6 +512,19 @@ class EngineTC(Engine):
             batch, ptr(g4), ptr(self.wp["dec.conv5t.x2t"]), ptr(self.store.view("dec.conv5t.b")), ptr(out), int(out_u8),
             _stream()))
         return out
+
+    def iw_decoder_ll(self, x, b, batch, kc, dec, log_pxz):
+        """importance-weighted likelihood: the decoder over the batch * kc rows of dec["z16"], then conv5t + sigmoid +
+        Laplace log-likelihood of row r against source image r / kc (gccvae_convt_ll_bf16) into log_pxz.  A uint8 image
+        is read from the raw-byte blocks the encoder's prep_x2 wrote into b["X2"]: once per call, not once per sample."""
+        rows = batch * kc
+        self.decoder_fwd(None, dec, z16_ready=True, fused_recon=True, batch=rows, head=True)
+        _lib.check(self.lib.gccvae_fill_f32(ptr(log_pxz), rows, -12288.0 * 0.6931471805599453, _stream()), "fill")
+        u8 = int(x.dtype == torch.uint8)
+        g4 = dec["dec.conv4t.out"]
+        self._run("dec.conv5t fwd ll", (g4[:rows], x), lambda: self.lib.gccvae_convt_ll_bf16(
+            rows, kc, ptr(g4), ptr(self.wp["dec.conv5t.x2t"]), ptr(self.store.view("dec.conv5t.b")),
+            self.xb_ptr(b["X2"], batch) if u8 else ptr(x), 2 * u8, ptr(log_pxz), _stream()))
 
     # ---- backward -----------------------------------------------------------------------------------------------
     def decoder_bwd(self, z, b, want_dz=True, tail=True):

@@ -8,8 +8,9 @@ sm_100a kernels.  Same class names, constructor arguments, method names and retu
     loss, c = learner.train_step(x, y, supervised)      # :302-311  (fwd + bwd + Adam)
     acc     = learner.classifier_accuracy(x, y)         # :421-446
     img     = learner.generate(y) / .reconstruct(x) / .intervene(x, y_new)   # extension, see below
+    ll      = learner.log_likelihood(x, y=None, k=100)                        # extension, see below
 
-Extensions the reference lacks (for parity testing, data parallelism and image generation):
+Extensions the reference lacks (for parity testing, data parallelism, image generation and likelihood evaluation):
   * every stochastic call takes an optional `noise=` dict of explicit draws
     (eps [B,45], eps_k [K,B,45], U_y [B,18], U1/U2 [18,18]); without it noise comes from an
     in-kernel Philox4x32-10 keyed by (seed, step counter);
@@ -19,7 +20,10 @@ Extensions the reference lacks (for parity testing, data parallelism and image g
     mean, and the gate sample c is identical on all ranks;
   * a forward-only generation path with no counterpart in the reference: `generate(y)` decodes target labels through
     the conditional prior, `reconstruct(x)` decodes an image's posterior, `intervene(x, y_new)` moves an image's classify
-    dims to new labels by a Gaussian counterfactual; each returns a [B,64,64,3] fp32 or uint8 image on the device.
+    dims to new labels by a Gaussian counterfactual; each returns a [B,64,64,3] fp32 or uint8 image on the device;
+  * the importance-weighted (IWAE) log-likelihood with K samples: `log_likelihood(x)` bounds log p(x) and
+    `log_likelihood(x, y)` bounds log p(x, y) per image (nats, tighter as K grows); `test_log_likelihood(loader)` is its
+    `accuracy(loader)` counterpart.
 """
 from __future__ import annotations
 
@@ -34,7 +38,7 @@ import torch
 
 from . import _lib, dp
 from ._lib import (GATE_WS_FLOATS, LATENT_PARTIAL_FLOATS, RESULT_SLOT_FLOATS, ChainBwdArgs, ChainFwdArgs, DpArgs,
-                   GenLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
+                   GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
 from .engine import Engine, _stream
 from .networks import Classifier, Conditional_Prior, Decoder, Encoder, _default_device, as_device_f32
 from .params import ParamStore, keras_default_init
@@ -816,6 +820,89 @@ class Learner:
             img = self.engine.image_fwd(z, b, B, dtype == torch.uint8)
         self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
         return img
+
+    # ---- importance-weighted log-likelihood (an extension: the reference scores a model by accuracy only) ------------
+    def log_likelihood(self, x, y=None, k=100, c=None, noise=None, max_rows=8192, keep_log_w=False):
+        """Importance-weighted (IWAE) estimate of log p(x) - or of log p(x, y) when labels y [B,18] (nonzero = 1) are
+        given - per image, in nats: log p_hat = logsumexp_k log w_k - ln k over k samples z_k = loc + scale eps_k of the
+        posterior, with
+            log w_k = log p(x|z_k) + log p(z_s) + log p(z_c|y_k, c) + log p(y_k) - log q(z_k|x) [- log q(y_k|z_c, c)]
+        where y_k = y, or (y=None) y_k ~ Bernoulli(sigmoid(classifier(z_c))) as unsup_loss draws it and the bracketed
+        term is included.  A lower bound that tightens as k grows; conditional on the call's gate sample c (in one-one
+        mode c = I exactly).  x: [B,64,64,3] fp32 in [0,1] or uint8.  Returns a fresh fp32 [B] device tensor.
+          c [18,18]: a fresh gate sample per call unless given (as `generate`);
+          noise={"eps": [k,B,45], "U_y": [k,B,18], "U1": [18,18], "U2": [18,18]}: explicit draws (eps layout: style
+            dims 0..26, classify dims 27..44); without it every call draws new noise;
+          max_rows: decoder rows per chunk - the k samples are decoded in chunks of max(1, max_rows // B) samples per
+            image; this bounds memory and changes only the order of float sums (no draw depends on it);
+          keep_log_w: also keep every log w_k.
+        `self.last` = {"ess": [B] effective sample size (sum w)^2 / sum w^2, "c": [18,18], "log_w": [k,B] or None}.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
+            raise ValueError("k must be an integer >= 1, got {!r}".format(k))
+        if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
+            raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
+        K = int(k)
+        x, _ = self._prep_inputs(x, None)
+        x = x.contiguous()
+        B = x.shape[0]
+        if B == 0:
+            raise ValueError("x holds no image")
+        if y is not None:
+            y = self._gen_labels(y, B, "y")
+        n = self._noise(noise, B, False, 0)
+        for key, shape in (("eps", (K, B, self.z_dim)), ("U_y", (K, B, self.y_dim)), ("U1", (18, 18)), ("U2", (18, 18))):
+            if n[key] is not None and tuple(n[key].shape) != shape:
+                raise ValueError("noise[{!r}] must be {}, got {}".format(key, list(shape), tuple(n[key].shape)))
+        if c is not None:
+            c = as_device_f32(c, self.device)
+            if tuple(c.shape) != (18, 18):
+                raise ValueError("c must be [18,18], got {}".format(tuple(c.shape)))
+        kc = max(1, min(K, int(max_rows) // B))
+        b, dec = self.engine.bufs(B), self.engine.dec_bufs(B * kc)
+        e = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)
+        lw_part, log_pxz, state, est, ess = e(B * kc), e(B * kc), e(B, 3), e(B), e(B)
+        log_w = e(K, B) if keep_log_w else None
+        with self._fresh_noise():
+            self._gate(n, c_in=c)
+            self.engine.encoder_fwd(x, b)
+            io = self.engine.latent_io(b)
+            a = IwLatentArgs()
+            a.batch, a.K, a.labelled = B, K, int(y is not None)
+            a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
+            a.y, a.eps, a.U_y = ptr(y), ptr(n["eps"]), ptr(n["U_y"])
+            a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
+            a.gate_ws, a.lw_part, a.z, a.z16 = ptr(self._gate_ws), ptr(lw_part), ptr(dec.get("z")), ptr(dec.get("z16"))
+            for k0 in range(0, K, kc):
+                kcc = min(kc, K - k0)
+                a.k0, a.kc = k0, kcc
+                _lib.check(self.lib.gccvae_iw_latent(C.byref(a), _stream()), "iw_latent")
+                self.engine.iw_decoder_ll(x, b, B, kcc, dec, log_pxz)
+                _lib.check(self.lib.gccvae_iw_accumulate(B, kcc, k0, K, ptr(lw_part), ptr(log_pxz), ptr(state), ptr(log_w),
+                                                         int(k0 == 0), int(k0 + kcc == K), ptr(est), ptr(ess), _stream()),
+                           "iw_accumulate")
+        self.last = dict(ess=ess, c=self._c.clone(), log_w=log_w)
+        return est
+
+    def test_log_likelihood(self, data_loader, k=100, labelled=False):
+        """The `accuracy(data_loader)` counterpart of `log_likelihood`: one gate sample c is drawn and used for every
+        batch; returns (mean nats per image, mean nats per pixel value (64 x 64 x 3 = 12288 per image), c).  The means
+        weight every image equally (a short last batch counts by its images).  `labelled=True` scores log p(x, y) with
+        the loader's labels, otherwise log p(x)."""
+        with self._fresh_noise():
+            self._gate(self._noise(None, 1, False, 0))
+        c = self._c.clone()
+        iterator = iter(data_loader.step())
+        num_batches = math.ceil(data_loader.n_s / self.train_config["batch_size"])
+        total = torch.zeros((), dtype=torch.float64, device=self.device)
+        images = 0
+        for _ in range(int(num_batches)):
+            xs, ys = next(iterator)
+            est = self.log_likelihood(xs, ys if labelled else None, k=k, c=c)
+            total += est.double().sum()
+            images += est.shape[0]
+        mean = float(total) / images
+        return mean, mean / (64 * 64 * 3), c
 
     # ---- checkpoints (gated_ccvae.py:146-165, 391-419) ---------------------------------------------------------------
     # file stem -> parameter prefix; inside a file the tensors follow Keras' own order (layer_names x weight_names),
