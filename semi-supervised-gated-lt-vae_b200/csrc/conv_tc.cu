@@ -1505,8 +1505,12 @@ __global__ void __launch_bounds__(256) prep_x2_u8_staged_kernel(const uint8_t* _
   }
 }
 
-// Fused Conv2DTranspose(32 -> 3, k4, s2, same) + sigmoid + Laplace log-likelihood (utils.py:101-105) + its
-// gradient w.r.t. the logits, written in block form D2 (the operand of conv5t's dgrad and wgrad).
+// conv5t = Conv2DTranspose(32 -> 3, k4, s2, same) + sigmoid, with one of four epilogues (OUT):
+//   RECON      Laplace log-likelihood (utils.py:101-105) + its gradient w.r.t. the logits, written in block form D2 (the
+//              operand of conv5t's dgrad and wgrad); optional fp32 reconstruction and bias gradient - the training step
+//   LL         Laplace log-likelihood of decoded row n against source image n / kc - the importance-weighted likelihood
+//   IMAGE_F32  the sigmoid into the [B,64,64,3] fp32 image - the generation path
+//   IMAGE_U8   the same as uint8 min(255, rint(255 x))
 // Output block (i, j) of an image = sum over the 2x2 taps (a, b) of g4[i - a, j - b, :] . W_ab  (K = 32 per tap, N = 16).
 // Tile = 128 CONSECUTIVE blocks f = 33 i + j of one image (9 tiles per image, the last one holds 65).  The operand of
 // all four taps is ONE TMA box of the decoder activation g4 [B,32,32,32]: 6 image rows x 33 columns starting at column
@@ -1515,18 +1519,22 @@ __global__ void __launch_bounds__(256) prep_x2_u8_staged_kernel(const uint8_t* _
 // 33): a start-address offset of the A descriptor.  The swizzle XOR is taken from the absolute shared-memory address, so
 // a K-major operand may start at ANY row of a swizzled buffer (scripts/microbench/desc_offset.cu,
 // profiles/r02_microbench_desc_offset.txt) - 198 box rows per tile instead of the 4 x 121 of one box per tap.
-struct alignas(64) CtrParams {
+enum ConvtOut { RECON, LL, IMAGE_F32, IMAGE_U8 };
+
+struct alignas(64) CtParams {
   CUtensorMap tmA, tmB;
-  const void* x;
+  const void* x;       // RECON / LL: the image operand (form XM)
   int x_u8;
   const float* bias;   // [3]
-  const float* coef;   // [B] dLoss/dlog_pxz per image (NULL: forward only, D2 is not written)
-  float* log_pxz;      // [B], pre-set to -12288 ln 2; -|x - xhat|_1 is added
-  uint4* D2;           // [B,33,33,16] bf16
-  float* xhat;         // optional [B,64,64,3] fp32 reconstruction
-  float* db;           // optional [3] += sum of dlogit (bias gradient of conv5t)
+  const float* coef;   // RECON: [B] dLoss/dlog_pxz per image (NULL: forward only, D2 is not written)
+  float* log_pxz;      // RECON / LL: [rows], pre-set to -12288 ln 2; -|x - xhat|_1 is added
+  uint4* D2;           // RECON: [B,33,33,16] bf16
+  float* xhat;         // RECON: optional [B,64,64,3] fp32 reconstruction
+  float* db;           // RECON: optional [3] += sum of dlogit (bias gradient of conv5t)
   int batch, total_tiles, stages;
   long long* timeline;
+  void* out;           // IMAGE_*: [B,64,64,3] fp32 or uint8
+  int kc;              // LL: decoded rows per source image
 };
 
 constexpr int CTR_BOX_ROWS = 6 * 33;          // rows of the A box (64 bytes each)
@@ -1543,19 +1551,23 @@ __device__ __forceinline__ float rcp_approx(float v) {
   return r;
 }
 
-// XM = form of the image operand: 0 fp32 NHWC, 1 uint8 NHWC, 2 uint8 raw-byte blocks XB [B,33,33,16] (prep_x2).
+// XM = form of the image operand of RECON / LL: 0 fp32 NHWC, 1 uint8 NHWC, 2 uint8 raw-byte blocks XB [B,33,33,16]
+// (prep_x2).  The IMAGE kinds read no image and are instantiated with XM = 0.
 // XM = 2: the 2 KB of raw bytes of a tile's 128 blocks travel with the tile's operand box (one bulk copy into the same
 // pipeline stage, same barrier); the stage is free again when the MMAs have read the box AND the four epilogue warps have
 // taken their bytes.  A register prefetch one tile ahead (XM = 0 / 1) is too short: a tile's epilogue is ~0.3 us of work,
 // an HBM access under load ~1.3 us (scripts/timeline_ctr.py: the epilogue warps sat ~1.1 us per tile on that load).
 constexpr int CTR_X_BYTES = 128 * 16;
-template <int XM>
-__global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid_constant__ CtrParams p) {
+template <int OUT, int XM>
+__global__ void __launch_bounds__(TG_THREADS, 4) convt_kernel(const __grid_constant__ CtParams p) {
+  constexpr bool HAS_X = OUT == RECON || OUT == LL;   // reads an image operand
+  static_assert(HAS_X || XM == 0, "the IMAGE kinds are instantiated with XM = 0");
+  constexpr bool RAW_X = HAS_X && XM == 2;            // the raw image bytes travel with the pipeline stage
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
   constexpr int B_TAP = 1024;
-  constexpr int STAGE = CTR_A_STAGE + (XM == 2 ? CTR_X_BYTES : 0);   // [A box][raw bytes of the tile's blocks]
+  constexpr int STAGE = CTR_A_STAGE + (RAW_X ? CTR_X_BYTES : 0);   // [A box][raw bytes of the tile's blocks]
   uint8_t* sB = smem;                 // 4 taps x [16 rows x 64 B]
   uint8_t* sA = smem + 4 * B_TAP;
   uint64_t* full = reinterpret_cast<uint64_t*>(sA + p.stages * STAGE);
@@ -1566,6 +1578,11 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
   float* s_db = reinterpret_cast<float*>(tmem_slot + 4);   // [4]
   float* s_lut = s_db + 4;                                 // [256] uint8 -> float(u) / 255
+  // the source image of decoded row n
+  auto src_image = [&](int n) {
+    if constexpr (OUT == LL) return n / p.kc;
+    else return n;
+  };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_launch_dependents();
@@ -1575,9 +1592,11 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&p.tmA);
     tma_prefetch_desc(&p.tmB);
+    // empty[s] completes when the MMA commit AND, when RAW_X, the four epilogue warps (which take their raw bytes from
+    // the stage) have arrived: the count must be 5 exactly when the epilogue warps arrive on it, else the producer hangs
     for (int s = 0; s < p.stages; ++s) {
       mbar_init(&full[s], 1);
-      mbar_init(&empty[s], XM == 2 ? 5 : 1);
+      mbar_init(&empty[s], RAW_X ? 5 : 1);
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(&tfull[s], 1);
@@ -1586,9 +1605,10 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
     mbar_init(bfull, 1);
     fence_mbar_init();
   }
-  if (threadIdx.x < 4) s_db[threadIdx.x] = 0.0f;
-  for (int i = threadIdx.x; i < 256; i += TG_THREADS) s_lut[i] = g_u8lut[i];
-  if (XM == 2)   // the last tile of an image brings 65 blocks: the other rows read whatever the stage holds (masked)
+  if (OUT == RECON && threadIdx.x < 4) s_db[threadIdx.x] = 0.0f;
+  if constexpr (HAS_X)
+    for (int i = threadIdx.x; i < 256; i += TG_THREADS) s_lut[i] = g_u8lut[i];
+  if (RAW_X)   // the last tile of an image brings 65 blocks: the other rows read whatever the stage holds (masked)
     for (int i = threadIdx.x; i < p.stages * (CTR_X_BYTES / 16); i += TG_THREADS)
       reinterpret_cast<uint4*>(sA + (i / (CTR_X_BYTES / 16)) * STAGE + CTR_A_STAGE)[i % (CTR_X_BYTES / 16)] = make_uint4(0u, 0u, 0u, 0u);
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes above, async-proxy (bulk copy) writes later
@@ -1613,14 +1633,15 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
       int n = tile_beg / 9, k = tile_beg - n * 9;
       for (int tile = tile_beg; tile < tile_end; ++tile) {
         const int i_first = (k * 128) / 33;
-        const uint32_t xbytes = XM == 2 ? (uint32_t)min(128, 33 * 33 - k * 128) * 16u : 0u;
+        const uint32_t xbytes = RAW_X ? (uint32_t)min(128, 33 * 33 - k * 128) * 16u : 0u;
         mbar_wait_relaxed(&empty[stage], ph ^ 1);   // runs stages ahead of its consumers: back off instead of spinning
         TL(tile - tile_beg, 0);
         mbar_expect_tx(&full[stage], CTR_BOX_ROWS * 64 + xbytes);
         tma_load_4d(sA + stage * STAGE, &p.tmA, &full[stage], 0, -1, i_first - 1, n);
-        if (XM == 2)
-          bulk_load_1d(sA + stage * STAGE + CTR_A_STAGE, reinterpret_cast<const uint4*>(p.x) + ((size_t)n * 1089 + (size_t)k * 128),
-                       xbytes, &full[stage]);
+        if (RAW_X)
+          bulk_load_1d(sA + stage * STAGE + CTR_A_STAGE,
+                       reinterpret_cast<const uint4*>(p.x) + ((size_t)src_image(n) * 1089 + (size_t)k * 128), xbytes,
+                       &full[stage]);
         TL(tile - tile_beg, 1);
         if (++stage == p.stages) { stage = 0; ph ^= 1; }
         if (++k == 9) { k = 0; ++n; }
@@ -1673,21 +1694,21 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
     using XT = typename std::conditional<XM == 0, float, uint8_t>::type;
     XT xn[XM == 2 ? 1 : 12];
     auto fetch_x = [&](int n, int k) {
-      if constexpr (XM != 2) {
+      if constexpr (HAS_X && XM != 2) {
         const int f = k * 128 + m;
         const XT* xs = reinterpret_cast<const XT*>(p.x);
         const int i = f / 33, j = f - i * 33;
 #pragma unroll
         for (int qq = 0; qq < 4; ++qq) {
           const int Y = min(max(2 * i - 1 + (qq >> 1), 0), 63), X = min(max(2 * j - 1 + (qq & 1), 0), 63);
-          const XT* px = xs + (((size_t)n * 64 + Y) * 64 + X) * 3;
+          const XT* px = xs + (((size_t)src_image(n) * 64 + Y) * 64 + X) * 3;
           xn[3 * qq] = __ldg(px); xn[3 * qq + 1] = __ldg(px + 1); xn[3 * qq + 2] = __ldg(px + 2);
         }
       }
     };
     int n = tile_beg / 9, k = tile_beg - n * 9;
     if (tile_beg < tile_end) fetch_x(n, k);
-    float l1 = 0.0f;   // |x - xhat|_1 of this thread's blocks of the current image
+    float l1 = 0.0f;   // |x - xhat|_1 of this thread's blocks of the current row
     int stage = 0;
     uint32_t ph = 0;
     for (int tile = tile_beg; tile < tile_end; ++tile) {
@@ -1696,16 +1717,16 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
       const bool row_ok = f < 33 * 33;
       const int n_cur = n;
       // (consumed at the very end of the tile: an L2 access that needs no prefetch)
-      const float cb = p.coef != nullptr ? __ldg(p.coef + n_cur) : 0.0f;
+      const float cb = OUT == RECON && p.coef != nullptr ? __ldg(p.coef + n_cur) : 0.0f;
       float xv[12];
       uint4 xb = make_uint4(0u, 0u, 0u, 0u);
-      if constexpr (XM == 2) {
+      if constexpr (RAW_X) {
         mbar_wait(&full[stage], ph);     // the MMA thread waits on the same phase; here it makes the bulk copy visible
         xb = lds_u4(smem_u32(sA + stage * STAGE + CTR_A_STAGE) + (uint32_t)m * 16u);
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[stage]);
         if (++stage == p.stages) { stage = 0; ph ^= 1; }
-      } else {
+      } else if constexpr (HAS_X) {
 #pragma unroll
         for (int k2 = 0; k2 < 12; ++k2) xv[k2] = px_value<XT>(xn[k2], s_lut);
       }
@@ -1720,7 +1741,7 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
       tc_fence_before();
       if (lane == 0) mbar_arrive(&tempty[as]);
       if (threadIdx.x == 64) TL(li, 5);
-      if constexpr (XM == 2) {   // table lookups: their shared-memory latency hides behind the sigmoid chains below
+      if constexpr (RAW_X) {   // table lookups: their shared-memory latency hides behind the sigmoid chains below
         const uint32_t w[3] = {xb.x, xb.y, xb.z};
 #pragma unroll
         for (int k2 = 0; k2 < 12; ++k2) xv[k2] = s_lut[(w[k2 >> 2] >> (8 * (k2 & 3))) & 0xffu];
@@ -1736,53 +1757,72 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
       }
       // branch-free arithmetic, 12 independent chains: xhat = 1 / (1 + 2^(-(a + b) log2 e)); every row of the tile reads
       // operand rows the box has written (zero-filled outside the image), so rows without work hold finite values
-      float xh[12], g[12];
+      float xh[12];
 #pragma unroll
       for (int k2 = 0; k2 < 12; ++k2) {
         const int qq = k2 / 3, c = k2 % 3;
         const float t = fmaf(__uint_as_float(acc[4 * qq + c]), -LOG2E, c == 0 ? nb0 : (c == 1 ? nb1 : nb2));
         xh[k2] = rcp_approx(1.0f + ex2_approx(t));
       }
-      float cq[4];
+      if constexpr (OUT == RECON) {
+        float g[12], cq[4];
 #pragma unroll
-      for (int qq = 0; qq < 4; ++qq) cq[qq] = okf[qq] * cb;
+        for (int qq = 0; qq < 4; ++qq) cq[qq] = okf[qq] * cb;
 #pragma unroll
-      for (int k2 = 0; k2 < 12; ++k2) {
-        const int qq = k2 / 3;
-        const float e = xv[k2] - xh[k2];
-        l1 = fmaf(okf[qq], fabsf(e), l1);
-        // dLoss/dlogit = coef * sign(x - xhat) * xhat (1 - xhat):  the sign bit of e flips s, e == 0 gives 0
-        const float s = fmaf(-xh[k2], xh[k2], xh[k2]) * cq[qq];
-        const float sg = __uint_as_float(__float_as_uint(s) ^ (__float_as_uint(e) & 0x80000000u));
-        g[k2] = e != 0.0f ? sg : 0.0f;
-      }
-      d0 += g[0] + g[3] + g[6] + g[9];
-      d1 += g[1] + g[4] + g[7] + g[10];
-      d2 += g[2] + g[5] + g[8] + g[11];
-      if (p.D2 != nullptr && row_ok) {
-        uint4* dst = p.D2 + ((size_t)n_cur * 1089 + f) * 2;
-        dst[0] = make_uint4(pack_bf16x2(g[0], g[1]), pack_bf16x2(g[2], 0.0f), pack_bf16x2(g[3], g[4]), pack_bf16x2(g[5], 0.0f));
-        dst[1] = make_uint4(pack_bf16x2(g[6], g[7]), pack_bf16x2(g[8], 0.0f), pack_bf16x2(g[9], g[10]), pack_bf16x2(g[11], 0.0f));
-      }
-      if (p.xhat != nullptr) {   // optional fp32 reconstruction (tests / module API), off the training path
+        for (int k2 = 0; k2 < 12; ++k2) {
+          const int qq = k2 / 3;
+          const float e = xv[k2] - xh[k2];
+          l1 = fmaf(okf[qq], fabsf(e), l1);
+          // dLoss/dlogit = coef * sign(x - xhat) * xhat (1 - xhat):  the sign bit of e flips s, e == 0 gives 0
+          const float s = fmaf(-xh[k2], xh[k2], xh[k2]) * cq[qq];
+          const float sg = __uint_as_float(__float_as_uint(s) ^ (__float_as_uint(e) & 0x80000000u));
+          g[k2] = e != 0.0f ? sg : 0.0f;
+        }
+        d0 += g[0] + g[3] + g[6] + g[9];
+        d1 += g[1] + g[4] + g[7] + g[10];
+        d2 += g[2] + g[5] + g[8] + g[11];
+        if (p.D2 != nullptr && row_ok) {
+          uint4* dst = p.D2 + ((size_t)n_cur * 1089 + f) * 2;
+          dst[0] = make_uint4(pack_bf16x2(g[0], g[1]), pack_bf16x2(g[2], 0.0f), pack_bf16x2(g[3], g[4]), pack_bf16x2(g[5], 0.0f));
+          dst[1] = make_uint4(pack_bf16x2(g[6], g[7]), pack_bf16x2(g[8], 0.0f), pack_bf16x2(g[9], g[10]), pack_bf16x2(g[11], 0.0f));
+        }
+        if (p.xhat != nullptr) {   // optional fp32 reconstruction (tests / module API), off the training path
+#pragma unroll
+          for (int qq = 0; qq < 4; ++qq)
+            if (ok[qq]) {
+              const int Y = 2 * i - 1 + (qq >> 1), X = 2 * j - 1 + (qq & 1);
+              float* dstx = p.xhat + (((size_t)n_cur * 64 + Y) * 64 + X) * 3;
+              dstx[0] = xh[3 * qq]; dstx[1] = xh[3 * qq + 1]; dstx[2] = xh[3 * qq + 2];
+            }
+        }
+      } else if constexpr (OUT == LL) {
+#pragma unroll
+        for (int k2 = 0; k2 < 12; ++k2) l1 = fmaf(okf[k2 / 3], fabsf(xv[k2] - xh[k2]), l1);
+      } else {
 #pragma unroll
         for (int qq = 0; qq < 4; ++qq)
           if (ok[qq]) {
             const int Y = 2 * i - 1 + (qq >> 1), X = 2 * j - 1 + (qq & 1);
-            float* dstx = p.xhat + (((size_t)n_cur * 64 + Y) * 64 + X) * 3;
-            dstx[0] = xh[3 * qq]; dstx[1] = xh[3 * qq + 1]; dstx[2] = xh[3 * qq + 2];
+            const size_t o = (((size_t)n_cur * 64 + Y) * 64 + X) * 3;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+              if constexpr (OUT == IMAGE_U8)
+                static_cast<uint8_t*>(p.out)[o + c] = (uint8_t)min(255u, __float2uint_rn(__fmul_rn(255.0f, xh[3 * qq + c])));
+              else
+                static_cast<float*>(p.out)[o + c] = xh[3 * qq + c];
+            }
           }
       }
-      // the likelihood sum leaves the registers once per image (and at the end of the CTA's range), not once per tile:
+      // the likelihood sum leaves the registers once per row (and at the end of the CTA's range), not once per tile:
       // five dependent shuffles per tile were 10 % of the kernel's stall samples
-      if (k == 0 || tile + 1 == tile_end) {
+      if (HAS_X && (k == 0 || tile + 1 == tile_end)) {
         l1 = warp_sum(l1);
         if (lane == 0 && l1 != 0.0f) atomicAdd(p.log_pxz + n_cur, -l1);
         l1 = 0.0f;
       }
       if (threadIdx.x == 64) TL(li, 6);
     }
-    if (p.db != nullptr) {
+    if (OUT == RECON && p.db != nullptr) {
       d0 = warp_sum(d0); d1 = warp_sum(d1); d2 = warp_sum(d2);
       if (lane == 0) { atomicAdd(&s_db[0], d0); atomicAdd(&s_db[1], d1); atomicAdd(&s_db[2], d2); }
     }
@@ -1794,351 +1834,7 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_recon_kernel(const __grid
     p.timeline[40 * 8 + 2 * blockIdx.x + 1] = (long long)gt;
   }
   __syncthreads();
-  if (p.db != nullptr && threadIdx.x < 3 && s_db[threadIdx.x] != 0.0f) atomicAdd(p.db + threadIdx.x, s_db[threadIdx.x]);
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 64);
-  }
-}
-
-// conv5t forward + sigmoid into the image [B,64,64,3] (fp32, or uint8 when U8) - the generation path's last layer.
-// TMA box, taps as descriptor row offsets, barriers, phases and MMA issue are those of convt_recon_kernel with an fp32
-// image operand (XM = 0); only the epilogue differs: it stores the sigmoid of every in-image pixel and nothing else.
-struct alignas(64) CtiParams {
-  CUtensorMap tmA, tmB;
-  const float* bias;   // [3]
-  void* out;           // [B,64,64,3] fp32 or uint8
-  int batch, total_tiles, stages;
-};
-
-template <bool U8>
-__global__ void __launch_bounds__(TG_THREADS, 4) convt_image_kernel(const __grid_constant__ CtiParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
-  constexpr int B_TAP = 1024;
-  constexpr int STAGE = CTR_A_STAGE;
-  uint8_t* sB = smem;                 // 4 taps x [16 rows x 64 B]
-  uint8_t* sA = smem + 4 * B_TAP;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sA + p.stages * STAGE);
-  uint64_t* empty = full + p.stages;
-  uint64_t* tfull = empty + p.stages;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* bfull = tempty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
-  const int per_cta = (p.total_tiles + (int)gridDim.x - 1) / (int)gridDim.x;
-  const int tile_beg = blockIdx.x * per_cta;
-  const int tile_end = min(tile_beg + per_cta, p.total_tiles);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA);
-    tma_prefetch_desc(&p.tmB);
-    for (int s = 0; s < p.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&tfull[s], 1);
-      mbar_init(&tempty[s], 4);
-    }
-    mbar_init(bfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc(tmem_slot, 64);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-
-  if (warp == 0) {
-    if (elect_one() && tile_beg < tile_end) {
-      mbar_expect_tx(bfull, 4 * B_TAP);
-      for (int t = 0; t < 4; ++t) tma_load_2d(sB + t * B_TAP, &p.tmB, bfull, t * 32, 0);
-      int stage = 0;
-      uint32_t ph = 0;
-      int n = tile_beg / 9, k = tile_beg - n * 9;
-      for (int tile = tile_beg; tile < tile_end; ++tile) {
-        const int i_first = (k * 128) / 33;
-        mbar_wait_relaxed(&empty[stage], ph ^ 1);
-        mbar_expect_tx(&full[stage], CTR_BOX_ROWS * 64);
-        tma_load_4d(sA + stage * STAGE, &p.tmA, &full[stage], 0, -1, i_first - 1, n);
-        if (++stage == p.stages) { stage = 0; ph ^= 1; }
-        if (++k == 9) { k = 0; ++n; }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0 && tile_beg < tile_end) {
-      const uint32_t idesc = instr_desc_bf16(128, 16, 0, 0);
-      const uint64_t dproto = smem_desc(0, 16, 8u * 64u, SW_64);
-      const uint64_t adesc0 = dproto + (uint64_t)(smem_u32(sA) >> 4), bdesc0 = dproto + (uint64_t)(smem_u32(sB) >> 4);
-      int stage = 0;
-      uint32_t ph = 0;
-      int k = tile_beg % 9;
-      mbar_wait(bfull, 0);
-      for (int tile = tile_beg; tile < tile_end; ++tile) {
-        const int li = tile - tile_beg, as = li & 1;
-        const int f0 = k * 128, d0 = f0 - (f0 / 33) * 33;
-        mbar_wait(&tempty[as], ((uint32_t)(li >> 1) & 1u) ^ 1u);
-        mbar_wait(&full[stage], ph);
-        tc_fence_after();
-        const uint64_t a_st = adesc0 + (uint64_t)((uint32_t)stage * (STAGE >> 4) + (uint32_t)(d0 + 34) * 4u);
-        const uint32_t tacc = tmem_base + (uint32_t)as * 32u;
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t row_off = (uint32_t)(33 * (t >> 1) + (t & 1)) * 4u;   // tap (a, b) = (t >> 1, t & 1)
-#pragma unroll
-          for (int kk = 0; kk < 2; ++kk)
-            umma_bf16(tacc, a_st - (uint64_t)row_off + (uint64_t)(2 * kk), bdesc0 + (uint64_t)(t * (B_TAP >> 4) + 2 * kk),
-                      idesc, (t > 0 || kk > 0) ? 1u : 0u);
-        }
-        umma_commit(&empty[stage]);
-        umma_commit(&tfull[as]);
-        if (++stage == p.stages) { stage = 0; ph ^= 1; }
-        if (++k == 9) k = 0;
-      }
-    }
-  } else {
-    const int q = warp & 3;
-    const int m = q * 32 + lane;
-    constexpr float LOG2E = 1.4426950408889634f;
-    const float nb0 = -LOG2E * __ldg(p.bias), nb1 = -LOG2E * __ldg(p.bias + 1), nb2 = -LOG2E * __ldg(p.bias + 2);
-    int n = tile_beg / 9, k = tile_beg - n * 9;
-    for (int tile = tile_beg; tile < tile_end; ++tile) {
-      const int li = tile - tile_beg, as = li & 1;
-      const int f = k * 128 + m, i = f / 33, j = f - i * 33;
-      const bool row_ok = f < 33 * 33;
-      const int n_cur = n;
-      if (++k == 9) { k = 0; ++n; }
-      mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
-      tc_fence_after();
-      uint32_t acc[16];
-      tmem_ld16(tmem_base + (uint32_t)as * 32u + ((uint32_t)(q * 32) << 16), acc);
-      tmem_ld_wait();
-      tc_fence_before();
-      if (lane == 0) mbar_arrive(&tempty[as]);
-      // the sigmoid of convt_recon_kernel: xhat = 1 / (1 + 2^(-(a + b) log2 e))
-      float xh[12];
-#pragma unroll
-      for (int k2 = 0; k2 < 12; ++k2) {
-        const int qq = k2 / 3, c = k2 % 3;
-        const float t = fmaf(__uint_as_float(acc[4 * qq + c]), -LOG2E, c == 0 ? nb0 : (c == 1 ? nb1 : nb2));
-        xh[k2] = rcp_approx(1.0f + ex2_approx(t));
-      }
-      // pixel (dy, dx) of block (i, j) lies in the image unless the block touches that border
-      const bool oky[2] = {row_ok && i > 0, row_ok && i < 32}, okx[2] = {j > 0, j < 32};
-#pragma unroll
-      for (int qq = 0; qq < 4; ++qq) {
-        if (!(oky[qq >> 1] && okx[qq & 1])) continue;
-        const int Yp = 2 * i - 1 + (qq >> 1), Xp = 2 * j - 1 + (qq & 1);
-        const size_t o = (((size_t)n_cur * 64 + Yp) * 64 + Xp) * 3;
-        if constexpr (U8) {
-          uint8_t* dst = static_cast<uint8_t*>(p.out) + o;
-#pragma unroll
-          for (int c = 0; c < 3; ++c) dst[c] = (uint8_t)min(255u, __float2uint_rn(__fmul_rn(255.0f, xh[3 * qq + c])));
-        } else {
-          float* dst = static_cast<float*>(p.out) + o;
-          dst[0] = xh[3 * qq]; dst[1] = xh[3 * qq + 1]; dst[2] = xh[3 * qq + 2];
-        }
-      }
-    }
-    tc_fence_before();
-  }
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 64);
-  }
-}
-
-// conv5t forward + sigmoid + Laplace log-likelihood of decoded row n against source image n / kc - the importance-
-// weighted likelihood's last layer.  Pipeline (TMA box, taps as descriptor row offsets, barriers, phases, MMA issue, the
-// XM = 2 bulk copy of the raw-byte blocks) and epilogue arithmetic are those of convt_recon_kernel; the only semantic
-// change is the source image of a row.  No gradient, no reconstruction, no bias gradient.
-struct alignas(64) CtlParams {
-  CUtensorMap tmA, tmB;
-  const void* x;       // the B source images (form XM)
-  const float* bias;   // [3]
-  float* log_pxz;      // [rows], pre-set to -12288 ln 2
-  int rows, kc, total_tiles, stages;
-};
-
-template <int XM>
-__global__ void __launch_bounds__(TG_THREADS, 4) convt_ll_kernel(const __grid_constant__ CtlParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
-  constexpr int B_TAP = 1024;
-  constexpr int STAGE = CTR_A_STAGE + (XM == 2 ? CTR_X_BYTES : 0);
-  uint8_t* sB = smem;
-  uint8_t* sA = smem + 4 * B_TAP;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sA + p.stages * STAGE);
-  uint64_t* empty = full + p.stages;
-  uint64_t* tfull = empty + p.stages;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* bfull = tempty + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
-  float* s_lut = reinterpret_cast<float*>(tmem_slot + 4) + 4;   // [256] uint8 -> float(u) / 255
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  pdl_launch_dependents();
-  const int per_cta = (p.total_tiles + (int)gridDim.x - 1) / (int)gridDim.x;
-  const int tile_beg = blockIdx.x * per_cta;
-  const int tile_end = min(tile_beg + per_cta, p.total_tiles);
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA);
-    tma_prefetch_desc(&p.tmB);
-    for (int s = 0; s < p.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], XM == 2 ? 5 : 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&tfull[s], 1);
-      mbar_init(&tempty[s], 4);
-    }
-    mbar_init(bfull, 1);
-    fence_mbar_init();
-  }
-  for (int i = threadIdx.x; i < 256; i += TG_THREADS) s_lut[i] = g_u8lut[i];
-  if (XM == 2)
-    for (int i = threadIdx.x; i < p.stages * (CTR_X_BYTES / 16); i += TG_THREADS)
-      reinterpret_cast<uint4*>(sA + (i / (CTR_X_BYTES / 16)) * STAGE + CTR_A_STAGE)[i % (CTR_X_BYTES / 16)] = make_uint4(0u, 0u, 0u, 0u);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  if (warp == 2) tmem_alloc(tmem_slot, 64);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-
-  if (warp == 0) {
-    if (elect_one() && tile_beg < tile_end) {
-      mbar_expect_tx(bfull, 4 * B_TAP);
-      for (int t = 0; t < 4; ++t) tma_load_2d(sB + t * B_TAP, &p.tmB, bfull, t * 32, 0);
-      int stage = 0;
-      uint32_t ph = 0;
-      int n = tile_beg / 9, k = tile_beg - n * 9;
-      for (int tile = tile_beg; tile < tile_end; ++tile) {
-        const int i_first = (k * 128) / 33;
-        const uint32_t xbytes = XM == 2 ? (uint32_t)min(128, 33 * 33 - k * 128) * 16u : 0u;
-        mbar_wait_relaxed(&empty[stage], ph ^ 1);
-        mbar_expect_tx(&full[stage], CTR_BOX_ROWS * 64 + xbytes);
-        tma_load_4d(sA + stage * STAGE, &p.tmA, &full[stage], 0, -1, i_first - 1, n);
-        if (XM == 2)   // the raw bytes of the SOURCE image of row n
-          bulk_load_1d(sA + stage * STAGE + CTR_A_STAGE,
-                       reinterpret_cast<const uint4*>(p.x) + ((size_t)(n / p.kc) * 1089 + (size_t)k * 128), xbytes,
-                       &full[stage]);
-        if (++stage == p.stages) { stage = 0; ph ^= 1; }
-        if (++k == 9) { k = 0; ++n; }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0 && tile_beg < tile_end) {
-      const uint32_t idesc = instr_desc_bf16(128, 16, 0, 0);
-      const uint64_t dproto = smem_desc(0, 16, 8u * 64u, SW_64);
-      const uint64_t adesc0 = dproto + (uint64_t)(smem_u32(sA) >> 4), bdesc0 = dproto + (uint64_t)(smem_u32(sB) >> 4);
-      int stage = 0;
-      uint32_t ph = 0;
-      int k = tile_beg % 9;
-      mbar_wait(bfull, 0);
-      for (int tile = tile_beg; tile < tile_end; ++tile) {
-        const int li = tile - tile_beg, as = li & 1;
-        const int f0 = k * 128, d0 = f0 - (f0 / 33) * 33;
-        mbar_wait(&tempty[as], ((uint32_t)(li >> 1) & 1u) ^ 1u);
-        mbar_wait(&full[stage], ph);
-        tc_fence_after();
-        const uint64_t a_st = adesc0 + (uint64_t)((uint32_t)stage * (STAGE >> 4) + (uint32_t)(d0 + 34) * 4u);
-        const uint32_t tacc = tmem_base + (uint32_t)as * 32u;
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-          const uint32_t row_off = (uint32_t)(33 * (t >> 1) + (t & 1)) * 4u;
-#pragma unroll
-          for (int kk = 0; kk < 2; ++kk)
-            umma_bf16(tacc, a_st - (uint64_t)row_off + (uint64_t)(2 * kk), bdesc0 + (uint64_t)(t * (B_TAP >> 4) + 2 * kk),
-                      idesc, (t > 0 || kk > 0) ? 1u : 0u);
-        }
-        umma_commit(&empty[stage]);
-        umma_commit(&tfull[as]);
-        if (++stage == p.stages) { stage = 0; ph ^= 1; }
-        if (++k == 9) k = 0;
-      }
-    }
-  } else {
-    const int q = warp & 3;
-    const int m = q * 32 + lane;
-    constexpr float LOG2E = 1.4426950408889634f;
-    const float nb0 = -LOG2E * __ldg(p.bias), nb1 = -LOG2E * __ldg(p.bias + 1), nb2 = -LOG2E * __ldg(p.bias + 2);
-    using XT = typename std::conditional<XM == 0, float, uint8_t>::type;
-    XT xn[XM == 2 ? 1 : 12];
-    auto fetch_x = [&](int n, int k) {   // the pixels of this thread's block of source image n / kc, one tile ahead
-      if constexpr (XM != 2) {
-        const int f = k * 128 + m;
-        const XT* xs = reinterpret_cast<const XT*>(p.x);
-        const int i = f / 33, j = f - i * 33;
-        const size_t src = (size_t)(n / p.kc);
-#pragma unroll
-        for (int qq = 0; qq < 4; ++qq) {
-          const int Y = min(max(2 * i - 1 + (qq >> 1), 0), 63), X = min(max(2 * j - 1 + (qq & 1), 0), 63);
-          const XT* px = xs + ((src * 64 + Y) * 64 + X) * 3;
-          xn[3 * qq] = __ldg(px); xn[3 * qq + 1] = __ldg(px + 1); xn[3 * qq + 2] = __ldg(px + 2);
-        }
-      }
-    };
-    int n = tile_beg / 9, k = tile_beg - n * 9;
-    if (tile_beg < tile_end) fetch_x(n, k);
-    float l1 = 0.0f;
-    int stage = 0;
-    uint32_t ph = 0;
-    for (int tile = tile_beg; tile < tile_end; ++tile) {
-      const int li = tile - tile_beg, as = li & 1;
-      const int f = k * 128 + m, i = f / 33, j = f - i * 33;
-      const bool row_ok = f < 33 * 33;
-      const int n_cur = n;
-      float xv[12];
-      uint4 xb = make_uint4(0u, 0u, 0u, 0u);
-      if constexpr (XM == 2) {
-        mbar_wait(&full[stage], ph);
-        xb = lds_u4(smem_u32(sA + stage * STAGE + CTR_A_STAGE) + (uint32_t)m * 16u);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&empty[stage]);
-        if (++stage == p.stages) { stage = 0; ph ^= 1; }
-      } else {
-#pragma unroll
-        for (int k2 = 0; k2 < 12; ++k2) xv[k2] = px_value<XT>(xn[k2], s_lut);
-      }
-      if (++k == 9) { k = 0; ++n; }
-      if (tile + 1 < tile_end) fetch_x(n, k);
-      mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
-      tc_fence_after();
-      uint32_t acc[16];
-      tmem_ld16(tmem_base + (uint32_t)as * 32u + ((uint32_t)(q * 32) << 16), acc);
-      tmem_ld_wait();
-      tc_fence_before();
-      if (lane == 0) mbar_arrive(&tempty[as]);
-      if constexpr (XM == 2) {
-        const uint32_t w[3] = {xb.x, xb.y, xb.z};
-#pragma unroll
-        for (int k2 = 0; k2 < 12; ++k2) xv[k2] = s_lut[(w[k2 >> 2] >> (8 * (k2 & 3))) & 0xffu];
-      }
-      const bool oky[2] = {row_ok && i > 0, row_ok && i < 32}, okx[2] = {j > 0, j < 32};
-#pragma unroll
-      for (int k2 = 0; k2 < 12; ++k2) {
-        const int qq = k2 / 3, c = k2 % 3;
-        const float t = fmaf(__uint_as_float(acc[4 * qq + c]), -LOG2E, c == 0 ? nb0 : (c == 1 ? nb1 : nb2));
-        const float xh = rcp_approx(1.0f + ex2_approx(t));
-        l1 = fmaf((oky[qq >> 1] && okx[qq & 1]) ? 1.0f : 0.0f, fabsf(xv[k2] - xh), l1);
-      }
-      if (k == 0 || tile + 1 == tile_end) {   // once per row (and at the end of the CTA's range)
-        l1 = warp_sum(l1);
-        if (lane == 0 && l1 != 0.0f) atomicAdd(p.log_pxz + n_cur, -l1);
-        l1 = 0.0f;
-      }
-    }
-    tc_fence_before();
-  }
-  __syncthreads();
+  if (OUT == RECON && p.db != nullptr && threadIdx.x < 3 && s_db[threadIdx.x] != 0.0f) atomicAdd(p.db + threadIdx.x, s_db[threadIdx.x]);
   if (warp == 2) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 64);
@@ -3153,10 +2849,6 @@ extern "C" int gccvae_tap4_wg_bf16(int batch, const void* in2, const void* S, in
   return GCCVAE_OK;
 }
 
-// Fused conv5t forward (Conv2DTranspose 32 -> 3, k4, s2, same) + sigmoid + Laplace log-likelihood + dLoss/dlogit.
-//   g4 [B,32,32,32] bf16, Wp8 = pack kind 8 ([16][4][32] bf16), bias [3], x [B,64,64,3] fp32 or uint8.
-//   log_pxz[b] = -|x - xhat|_1 - 12288 ln 2.  coef != NULL: D2 [B,33,33,16] bf16 = coef[b] sign(x - xhat) xhat (1 - xhat)
-//   in x2 block form and db[3] += its sums.  xhat (optional): the reconstruction, fp32 [B,64,64,3].
 extern "C" int gccvae_fill_f32(float* p, long long n, float v, void* stream) {
   GCC_REQUIRE(p && n > 0 && n < (1LL << 31), "fill_f32: bad args");
   fill_kernel<<<(int)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p, (int)n, v);
@@ -3164,6 +2856,60 @@ extern "C" int gccvae_fill_f32(float* p, long long n, float v, void* stream) {
   return GCCVAE_OK;
 }
 
+// Launch shape of every conv5t kind: more resident CTAs = more tiles in flight (the per-tile chain TMA -> MMA -> epilogue
+// is latency-bound).  Limits: registers x 192 threads, 64 TMEM columns and the shared memory of convt_smem per CTA.
+// 4 CTAs per SM beat 2 and 3 in the training step (profiles/r01d_ab_log.txt).
+constexpr int CT_PER_SM = 4, CT_STAGES = 3;
+constexpr int convt_smem(bool raw_x) { return 4096 + CT_STAGES * (CTR_A_STAGE + (raw_x ? CTR_X_BYTES : 0)) + 1024 + 2048; }
+static_assert(CT_PER_SM * (convt_smem(true) + 1024) <= 227 * 1024, "conv5t: CT_PER_SM CTAs do not fit in shared memory");
+
+// The common launch of conv5t over `rows` decoded rows of g4 [rows,32,32,32] bf16 (Wp8 = pack kind 8): the tensor maps,
+// the launch shape, and the (out, x_form) instantiation; the caller fills the rest of p.
+static int launch_convt(int out, int rows, const void* g4, const void* Wp8, CtParams& p, int x_form, cudaStream_t st) {
+  static const char* const name[4] = {"convt_recon", "convt_ll", "convt_image", "convt_image"};
+  EncodeTiledFn enc = get_encode();
+  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
+  {
+    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)rows};
+    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
+    cuuint32_t box[4] = {32, 33, 6, 1};   // 6 image rows x (zero column + 32 pixels): CTR_BOX_ROWS rows of 64 bytes
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    GCC_REQUIRE(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled failed: %d", name[out], (int)r);
+  }
+  int rc;
+  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
+  if ((out == RECON || out == LL) && (rc = ensure_u8lut())) return rc;
+  p.total_tiles = rows * 9;
+  p.stages = CT_STAGES;
+  const size_t smem = convt_smem((out == RECON || out == LL) && x_form == 2);
+  using Kernel = void (*)(const CtParams);
+  static const Kernel kernels[4][3] = {{convt_kernel<RECON, 0>, convt_kernel<RECON, 1>, convt_kernel<RECON, 2>},
+                                       {convt_kernel<LL, 0>, convt_kernel<LL, 1>, convt_kernel<LL, 2>},
+                                       {convt_kernel<IMAGE_F32, 0>, nullptr, nullptr},
+                                       {convt_kernel<IMAGE_U8, 0>, nullptr, nullptr}};
+  static bool attr_set[4][3] = {};
+  const Kernel kernel = kernels[out][x_form];
+  if (!attr_set[out][x_form]) {
+    GCC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr_set[out][x_form] = true;
+  }
+  int ctas = p.total_tiles < 148 * CT_PER_SM ? p.total_tiles : 148 * CT_PER_SM;
+  {
+    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
+    ctas = (p.total_tiles + per_cta - 1) / per_cta;
+  }
+  GCC_CUDA(launch_pdl(kernel, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
+  GCC_CHECK_LAUNCH(name[out]);
+  return GCCVAE_OK;
+}
+
+// Fused conv5t forward (Conv2DTranspose 32 -> 3, k4, s2, same) + sigmoid + Laplace log-likelihood + dLoss/dlogit.
+//   g4 [B,32,32,32] bf16, Wp8 = pack kind 8 ([16][4][32] bf16), bias [3], x [B,64,64,3] fp32 or uint8.
+//   log_pxz[b] = -|x - xhat|_1 - 12288 ln 2.  coef != NULL: D2 [B,33,33,16] bf16 = coef[b] sign(x - xhat) xhat (1 - xhat)
+//   in x2 block form and db[3] += its sums.  xhat (optional): the reconstruction, fp32 [B,64,64,3].
 extern "C" int gccvae_convt_recon_bf16(int batch, const void* g4, const void* Wp8, const float* bias, const void* x,
                                        int x_u8, const float* coef, float* log_pxz, void* D2, float* xhat, float* db,
                                        int log_pxz_ready, void* stream) {
@@ -3171,65 +2917,16 @@ extern "C" int gccvae_convt_recon_bf16(int batch, const void* g4, const void* Wp
   GCC_REQUIRE((coef == nullptr) == (D2 == nullptr), "convt_recon: coef and D2 go together");
   GCC_REQUIRE(x_u8 >= 0 && x_u8 <= 2 && (x_u8 != 2 || (uintptr_t)x % 16 == 0), "convt_recon: x_u8 = %d (0 fp32 image, 1 uint8 image, 2 raw-byte blocks, 16-byte aligned)", x_u8);
   cudaStream_t st = (cudaStream_t)stream;
-  CtrParams p;
+  CtParams p;
   memset(&p, 0, sizeof(p));
-  EncodeTiledFn enc = get_encode();
-  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
-  {
-    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)batch};
-    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
-    cuuint32_t box[4] = {32, 33, 6, 1};   // 6 image rows x (zero column + 32 pixels): CTR_BOX_ROWS rows of 64 bytes
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    GCC_REQUIRE(r == CUDA_SUCCESS, "convt_recon: cuTensorMapEncodeTiled failed: %d", (int)r);
-  }
-  int rc;
-  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
   p.x = x; p.x_u8 = x_u8; p.bias = bias; p.coef = coef; p.log_pxz = log_pxz; p.D2 = (uint4*)D2; p.xhat = xhat; p.db = db;
-  p.batch = batch; p.total_tiles = batch * 9;
+  p.batch = batch;
   p.timeline = g_timeline;
-  // CTAs per SM and A stages per CTA: more resident CTAs = more tiles in flight (the per-tile chain TMA -> MMA ->
-  // epilogue is latency-bound).  Limits: registers x 192 threads, 64 TMEM columns and 4 KB + stages x 13 KB of shared
-  // memory per CTA.  GCCVAE_CTR_PER_SM / GCCVAE_CTR_STAGES override (A/B runs).
-  static int env_per_sm = -1, env_stages = -1;
-  if (env_per_sm < 0) {
-    const char* e = getenv("GCCVAE_CTR_PER_SM");
-    env_per_sm = e ? atoi(e) : 0;
-    e = getenv("GCCVAE_CTR_STAGES");
-    env_stages = e ? atoi(e) : 0;
-  }
-  int per_sm = env_per_sm > 0 ? env_per_sm : 4;
-  if (per_sm > 6) per_sm = 6;
-  int stages = env_stages > 0 ? env_stages : 3;
-  if (stages > 4) stages = 4;
-  const int stage_bytes = CTR_A_STAGE + (x_u8 == 2 ? CTR_X_BYTES : 0);
-  while (stages > 1 && per_sm * (4096 + stages * stage_bytes + 1024 + 2048 + 1024) > 227 * 1024) --stages;
-  p.stages = stages;
-  const size_t smem = 4096 + (size_t)stages * stage_bytes + 1024 + 2048;
-  if (int rc2 = ensure_u8lut()) return rc2;
-  static bool attr_set = false;
-  if (!attr_set) {
-    GCC_CUDA(cudaFuncSetAttribute(convt_recon_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    GCC_CUDA(cudaFuncSetAttribute(convt_recon_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    GCC_CUDA(cudaFuncSetAttribute(convt_recon_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    attr_set = true;
-  }
   if (!log_pxz_ready) {   // otherwise the caller pre-set log_pxz[b] = -12288 ln 2 (gccvae_fill_f32) off the critical path
     fill_kernel<<<(batch + 255) / 256, 256, 0, st>>>(log_pxz, batch, (float)(-12288.0 * 0.6931471805599453));
     GCC_CHECK_LAUNCH("recon_fill");
   }
-  int ctas = p.total_tiles < 148 * per_sm ? p.total_tiles : 148 * per_sm;
-  {
-    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
-    ctas = (p.total_tiles + per_cta - 1) / per_cta;
-  }
-  if (x_u8 == 2) GCC_CUDA(launch_pdl(convt_recon_kernel<2>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  else if (x_u8) GCC_CUDA(launch_pdl(convt_recon_kernel<1>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  else GCC_CUDA(launch_pdl(convt_recon_kernel<0>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  GCC_CHECK_LAUNCH("convt_recon");
-  return GCCVAE_OK;
+  return launch_convt(RECON, batch, g4, Wp8, p, x_u8, st);
 }
 
 // conv5t forward + sigmoid into the image (generation path): g4 [B,32,32,32] bf16, Wp8 = pack kind 8, bias [3],
@@ -3240,43 +2937,10 @@ extern "C" int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp
   GCC_REQUIRE(batch > 0 && batch <= (1 << 26), "convt_image: bad batch %d", batch);
   GCC_REQUIRE(out_u8 == 0 || out_u8 == 1, "convt_image: out_u8 = %d (0 fp32, 1 uint8)", out_u8);
   GCC_REQUIRE((uintptr_t)out % 16 == 0 && (uintptr_t)g4 % 16 == 0, "convt_image: out and g4 must be 16-byte aligned");
-  CtiParams p;
+  CtParams p;
   memset(&p, 0, sizeof(p));
-  EncodeTiledFn enc = get_encode();
-  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
-  {   // the A box of convt_recon: 6 image rows x (zero column + 32 pixels)
-    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)batch};
-    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
-    cuuint32_t box[4] = {32, 33, 6, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    GCC_REQUIRE(r == CUDA_SUCCESS, "convt_image: cuTensorMapEncodeTiled failed: %d", (int)r);
-  }
-  int rc;
-  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
-  p.bias = bias; p.out = out; p.batch = batch; p.total_tiles = batch * 9;
-  // the launch shape of convt_recon's default: 4 CTAs per SM, 3 stages of the A box
-  const int per_sm = 4;
-  p.stages = 3;
-  const size_t smem = 4096 + (size_t)p.stages * CTR_A_STAGE + 1024 + 2048;
-  static bool attr_set = false;
-  if (!attr_set) {
-    GCC_CUDA(cudaFuncSetAttribute(convt_image_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    GCC_CUDA(cudaFuncSetAttribute(convt_image_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
-  int ctas = p.total_tiles < 148 * per_sm ? p.total_tiles : 148 * per_sm;
-  {
-    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
-    ctas = (p.total_tiles + per_cta - 1) / per_cta;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  if (out_u8) GCC_CUDA(launch_pdl(convt_image_kernel<true>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  else GCC_CUDA(launch_pdl(convt_image_kernel<false>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  GCC_CHECK_LAUNCH("convt_image");
-  return GCCVAE_OK;
+  p.bias = bias; p.out = out; p.batch = batch;
+  return launch_convt(out_u8 ? IMAGE_U8 : IMAGE_F32, batch, g4, Wp8, p, 0, (cudaStream_t)stream);
 }
 
 // conv5t forward + sigmoid + Laplace log-likelihood of `rows` decoded rows, row r against source image r / kc
@@ -3288,48 +2952,10 @@ extern "C" int gccvae_convt_ll_bf16(int rows, int kc, const void* g4, const void
   GCC_REQUIRE(x_u8 >= 0 && x_u8 <= 2 && (x_u8 != 2 || (uintptr_t)x % 16 == 0),
               "convt_ll: x_u8 = %d (0 fp32 image, 1 uint8 image, 2 raw-byte blocks, 16-byte aligned)", x_u8);
   GCC_REQUIRE((uintptr_t)g4 % 16 == 0, "convt_ll: g4 must be 16-byte aligned");
-  CtlParams p;
+  CtParams p;
   memset(&p, 0, sizeof(p));
-  EncodeTiledFn enc = get_encode();
-  GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
-  {   // the A box of convt_recon: 6 image rows x (zero column + 32 pixels)
-    cuuint64_t dims[4] = {32, 32, 32, (cuuint64_t)rows};
-    cuuint64_t strides[3] = {64, 32 * 64, 32 * 32 * 64};
-    cuuint32_t box[4] = {32, 33, 6, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&p.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(g4), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    GCC_REQUIRE(r == CUDA_SUCCESS, "convt_ll: cuTensorMapEncodeTiled failed: %d", (int)r);
-  }
-  int rc;
-  if ((rc = encode_mat_map(&p.tmB, Wp8, 16, 128, 32, 16))) return rc;
-  p.x = x; p.bias = bias; p.log_pxz = log_pxz; p.rows = rows; p.kc = kc; p.total_tiles = rows * 9;
-  // the launch shape of convt_recon's default: 4 CTAs per SM, 3 stages
-  const int per_sm = 4;
-  p.stages = 3;
-  const int stage_bytes = CTR_A_STAGE + (x_u8 == 2 ? CTR_X_BYTES : 0);
-  const size_t smem = 4096 + (size_t)p.stages * stage_bytes + 1024 + 2048;
-  if (int rc2 = ensure_u8lut()) return rc2;
-  static bool attr_set = false;
-  if (!attr_set) {
-    const int mx = 4096 + 3 * (CTR_A_STAGE + CTR_X_BYTES) + 1024 + 2048;
-    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-    GCC_CUDA(cudaFuncSetAttribute(convt_ll_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx));
-    attr_set = true;
-  }
-  int ctas = p.total_tiles < 148 * per_sm ? p.total_tiles : 148 * per_sm;
-  {
-    const int per_cta = (p.total_tiles + ctas - 1) / ctas;
-    ctas = (p.total_tiles + per_cta - 1) / per_cta;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  if (x_u8 == 2) GCC_CUDA(launch_pdl(convt_ll_kernel<2>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  else if (x_u8) GCC_CUDA(launch_pdl(convt_ll_kernel<1>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  else GCC_CUDA(launch_pdl(convt_ll_kernel<0>, dim3(ctas, 1, 1), TG_THREADS, smem, st, p));
-  GCC_CHECK_LAUNCH("convt_ll");
-  return GCCVAE_OK;
+  p.x = x; p.x_u8 = x_u8; p.bias = bias; p.log_pxz = log_pxz; p.batch = rows; p.kc = kc;
+  return launch_convt(LL, rows, g4, Wp8, p, x_u8, (cudaStream_t)stream);
 }
 
 
