@@ -190,13 +190,6 @@ int gccvae_convt_ll_bf16(int rows, int kc, const void* g4, const void* Wp8, cons
  * phases per CTA from three column-shifted halo boxes (3.6x less L2 traffic than gccvae_sl_bf16), one MMA per
  * shifted view with N = 4*C_L.  Weights packed "sl9" = [9 views][4 phases][C_L padded to 16][C_S]
  * (gccvae_pack_jobs_bf16 kind 6; gccvae_packed_weight_elems(g, 2) elements). */
-/* S -> L of a k4/s2/p1 layer (Conv2DTranspose forward, networks.py:46-48 / Conv2D dgrad of :12-14) in block form: a
- * 2x2-tap gather over S [B,HS,WS,CS] whose rows are the (HS+1) x (WS+1) output blocks of 2x2 pixels and whose
- * N = 4 CL columns are (dy, dx, channel); the epilogue writes every slot to its pixel of L [B,2HS,2WS,CL] (NHWC, or
- * s2d storage with GCCVAE_OUT_S2D; mask likewise with GCCVAE_MASK_S2D).  Wp: pack kind 10, [(dy,dx,cl)][(a,b,cs)]. */
-int gccvae_sl_blk_supported(int HS, int WS, int CS, int CL);
-int gccvae_sl_blk_bf16(int batch, int HS, int WS, int CS, const void* S, const void* Wp, int CL, const float* bias,
-                       int act, const void* mask, void* L, void* stream);
 int gccvae_sl_halo_supported(const gccvae_geom* g);
 int gccvae_sl_halo_bf16(const gccvae_geom* g, const void* S, const void* Wp_sl9, const float* bias, int act,
                         const void* mask, void* L, int out_f32, void* stream);

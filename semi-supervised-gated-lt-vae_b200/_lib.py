@@ -154,8 +154,6 @@ SIGNATURES = {
     "gccvae_colsum_bf16": (_I, [_P, _LL, _I, _I, _P, _P]),
     "gccvae_gemm_bf16": (_I, [_LL, _I, _I, _P, _P, _P, _I, _I, _I, _P, _P, _I, _P]),
     "gccvae_gemm_tn_bf16": (_I, [_LL, _I, _I, _P, _P, C.POINTER(WgOut), _P]),
-    "gccvae_sl_blk_supported": (_I, [_I, _I, _I, _I]),
-    "gccvae_sl_blk_bf16": (_I, [_I, _I, _I, _I, _P, _P, _I, _P, _I, _P, _P, _P]),
     "gccvae_sl_halo_supported": (_I, [_G]),
     "gccvae_sl_halo_bf16": (_I, [_G, _P, _P, _P, _I, _P, _P, _I, _P]),
     "gccvae_cast_f32_to_bf16": (_I, [_P, _LL, _P, _P]),

@@ -80,25 +80,17 @@ __host__ __device__ __forceinline__ float u32_to_unit_open0(uint32_t x) {
 }
 
 #ifdef __CUDACC__
-// Launch with the programmatic-stream-serialization attribute (programmatic dependent launch).  EVERY kernel
-// launched through this helper must execute griddepcontrol.wait before it touches global memory.
-// Measured on B200: PDL pays for the tensor-core kernels (long prologues: 2.30 -> 2.10 ms per step) but NOT for
-// the prologue-less auxiliary kernels routed through this helper (2.10 -> 2.17 ms: their early-scheduled CTAs only
-// occupy SM slots), so for them the attribute is off unless GCCVAE_PDL_AUX=1.
-bool pdl_enabled();
+// Launch of the prologue-less auxiliary kernels, WITHOUT the programmatic-stream-serialization attribute.
+// Measured on B200: programmatic dependent launch pays for the tensor-core kernels (long prologues: 2.30 -> 2.10 ms
+// per step) but NOT for these (2.10 -> 2.17 ms: their early-scheduled CTAs only occupy SM slots).
 template <class... KArgs, class... Args>
-static inline cudaError_t launch_pdl_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                       Args... args) {
-  cudaLaunchConfig_t cfg;
+static inline cudaError_t launch_aux(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                     Args... args) {
+  cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 __device__ __forceinline__ void pdl_prologue() {   // let the successor start, then wait for the predecessor

@@ -62,14 +62,9 @@ struct alignas(64) TapGemmParams {
   int total_items;  // tiles * n_slabs * phases, spread contiguously over the persistent CTAs
   int bias_n;       // number of valid bias entries (channels >= bias_n get no bias)
   long long* timeline;  // debug: block 0 records clock64() at pipeline events [item][8] (NULL = off)
-  float* colsum;        // optional: += column sums of the stored tile (bias gradient of the producer layer)
-  int colsum_n, colsum_mod;
   int out_s2d, mask_s2d;   // the output / the mask tensor is stored in s2d block form (bf16 only)
   int rows_valid;          // rows of the 128-row tile that carry work (TMA box rows); the rest is never stored
-  // S -> L in block form (BLK kernels): the tile's rows are output BLOCKS (i, j) of 2x2 pixels, the N = 4 * blk_cl
-  // columns are (dy, dx, channel); the epilogue scatters the four slots to pixels (2i - 1 + dy, 2j - 1 + dx) of the
-  // OH x OW x OC plane (plain NHWC or s2d storage) and skips the slots outside the plane
-  int blk_cl;
+  int pad_;                // keeps halo2 / a_box_rows 8-byte aligned: the kernel reads the pair with one 64-bit load
   // "halo2" (4-tap L -> S over s2d blocks, full-width tiles of one image): instead of four shifted boxes of BH x BW block
   // rows, TWO column-shifted boxes (b = 0, 1) of (BH + 1) x BW rows are loaded per chunk and the row tap a = 0, 1 is a
   // start-address offset of BW rows (a multiple of the 1 KB swizzle atom) in the A descriptor: (BH + 1) / (2 BH) of the
@@ -88,10 +83,8 @@ struct alignas(64) TapGemmParams {
     if (p.timeline != nullptr && blockIdx.x == 0 && (item_local) < 32)                    \
       p.timeline[(item_local) * 8 + (slot)] = clock64();                                  \
   } while (0)
-#define C3_DBG(p) ((p).dbg)      // GCCVAE_C3_DBG bit switches of c3conv (skip stores / loads / relaxed waits)
 #else
 #define TL_ON(p) false
-#define C3_DBG(p) 0
 #define TL(item_local, slot) \
   do {                       \
   } while (0)
@@ -99,41 +92,6 @@ struct alignas(64) TapGemmParams {
 
 constexpr int TG_THREADS = 192;
 
-// Column sums of a [32 lanes x 16 columns] register tile: recursive halving (16 shuffles) leaves the sum of
-// column `col` in every lane; lanes with an even id add it to the CTA's shared-memory accumulator.
-__device__ __forceinline__ void warp_colsum16(const float (&v)[16], float* s_col, int idx_base, int n_valid_cols,
-                                              int lane) {
-  float w8[8], w4[4], w2[2], w1;
-  const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4, b1 = lane & 2;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const float send = b4 ? v[i] : v[i + 8];
-    const float keep = b4 ? v[i + 8] : v[i];
-    w8[i] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float send = b3 ? w8[i] : w8[i + 4];
-    const float keep = b3 ? w8[i + 4] : w8[i];
-    w4[i] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-  }
-#pragma unroll
-  for (int i = 0; i < 2; ++i) {
-    const float send = b2 ? w4[i] : w4[i + 2];
-    const float keep = b2 ? w4[i + 2] : w4[i];
-    w2[i] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-  }
-  {
-    const float send = b1 ? w2[0] : w2[1];
-    const float keep = b1 ? w2[1] : w2[0];
-    w1 = keep + __shfl_xor_sync(0xffffffffu, send, 2);
-  }
-  w1 += __shfl_xor_sync(0xffffffffu, w1, 1);
-  const int col = (b4 ? 8 : 0) + (b3 ? 4 : 0) + (b2 ? 2 : 0) + (b1 ? 1 : 0);
-  if ((lane & 1) == 0 && col < n_valid_cols) atomicAdd(s_col + idx_base + col, w1);
-}
-
-template <bool COLSUM, bool BLK = false>
 __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_constant__ TapGemmParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -148,13 +106,10 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
   uint64_t* tfull = empty + p.stages;   // [2] accumulator stage ready for the epilogue
   uint64_t* tempty = tfull + 2;         // [2] accumulator stage drained by the epilogue
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
-  float* s_col = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 15) & ~(uintptr_t)15);   // [256] column sums
-  float* s_bias = s_col + 256;                                // [256] bias (zero beyond bias_n)
+  float* s_bias = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 15) & ~(uintptr_t)15);   // [256] bias (zero beyond bias_n)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_launch_dependents();
-  if (COLSUM)
-    for (int i = threadIdx.x; i < 256; i += TG_THREADS) s_col[i] = 0.0f;
   // persistent: this CTA owns a contiguous range of work items; item = (tile, slab, phase), phase fastest,
   // so the 4 output-parity phases that re-read one input tile run back to back on the same SM.
   const int per_cta = (p.total_items + (int)gridDim.x - 1) / (int)gridDim.x;
@@ -322,16 +277,6 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
       for (int i = threadIdx.x - 64; i < 256; i += 128) s_bias[i] = i < nb ? p.bias[i] : 0.0f;
       asm volatile("bar.sync 1, 128;" ::: "memory");
     }
-    // bias-gradient column sums: with a single N slab of <= 64 columns every thread keeps running sums of its own
-    // row in registers across all items and the cross-lane reduction happens once, after the loop
-    float cacc[COLSUM ? 4 : 1][16];
-    if (COLSUM) {
-#pragma unroll
-      for (int a = 0; a < (COLSUM ? 4 : 1); ++a)
-#pragma unroll
-        for (int i = 0; i < 16; ++i) cacc[a][i] = 0.0f;
-    }
-    const bool reg_colsum = COLSUM && p.n_slabs == 1 && p.N <= 64;
     for (int item = item_beg; item < item_end; ++item) {
       const int li = item - item_beg, as = li & 1;
       const int phase_id = item % p.phases, slab = (item / p.phases) % p.n_slabs, tile = item / (p.phases * p.n_slabs);
@@ -340,91 +285,6 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
       const int slab0 = slab * p.N;
       const int n = n0 + dn, y = h0 + dy, x = w0 + dx;
       const bool valid = n < p.batch && m < p.rows_valid;
-      if constexpr (BLK) {
-        // ---- block-form S -> L epilogue: row = block (y, x) of image n, columns = 4 slots x blk_cl channels ----
-        const int CLb = p.blk_cl;
-        const uint32_t tacc = tmem_base + (uint32_t)as * acc_cols + ((uint32_t)(q * 32) << 16);
-        // pixel index of each slot (in units of OC channels), or -1 outside the plane / for rows without work
-        long long spix[4];
-#pragma unroll
-        for (int sl = 0; sl < 4; ++sl) {
-          const int py = 2 * y - 1 + (sl >> 1), px = 2 * x - 1 + (sl & 1);
-          const bool in = valid && py >= 0 && py < p.OH && px >= 0 && px < p.OW;
-          spix[sl] = in ? (long long)(((size_t)n * p.OH + (size_t)py) * p.OW + px) : -1;
-        }
-        // with s2d storage the four slots of a block are consecutive: block index * 4 + slot
-        const long long blk4 = (long long)((((size_t)n * ((p.OH >> 1) + 1) + (size_t)y) * ((p.OW >> 1) + 1) + x) * 4);
-        // the ReLU mask of the whole row (N / 16 chunks of 32 bytes) is fetched before waiting for the accumulator
-        uint32_t mk[8][8];
-        const bool use_mask = p.mask != nullptr;
-        if (use_mask) {
-#pragma unroll
-          for (int ch = 0; ch < 8; ++ch) {
-            const int c0 = ch * 16;
-            if (c0 >= p.N) break;
-            const int sl = c0 / CLb;
-            if (spix[sl] < 0) continue;
-            const long long mp = p.mask_s2d ? blk4 + sl : spix[sl];
-            ld_global_nc_256(reinterpret_cast<const __nv_bfloat16*>(p.mask) + mp * p.OC + (c0 - sl * CLb), mk[ch]);
-          }
-        }
-        mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
-        tc_fence_after();
-        const uint32_t s_bias_u32 = smem_u32(s_bias);
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-          if (half * 128 >= p.N) break;
-#pragma unroll
-          for (int ch = 0; ch < 8; ++ch) {
-            const int c0 = half * 128 + ch * 16;
-            uint32_t r[16];
-            tmem_ld16(tacc + (uint32_t)c0, r);
-            tmem_ld_wait();
-            if (c0 + 16 >= p.N) {  // accumulator fully read: hand the TMEM stage back to the MMA warp
-              tc_fence_before();
-              if (lane == 0) mbar_arrive(&tempty[as]);
-            }
-            const int sl = c0 / CLb, cc = c0 - sl * CLb;
-            if (spix[sl] < 0) continue;
-            const uint32_t bsrc = s_bias_u32 + (uint32_t)(cc * 4);
-            float v[16];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const float4 t = lds_f4(bsrc + 16u * i);
-              v[4 * i] = __uint_as_float(r[4 * i]) + t.x;
-              v[4 * i + 1] = __uint_as_float(r[4 * i + 1]) + t.y;
-              v[4 * i + 2] = __uint_as_float(r[4 * i + 2]) + t.z;
-              v[4 * i + 3] = __uint_as_float(r[4 * i + 3]) + t.w;
-            }
-            if (p.act == GCCVAE_ACT_RELU) {
-#pragma unroll
-              for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], 0.0f);
-            }
-            if (use_mask) {
-              uint32_t mw[8];
-              if (half == 0) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) mw[i] = mk[ch][i];
-              } else {   // N = 256: the second half of the row's mask is fetched here
-                const long long mp = p.mask_s2d ? blk4 + sl : spix[sl];
-                ld_global_nc_256(reinterpret_cast<const __nv_bfloat16*>(p.mask) + mp * p.OC + cc, mw);
-              }
-#pragma unroll
-              for (int i = 0; i < 8; ++i) {
-                const uint32_t lo = mw[i] & 0xffffu, hi = mw[i] >> 16;
-                if (!(lo != 0 && lo < 0x8000u)) v[2 * i] = 0.0f;
-                if (!(hi != 0 && hi < 0x8000u)) v[2 * i + 1] = 0.0f;
-              }
-            }
-            const long long op = p.out_s2d ? blk4 + sl : spix[sl];
-            uint32_t w[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) w[i] = pack_bf16x2(v[2 * i], v[2 * i + 1]);
-            st_global_256(reinterpret_cast<__nv_bfloat16*>(p.out) + op * p.OC + cc, w);
-          }
-        }
-        continue;
-      }
       const int oyy = y * p.oys + p.oy0[phase_id], oxx = x * p.oxs + p.ox0[phase_id];
       const size_t opix_lin = ((size_t)n * p.OH + (size_t)oyy) * p.OW + oxx;
       const size_t opix_s2d = (p.out_s2d | p.mask_s2d) ? s2d_slot(n, oyy, oxx, p.OH, p.OW) : 0;
@@ -460,7 +320,7 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
           if (lane == 0) mbar_arrive(&tempty[as]);
           if (threadIdx.x == 64) TL(li, 5);
         }
-        if ((!valid && !COLSUM) || cg >= p.n_store) continue;
+        if (!valid || cg >= p.n_store) continue;
         float v[16];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -516,38 +376,6 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
             if (!(hi != 0 && hi < 0x8000u)) v[2 * i + 1] = 0.0f;
           }
         }
-        if constexpr (COLSUM) {
-          if (!valid) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = 0.0f;
-          }
-          if (reg_colsum) {
-            switch (c0 >> 4) {   // static indexing keeps cacc[][] in registers
-              case 0:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[0][i] += v[i];
-                break;
-              case 1:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[1][i] += v[i];
-                break;
-              case 2:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[2][i] += v[i];
-                break;
-              default:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[3][i] += v[i];
-                break;
-            }
-          } else {
-            {   // with a wrap (mod) every column of the slab is valid; otherwise columns below colsum_n
-              const int cidx = cg % p.colsum_mod;
-              warp_colsum16(v, s_col, cidx, (p.colsum_mod < (1 << 29) ? p.colsum_mod - cidx : p.colsum_n - cg), lane);
-            }
-          }
-          if (!valid) continue;
-        }
         if (p.out_f32 == 2) {
           // 3-channel image padded to 4 (decoder output): one float4 per pixel, pad channel = 0
           if (c0 == 0) reinterpret_cast<float4*>(p.out)[opix] = make_float4(v[0], v[1], v[2], 0.0f);
@@ -567,12 +395,6 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
       }
       if (threadIdx.x == 64) TL(li, 6);
     }
-    if constexpr (COLSUM) if (reg_colsum) {
-#pragma unroll
-      for (int a = 0; a < 4; ++a)
-        if (a * 16 < p.N && a * 16 < p.colsum_n)
-          warp_colsum16(cacc[a], s_col, (a * 16) % p.colsum_mod, p.colsum_n - a * 16, lane);
-    }
     tc_fence_before();
   }
   __syncthreads();
@@ -580,11 +402,6 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
     unsigned long long gt;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
     p.timeline[40 * 8 + 2 * blockIdx.x + 1] = (long long)gt;
-  }
-  if (COLSUM) {
-    const int ncol = p.colsum_mod < p.colsum_n ? p.colsum_mod : p.colsum_n;
-    for (int i = threadIdx.x; i < ncol; i += TG_THREADS)
-      if (s_col[i] != 0.0f) atomicAdd(p.colsum + i, s_col[i]);
   }
   if (warp == 2) {
     tc_fence_after();
@@ -613,14 +430,11 @@ struct alignas(64) SlHaloParams {
   const float* bias;
   int bias_n, act, out_f32;
   int OH, OW, OC, batch, total_tiles, stages;
-  float* colsum;
-  int colsum_n;
   long long* timeline;  // debug: block 0 records clock64() at pipeline events [tile][8] (NULL = off)
   int mask_s2d;         // the mask tensor is stored in s2d block form
 };
 constexpr int HALO_THREADS = 320;
 
-template <bool COLSUM>
 __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_constant__ SlHaloParams p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -638,7 +452,6 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
   uint64_t* bfull = tempty + 2;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
   float* s_bias = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 15) & ~(uintptr_t)15);   // [256], 16-byte aligned (ld.shared.v4)
-  float* s_col = s_bias + 256;                                // [256] per-CTA column sums
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_launch_dependents();
@@ -663,10 +476,8 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
     fence_mbar_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, tmem_cols);
-  for (int i = threadIdx.x; i < 256; i += HALO_THREADS) {
+  for (int i = threadIdx.x; i < 256; i += HALO_THREADS)
     s_bias[i] = (p.bias != nullptr && i < p.bias_n) ? p.bias[i] : 0.0f;   // parameters: not written by the predecessor
-    s_col[i] = 0.0f;
-  }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -751,13 +562,6 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
     const uint32_t s_bias_u32 = smem_u32(s_bias);
     const int m = q * 32 + lane;
     const int dy = m / p.BW, dx = m % p.BW;
-    float cacc[COLSUM ? 4 : 1][16];   // running column sums of this thread's rows (bias gradient)
-    if (COLSUM) {
-#pragma unroll
-      for (int a = 0; a < (COLSUM ? 4 : 1); ++a)
-#pragma unroll
-        for (int i = 0; i < 16; ++i) cacc[a][i] = 0.0f;
-    }
     for (int tile = tile_beg; tile < tile_end; ++tile) {
       const int li = tile - tile_beg, as = li & 1;
       const int n = tile / p.tiles_h, h0 = (tile % p.tiles_h) * p.BH;
@@ -834,26 +638,6 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
               if (!(hi != 0 && hi < 0x8000u)) v[2 * i + 1] = 0.0f;
             }
           }
-          if constexpr (COLSUM) {
-            switch (c0 >> 4) {
-              case 0:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[0][i] += v[i];
-                break;
-              case 1:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[1][i] += v[i];
-                break;
-              case 2:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[2][i] += v[i];
-                break;
-              default:
-#pragma unroll
-                for (int i = 0; i < 16; ++i) cacc[3][i] += v[i];
-                break;
-            }
-          }
           if (p.out_f32 == 2) {
             if (c0 == 0) reinterpret_cast<float4*>(p.out)[opix[j]] = make_float4(v[0], v[1], v[2], 0.0f);
           } else if (p.out_f32) {
@@ -873,17 +657,9 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
       }
       if (threadIdx.x == 64) TL(li, 6);
     }
-    if constexpr (COLSUM) {
-#pragma unroll
-      for (int a = 0; a < 4; ++a)
-        if (a * 16 < p.N && a * 16 < p.colsum_n) warp_colsum16(cacc[a], s_col, a * 16, p.colsum_n - a * 16, lane);
-    }
     tc_fence_before();
   }
   __syncthreads();
-  if (COLSUM)
-    for (int i = threadIdx.x; i < p.colsum_n; i += HALO_THREADS)
-      if (s_col[i] != 0.0f) atomicAdd(p.colsum + i, s_col[i]);
   if (warp == 2) {
     tc_fence_after();
     tmem_dealloc(tmem_base, tmem_cols);
@@ -901,17 +677,13 @@ __global__ void __launch_bounds__(HALO_THREADS) sl_halo_kernel(const __grid_cons
 struct alignas(64) WgParams {
   CUtensorMap tmA, tmB;
   int blocks_per_mtile, blocks_per_tap, taps, kcA, b_loads, kcB, swzA, swzB;
-  int c4_rows;  // rows are (tap, c4): scatter row m -> (m/4)*3 + m%4, dropping the pad channel
+  int c4_rows;  // 0: dW rows as computed; 2: x2 rows, 3: s2d rows, scattered to Keras (kh, kw, c) order (see the epilogue)
   int a_scale, BW, BH, BN, tiles_w, tiles_h;
   short a_dw[16], a_dh[16];
   int N;
   int tiles_total, tiles_per_cta;
   gccvae_wg_out out;   // destination segments (columns -> tensors); out.m_valid rows are stored
   int stages;
-  // bias gradient fused into the main loop (the four epilogue warps are idle there): column sums of the
-  // S operand (side 1: Conv2D / Dense, dout = S) or of the L operand's own-pixel taps (side 2: Conv2DTranspose)
-  float* colsum;
-  int colsum_side, colsum_n;
   // x2 mode: the A operand (128 pixels x 64 (a,b,dy,dx,c4) values, 128-byte rows) is built by warps 2-5 with cp.async
   // from the [B,33,33,16] block tensor instead of 8 TMA boxes of 32-byte rows (TMA is row-rate bound)
   const uint4* in2;
@@ -932,24 +704,10 @@ __global__ void __launch_bounds__(TG_THREADS) wgrad_kernel(const __grid_constant
   uint64_t* empty = full + p.stages;
   uint64_t* tmem_full = empty + p.stages;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-  float* s_red = reinterpret_cast<float*>(tmem_slot + 4);   // [4 slabs][64 channels] column-sum staging
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_launch_dependents();
   const int mtile = blockIdx.y;
-  // which smem slabs of this CTA feed the fused bias gradient (bit s = slab s)
-  uint32_t cs_mask = 0;
-  if (p.colsum != nullptr) {
-    if (p.colsum_side == 1) {
-      if (mtile == 0) cs_mask = (1u << p.b_loads) - 1u;
-    } else {
-      for (int bl = 0; bl < p.blocks_per_mtile; ++bl) {
-        const int t = (mtile * p.blocks_per_mtile + bl) / p.blocks_per_tap;
-        const int kh = t >> 2, kw = t & 3;   // k4/s2/p1: taps (1..2, 1..2) visit every L pixel exactly once
-        if (t < p.taps && (kh == 1 || kh == 2) && (kw == 1 || kw == 2)) cs_mask |= 1u << bl;
-      }
-    }
-  }
   const int tile_beg = blockIdx.x * p.tiles_per_cta;
   int tile_end = tile_beg + p.tiles_per_cta;
   if (tile_end > p.tiles_total) tile_end = p.tiles_total;
@@ -962,7 +720,7 @@ __global__ void __launch_bounds__(TG_THREADS) wgrad_kernel(const __grid_constant
     tma_prefetch_desc(&p.tmB);
     for (int s = 0; s < p.stages; ++s) {
       mbar_init(&full[s], p.in2 != nullptr ? 129 : 1);   // TMA transaction (+ one cp.async arrival per A-builder thread)
-      mbar_init(&empty[s], cs_mask ? 5 : 1);   // MMA commit (+ the four column-sum warps)
+      mbar_init(&empty[s], 1);
     }
     mbar_init(tmem_full, 1);
     fence_mbar_init();
@@ -1072,56 +830,6 @@ __global__ void __launch_bounds__(TG_THREADS) wgrad_kernel(const __grid_constant
           if (++stage == p.stages) { stage = 0; ph ^= 1; }
         }
       }
-      if (cs_mask) {
-        // ---- fused bias gradient: column sums of the staged operand tiles, straight from shared memory ----
-        const bool sideS = p.colsum_side == 1;
-        const int kc = sideS ? p.kcB : p.kcA, rowb = kc * 2, slab = sideS ? b_slab : a_slab;
-        const uint32_t swmask = (rowb >= 128) ? 7u : ((rowb >= 64) ? 3u : 1u);
-        const int t = threadIdx.x - 64, pairs = kc >> 1, tpp = 128 / pairs;
-        const int pair = t % pairs, rg = t / pairs;
-        float acc[4][2];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) acc[i][0] = acc[i][1] = 0.0f;
-        int stage = 0;
-        uint32_t ph = 0;
-        for (int it = 0; it < n_tiles; ++it) {
-          mbar_wait(&full[stage], ph);
-          const uint8_t* tile0 = (sideS ? sB + stage * b_bytes : sA + stage * a_bytes);
-#pragma unroll
-          for (int sl = 0; sl < 4; ++sl) {
-            if (!((cs_mask >> sl) & 1u)) continue;
-            const uint8_t* sbase = tile0 + sl * slab;
-            float a0 = 0.0f, a1 = 0.0f;
-            for (int r = rg; r < 128; r += tpp) {
-              uint32_t off = (uint32_t)(r * rowb + pair * 4);
-              off ^= ((off >> 7) & swmask) << 4;
-              const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(sbase + off);
-              a0 += __low2float(v);
-              a1 += __high2float(v);
-            }
-            acc[sl][0] += a0;
-            acc[sl][1] += a1;
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&empty[stage]);
-          if (++stage == p.stages) { stage = 0; ph ^= 1; }
-        }
-        for (int i = t; i < 256; i += 128) s_red[i] = 0.0f;
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-#pragma unroll
-        for (int sl = 0; sl < 4; ++sl)
-          if ((cs_mask >> sl) & 1u) {
-            atomicAdd(&s_red[sl * 64 + pair * 2], acc[sl][0]);
-            atomicAdd(&s_red[sl * 64 + pair * 2 + 1], acc[sl][1]);
-          }
-        asm volatile("bar.sync 1, 128;" ::: "memory");
-        for (int i = t; i < 256; i += 128) {
-          const int sl = i >> 6, c = i & 63;
-          if (!((cs_mask >> sl) & 1u) || c >= kc) continue;
-          const int ch = sideS ? sl * kc + c : ((mtile * p.blocks_per_mtile + sl) % p.blocks_per_tap) * kc + c;
-          if (ch < p.colsum_n && s_red[i] != 0.0f) atomicAdd(p.colsum + ch, s_red[i]);
-        }
-      }
       const int q = warp & 3;
       const int m = mtile * 128 + q * 32 + lane;
       mbar_wait(tmem_full, 0);
@@ -1131,8 +839,8 @@ __global__ void __launch_bounds__(TG_THREADS) wgrad_kernel(const __grid_constant
         uint32_t r[16];
         tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
         tmem_ld_wait();
-        // c4_rows 1: rows are (tap16, c4) -> (tap16, c3);  2: x2 rows (a, b, dy, dx, c4) -> ((2a+dy)*4 + 2b+dx, c3)
-        //             3: s2d rows (a, b, dy, dx, c < CL) -> ((2a+dy)*4 + 2b+dx, c)   [CL = p.kcB_unused / out.cl]
+        // c4_rows 2: x2 rows (a, b, dy, dx, c4) -> ((2a+dy)*4 + 2b+dx, c3)
+        //         3: s2d rows (a, b, dy, dx, c < CL) -> ((2a+dy)*4 + 2b+dx, c)   [CL = p.kcB_unused / out.cl]
         int mrow;
         if (p.c4_rows == 3) {
           const int CL = p.s2d_cl, t = m / (4 * CL), r = m - t * 4 * CL, sub = r / CL, c = r - sub * CL;
@@ -1140,14 +848,14 @@ __global__ void __launch_bounds__(TG_THREADS) wgrad_kernel(const __grid_constant
         } else {
           mrow = p.c4_rows == 2
                      ? ((2 * (m >> 5) + ((m >> 3) & 1)) * 4 + 2 * ((m >> 4) & 1) + ((m >> 2) & 1)) * 3 + (m & 3)
-                     : (p.c4_rows ? ((m >> 2) * 3 + (m & 3)) : m);
+                     : m;
         }
         if (p.ones_db != nullptr && m == 15) {
 #pragma unroll
           for (int i = 0; i < 16; ++i)
             if (c0 + i < p.N) atomicAdd(p.ones_db + c0 + i, __uint_as_float(r[i]));
         }
-        if (m < p.out.m_valid && !((p.c4_rows == 1 || p.c4_rows == 2) && (m & 3) == 3)) {
+        if (m < p.out.m_valid && !(p.c4_rows == 2 && (m & 3) == 3)) {
 #pragma unroll
           for (int sg = 0; sg < 2; ++sg) {
             if (sg >= p.out.n_seg) break;
@@ -1328,17 +1036,6 @@ __global__ void __launch_bounds__(256) pack_jobs_kernel(const __grid_constant__ 
       const int t = k / (4 * CL), r = k % (4 * CL), sub = r / CL, c = r % CL;
       const int kh = 2 * (t >> 1) + (sub >> 1), kw = 2 * (t & 1) + (sub & 1);
       out[i] = __float2bfloat16(cs < CS ? W[((size_t)(kh * 4 + kw) * CL + c) * CS + cs] : 0.0f);
-    }
-  } else if (jb.kind == 10) {
-    // block-form S -> L packing of a k4/s2/p1 kernel W[kh,kw,CL,CS]: out[(dy,dx,cl)][(a,b,cs)], kh = 2a+dy, kw = 2b+dx
-    // (B operand of the 4-tap S -> L GEMM whose rows are output blocks: gccvae_sl_blk_bf16; N = 4 CL, K = 4 CS)
-    const int K = 4 * CS;
-    const long long n = (long long)4 * CL * K;
-    for (long long i = i0; i < n; i += stride) {
-      const int row = (int)(i / K), k = (int)(i % K);
-      const int sub = row / CL, cl = row % CL, t = k / CS, cs = k % CS;
-      const int kh = 2 * (t >> 1) + (sub >> 1), kw = 2 * (t & 1) + (sub & 1);
-      out[i] = __float2bfloat16(W[((size_t)(kh * 4 + kw) * CL + cl) * CS + cs]);
     }
   } else if (jb.kind == 7 || jb.kind == 8) {
     // x2 (space-to-depth) packing of a 3-channel k4/s2/p1 kernel W[kh,kw,3,CS]:
@@ -1857,9 +1554,7 @@ struct alignas(64) C3Params {
   const float* bias;        // optional [N]
   int act, N, batch, total_tiles, stages;
   int out_s2d;              // store the 32x32xN output in s2d block form [B,17,17,4N]
-  float* colsum;            // optional: += column sums of the stored values (bias gradient of the producer layer)
   long long* timeline;      // debug (see TL)
-  int dbg;                  // debug: bit 0 = no output stores, bit 1 = no cp.async (tile content undefined)
 };
 constexpr int C3_THREADS = 288;
 
@@ -1879,7 +1574,6 @@ __global__ void __launch_bounds__(C3_THREADS, 2) c3conv_kernel(const __grid_cons
   uint64_t* bfull = tempty + ACC;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bfull + 1);
   float* s_bias = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 15) & ~(uintptr_t)15);   // [64]
-  float* s_col = s_bias + 64;                                                                                     // [64]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_launch_dependents();
@@ -1923,13 +1617,11 @@ __global__ void __launch_bounds__(C3_THREADS, 2) c3conv_kernel(const __grid_cons
     for (int tile = tile_beg; tile < tile_end; ++tile) {
       const int n = tile >> 3, h0 = (tile & 7) * 4;
       const uint4* src = p.in2 + (((size_t)n * 33 + (h0 + dy)) * 33 + dx) * 2;
-      if (C3_DBG(p) & 4) mbar_wait(&empty[stage], ph ^ 1);
-      else mbar_wait_relaxed(&empty[stage], ph ^ 1);
+      mbar_wait_relaxed(&empty[stage], ph ^ 1);
       if (m == 0) TL(tile - tile_beg, 0);
       const uint32_t dst = smem_u32(sA + stage * A_TILE) + row_off;
 #pragma unroll
       for (int t = 0; t < 4; ++t) {
-        if (C3_DBG(p) & 2) break;
         const uint4* sp = src + ((t >> 1) * 33 + (t & 1)) * 2;
 #pragma unroll
         for (int h = 0; h < 2; ++h)
@@ -1976,10 +1668,7 @@ __global__ void __launch_bounds__(C3_THREADS, 2) c3conv_kernel(const __grid_cons
     // L2 round trip on the epilogue's critical path
     {
       const int et = threadIdx.x - 160;
-      if (et < 64) {
-        s_bias[et] = (p.bias != nullptr && et < p.N) ? p.bias[et] : 0.0f;
-        s_col[et] = 0.0f;
-      }
+      if (et < 64) s_bias[et] = (p.bias != nullptr && et < p.N) ? p.bias[et] : 0.0f;
       asm volatile("bar.sync 1, 128;" ::: "memory");
     }
     const uint32_t s_bias_u32 = smem_u32(s_bias);
@@ -2044,18 +1733,16 @@ __global__ void __launch_bounds__(C3_THREADS, 2) c3conv_kernel(const __grid_cons
             if (!(hi != 0 && hi < 0x8000u)) v[2 * i + 1] = 0.0f;
           }
         }
-        if (p.colsum != nullptr) warp_colsum16(v, s_col, c0, p.N - c0, lane);   // bias gradient of the producer layer
         uint32_t w[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) w[i] = pack_bf16x2(v[2 * i], v[2 * i + 1]);
-        if (!(C3_DBG(p) & 1)) st_global_256(reinterpret_cast<__nv_bfloat16*>(p.out) + opix * p.N + c0, w);
+        st_global_256(reinterpret_cast<__nv_bfloat16*>(p.out) + opix * p.N + c0, w);
       }
       if (threadIdx.x == 160) TL(li, 6);
     }
     tc_fence_before();
   }
   __syncthreads();
-  if (p.colsum != nullptr && threadIdx.x < p.N && s_col[threadIdx.x] != 0.0f) atomicAdd(p.colsum + threadIdx.x, s_col[threadIdx.x]);
   if (warp == 4) {
     tc_fence_after();
     tmem_dealloc(tmem_base, acc_cols * ACC);
@@ -2122,11 +1809,6 @@ __global__ void cast_f32_kernel(const __nv_bfloat16* __restrict__ in, long long 
 // ---------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------
-// (the column-sum epilogues of the dgrad / wgrad kernels - bias gradients fused into the producing launch - were measured
-// slower than the separate bandwidth-bound pass on B200 and have no entry point any more; the kernels keep the hooks)
-static float* g_colsum = nullptr;
-static int g_colsum_n = 0, g_colsum_mod = 0;
-
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -2223,30 +1905,14 @@ static int pick_tile(int H, int W, int* bw, int* bh, int* bn) {
   return 0;
 }
 
-static bool g_pdl = true;   // programmatic dependent launch for the tensor-core kernels (GCCVAE_PDL=0 disables)
-
 // CTAs per SM of the weight-gradient kernels and their shared-memory budget per CTA (KB).  They run on a side stream
 // UNDER the dgrad chain: what they occupy is not available to the critical path's persistent CTAs.
-static int wg_per_sm() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GCCVAE_WG_PER_SM"); v = e ? atoi(e) : 2; if (v < 1) v = 1; if (v > 2) v = 2; }
-  return v;
-}
-static int wg_smem_kb() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GCCVAE_WG_SMEM_KB"); v = e ? atoi(e) : 100; if (v < 40) v = 40; if (v > 190) v = 190; }
-  return v;
-}
+constexpr int WG_PER_SM = 2, WG_SMEM_KB = 100;
 
+// tensor-core kernels: launched with programmatic dependent launch (their prologues overlap the predecessor's tail)
 template <class Params>
 static cudaError_t launch_pdl(void (*kernel)(const Params), dim3 grid, int threads, size_t smem, cudaStream_t st,
                               const Params& p) {
-  static bool env_read = false;
-  if (!env_read) {
-    const char* e = getenv("GCCVAE_PDL");
-    if (e && e[0] == '0') g_pdl = false;
-    env_read = true;
-  }
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid;
@@ -2257,7 +1923,7 @@ static cudaError_t launch_pdl(void (*kernel)(const Params), dim3 grid, int threa
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, p);
 }
 
@@ -2265,43 +1931,24 @@ static long long* g_timeline = nullptr;
 
 static int launch_tapgemm(TapGemmParams& p, int groups, int phases, cudaStream_t st, const char* name) {
   p.timeline = g_timeline;
-  p.colsum = g_colsum; p.colsum_n = g_colsum_n; p.colsum_mod = g_colsum_mod > 0 ? g_colsum_mod : (1 << 30);
-  g_colsum = nullptr;
-  if (p.colsum) {
-    GCC_REQUIRE(p.colsum_n > 0 && (p.colsum_mod >= p.colsum_n ? p.colsum_n : p.colsum_mod) <= 256 &&
-                    (p.colsum_mod >= (1 << 29) || p.colsum_mod % 16 == 0),
-                "%s: unsupported column-sum shape (n=%d mod=%d)", name, p.colsum_n, p.colsum_mod);
-  }
   if (p.rows_valid <= 0) p.rows_valid = 128;
   if (p.a_box_rows <= 0) p.a_box_rows = 128;
-  const bool blk = p.blk_cl > 0;
-  GCC_REQUIRE(!blk || p.colsum == nullptr, "%s: no fused column sums in block form", name);
   const int a_stride = (p.a_box_rows * p.KC * 2 + 1023) & ~1023,
             b_stride = ((p.halo2 ? 2 : 1) * p.N * p.KC * 2 + 1023) & ~1023;
   // Persistent CTAs, `per_sm` of them per SM (their epilogues and issue threads overlap).  The single MMA-issuing
   // thread pays ~400 cycles per pipeline stage (barrier wait, fences, commit) and ~50 per MMA, so a stage carries
   // `tps` k-blocks (taps x chunks): few, fat stages.  TMEM: two accumulator stages per CTA, 512 columns per SM.
-  static int env_tps = -1, env_per_sm = -1, env_stage_kb = -1;
-  if (env_tps < 0) {
-    const char* e = getenv("GCCVAE_TPS");
-    env_tps = e ? atoi(e) : 0;
-    e = getenv("GCCVAE_TG_PER_SM");
-    env_per_sm = e ? atoi(e) : 0;
-    e = getenv("GCCVAE_STAGE_KB");
-    env_stage_kb = e ? atoi(e) : 0;
-  }
   uint32_t acc_cols = 32;
   while ((int)acc_cols < p.N) acc_cols <<= 1;
   const int k_iters = p.num_taps * p.chunks;
-  int per_sm = env_per_sm > 0 ? env_per_sm : 2;
+  int per_sm = 2;
   if (per_sm > 512 / (2 * (int)acc_cols)) per_sm = 512 / (2 * (int)acc_cols);
   if (per_sm < 1) per_sm = 1;
   const int budget = 200 * 1024 / per_sm - 4608;
-  const int stage_target = (env_stage_kb > 0 ? env_stage_kb : 48) * 1024;
+  const int stage_target = 48 * 1024;
   int tps = 1;
   for (int d = 1; d <= k_iters; ++d)
     if (k_iters % d == 0 && d * (a_stride + b_stride) <= stage_target && 2 * d * (a_stride + b_stride) <= budget) tps = d;
-  if (env_tps > 0 && k_iters % env_tps == 0 && 2 * env_tps * (a_stride + b_stride) <= budget) tps = env_tps;
   p.tps = tps;
   int stages = budget / (tps * (a_stride + b_stride));
   if (stages > 8) stages = 8;
@@ -2310,33 +1957,28 @@ static int launch_tapgemm(TapGemmParams& p, int groups, int phases, cudaStream_t
   const size_t smem = (size_t)stages * tps * (a_stride + b_stride) + 1024 + 256 + 2048 + 64;
   static bool attr_set = false;
   if (!attr_set) {
-    GCC_CUDA(cudaFuncSetAttribute(tapgemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    GCC_CUDA(cudaFuncSetAttribute(tapgemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    GCC_CUDA(cudaFuncSetAttribute(tapgemm_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
+    GCC_CUDA(cudaFuncSetAttribute(tapgemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
     attr_set = true;
   }
   GCC_REQUIRE(smem <= 200 * 1024, "%s: %zu bytes of shared memory", name, smem);
   if (p.n_slabs < 1) p.n_slabs = 1;
   if (p.bias_mod < 1 || p.bias == nullptr) p.bias_mod = 1 << 30;
   if (p.bias_n < 1) p.bias_n = p.n_store;
-  GCC_REQUIRE(blk || p.bias_mod >= p.n_store || p.bias_mod % p.N == 0, "%s: bias_mod %d incompatible with N slab %d", name,
+  GCC_REQUIRE(p.bias_mod >= p.n_store || p.bias_mod % p.N == 0, "%s: bias_mod %d incompatible with N slab %d", name,
               p.bias_mod, p.N);
   GCC_REQUIRE(p.bias == nullptr || ((uintptr_t)p.bias % 16) == 0, "%s: bias must be 16-byte aligned", name);
   p.phases = phases;
   p.total_items = groups * p.tiles_w * p.tiles_h * p.n_slabs * phases;
   // never launch more persistent CTAs than are resident at once: a second wave would serialise behind the first.
   // Residency limits: registers (64K per SM), shared memory (227 KB per SM, 1 KB reserved per CTA), TMEM (above).
-  static int regs_per_cta[3] = {0, 0, 0};
-  const int ki = blk ? 2 : (p.colsum != nullptr ? 1 : 0);
-  if (regs_per_cta[ki] == 0) {
+  static int regs_per_cta = 0;
+  if (regs_per_cta == 0) {
     cudaFuncAttributes fa;
-    if (ki == 2) GCC_CUDA(cudaFuncGetAttributes(&fa, tapgemm_kernel<false, true>));
-    else if (ki) GCC_CUDA(cudaFuncGetAttributes(&fa, tapgemm_kernel<true>));
-    else GCC_CUDA(cudaFuncGetAttributes(&fa, tapgemm_kernel<false>));
+    GCC_CUDA(cudaFuncGetAttributes(&fa, tapgemm_kernel));
     const int per_warp = ((fa.numRegs + 7) / 8) * 8 * 32;
-    regs_per_cta[ki] = per_warp * (TG_THREADS / 32);
+    regs_per_cta = per_warp * (TG_THREADS / 32);
   }
-  int occ = 65536 / regs_per_cta[ki];
+  int occ = 65536 / regs_per_cta;
   const int occ_smem = (int)((227 * 1024) / (smem + 1024));
   if (occ > occ_smem) occ = occ_smem;
   if (occ < 1) occ = 1;
@@ -2351,9 +1993,7 @@ static int launch_tapgemm(TapGemmParams& p, int groups, int phases, cudaStream_t
     ctas = (p.total_items + per_cta - 1) / per_cta;
   }
   dim3 grid(ctas, 1, 1);
-  if (blk) GCC_CUDA(launch_pdl(tapgemm_kernel<false, true>, grid, TG_THREADS, smem, st, p));
-  else if (p.colsum != nullptr) GCC_CUDA(launch_pdl(tapgemm_kernel<true>, grid, TG_THREADS, smem, st, p));
-  else GCC_CUDA(launch_pdl(tapgemm_kernel<false>, grid, TG_THREADS, smem, st, p));
+  GCC_CUDA(launch_pdl(tapgemm_kernel, grid, TG_THREADS, smem, st, p));
   GCC_CHECK_LAUNCH(name);
   return GCCVAE_OK;
 }
@@ -2506,13 +2146,6 @@ static int wg_bf16_impl(const gccvae_geom* g, const void* L, const void* S, cons
   if ((rc = encode_act_map(&p.tmB, S, g->batch, g->HS, g->WS, CS, p.kcB, bw, bh, bn, 1))) return rc;
   p.BW = bw; p.BH = bh; p.BN = bn; p.tiles_w = g->WS / bw; p.tiles_h = g->HS / bh;
   p.N = CS; p.out = *out;
-  if (g_colsum != nullptr && g_colsum_mod < 0) {   // armed by gccvae_next_launch_colsum(ptr, n, -1 | -2)
-    p.colsum = g_colsum; p.colsum_n = g_colsum_n; p.colsum_side = -g_colsum_mod;
-    g_colsum = nullptr;
-    GCC_REQUIRE(p.colsum_side == 1 || (p.colsum_side == 2 && !dense && !c4_rows),
-                "wg_bf16: fused bias gradient side %d unsupported here", p.colsum_side);
-    GCC_REQUIRE(p.colsum_n > 0 && p.colsum_n <= (p.colsum_side == 1 ? CS : CL), "wg_bf16: colsum_n");
-  }
   const int groups = (g->batch + bn - 1) / bn;
   p.tiles_total = groups * p.tiles_w * p.tiles_h;
   const int mtiles = (taps * p.blocks_per_tap + p.blocks_per_mtile - 1) / p.blocks_per_mtile;
@@ -2570,11 +2203,11 @@ extern "C" int gccvae_colsum_bf16(const void* in, long long rows, int cols, int 
   const int rpc = (int)((rows + ctas - 1) / ctas);
   ctas = (rows + rpc - 1) / rpc;
   if (cols % 8 == 0 && 256 % (cols / 8) == 0 && (uintptr_t)in % 16 == 0)
-    GCC_CUDA(launch_pdl_k(colsum_bf16_v8_kernel, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream,
-                          (const __nv_bfloat16*)in, rows, cols, rpc, n_valid, out));
+    GCC_CUDA(launch_aux(colsum_bf16_v8_kernel, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream,
+                        (const __nv_bfloat16*)in, rows, cols, rpc, n_valid, out));
   else
-    GCC_CUDA(launch_pdl_k(colsum_bf16_kernel, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream,
-                          (const __nv_bfloat16*)in, rows, cols, rpc, n_valid, out));
+    GCC_CUDA(launch_aux(colsum_bf16_kernel, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream,
+                        (const __nv_bfloat16*)in, rows, cols, rpc, n_valid, out));
   GCC_CHECK_LAUNCH("colsum_bf16");
   return GCCVAE_OK;
 }
@@ -2653,10 +2286,7 @@ extern "C" int gccvae_sl_halo_bf16(const gccvae_geom* g, const void* S, const vo
   GCC_REQUIRE(!(act & GCCVAE_OUT_S2D), "sl_halo: s2d output is not supported");
   hp.OH = g->HL; hp.OW = g->WL; hp.OC = g->CL; hp.batch = g->batch;
   hp.total_tiles = g->batch * hp.tiles_h;
-  hp.colsum = g_colsum; hp.colsum_n = g_colsum_n;
-  g_colsum = nullptr;
   hp.timeline = g_timeline;
-  GCC_REQUIRE(hp.colsum == nullptr || (hp.colsum_n > 0 && hp.colsum_n <= 256), "sl_halo: colsum_n");
   const int rowb = g->CS * 2, a_stage = 3 * (bh + 2) * bw * rowb, b_bytes = (9 * 4 * rows_pad * rowb + 1023) & ~1023;
   int stages = (196 * 1024 - b_bytes - 5120) / a_stage;
   if (stages > 5) stages = 5;
@@ -2665,15 +2295,11 @@ extern "C" int gccvae_sl_halo_bf16(const gccvae_geom* g, const void* S, const vo
   const size_t smem = (size_t)b_bytes + (size_t)stages * a_stage + 1024 + 3072;
   static bool attr_set = false;
   if (!attr_set) {
-    GCC_CUDA(cudaFuncSetAttribute(sl_halo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    GCC_CUDA(cudaFuncSetAttribute(sl_halo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
+    GCC_CUDA(cudaFuncSetAttribute(sl_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
     attr_set = true;
   }
   const int ctas = hp.total_tiles < 148 ? hp.total_tiles : 148;
-  if (hp.colsum != nullptr)
-    GCC_CUDA(launch_pdl(sl_halo_kernel<true>, dim3(ctas, 1, 1), HALO_THREADS, smem, (cudaStream_t)stream, hp));
-  else
-    GCC_CUDA(launch_pdl(sl_halo_kernel<false>, dim3(ctas, 1, 1), HALO_THREADS, smem, (cudaStream_t)stream, hp));
+  GCC_CUDA(launch_pdl(sl_halo_kernel, dim3(ctas, 1, 1), HALO_THREADS, smem, (cudaStream_t)stream, hp));
   GCC_CHECK_LAUNCH("sl_halo_bf16");
   return GCCVAE_OK;
 }
@@ -2691,14 +2317,14 @@ extern "C" int gccvae_prep_x2_bf16(const void* x, int x_u8, int batch, void* X2,
   if (ctas > 148 * 16) ctas = 148 * 16;
   if (int rc2 = ensure_u8lut()) return rc2;
   if (x_u8 && (uintptr_t)x % 16 == 0)
-    GCC_CUDA(launch_pdl_k(prep_x2_u8_staged_kernel, dim3(batch < 148 * 8 ? batch : 148 * 8), dim3(256), 0, (cudaStream_t)stream,
-                          (const uint8_t*)x, batch, (uint4*)X2, (uint4*)XB));
+    GCC_CUDA(launch_aux(prep_x2_u8_staged_kernel, dim3(batch < 148 * 8 ? batch : 148 * 8), dim3(256), 0, (cudaStream_t)stream,
+                        (const uint8_t*)x, batch, (uint4*)X2, (uint4*)XB));
   else if (x_u8)
-    GCC_CUDA(launch_pdl_k(prep_x2_kernel<uint8_t>, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream, (const uint8_t*)x,
-                          total, (uint4*)X2, (uint4*)XB));
+    GCC_CUDA(launch_aux(prep_x2_kernel<uint8_t>, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream, (const uint8_t*)x,
+                        total, (uint4*)X2, (uint4*)XB));
   else
-    GCC_CUDA(launch_pdl_k(prep_x2_kernel<float>, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream, (const float*)x, total,
-                          (uint4*)X2, (uint4*)nullptr));
+    GCC_CUDA(launch_aux(prep_x2_kernel<float>, dim3((int)ctas), dim3(256), 0, (cudaStream_t)stream, (const float*)x, total,
+                        (uint4*)X2, (uint4*)nullptr));
   GCC_CHECK_LAUNCH("prep_x2");
   return GCCVAE_OK;
 }
@@ -2742,43 +2368,6 @@ extern "C" int gccvae_tap4_ls_bf16(int batch, int HB, int WB, int CB, const void
   return launch_tapgemm(p, groups, 1, (cudaStream_t)stream, "tap4_ls");
 }
 
-// S -> L of a k4/s2/p1 layer (Conv2DTranspose forward / Conv2D dgrad) in BLOCK form:
-//   blocks[n, i, j, (dy,dx), cl] = sum_{a,b in {0,1}} sum_cs S[n, i - a, j - b, cs] * W[2a + dy, 2b + dx, cl, cs]
-// (restated in the test tree, block_forms.py: convT_k4s2_to_blocks) - a 2x2-tap stride-1 gather over S with N = 4 CL output columns, so one
-// 128-row tile produces 4 x 128 output pixels from 4 x (128 x CS) operand bytes, against 16 (phase, tap) operand tiles
-// per 128 pixels in the phase formulation.  The tile's rows are the (WS + 1) blocks of one block row of `bn` images;
-// the epilogue writes each slot to its pixel of L (NHWC, or s2d storage with GCCVAE_OUT_S2D) and drops the slots that
-// fall outside the plane.  Wp = pack kind 10: [(dy,dx,cl)][(a,b,cs)] bf16.
-extern "C" int gccvae_sl_blk_supported(int HS, int WS, int CS, int CL) {
-  return (WS + 1 <= 128 && (CS == 32 || CS == 64 || CS == 128) && (CL == 32 || CL == 64) && HS >= 1) ? 1 : 0;
-}
-extern "C" int gccvae_sl_blk_bf16(int batch, int HS, int WS, int CS, const void* S, const void* Wp, int CL, const float* bias,
-                                  int act, const void* mask, void* L, void* stream) {
-  GCC_REQUIRE(S && Wp && L && batch > 0, "sl_blk: null pointer");
-  GCC_REQUIRE(gccvae_sl_blk_supported(HS, WS, CS, CL), "sl_blk: unsupported shape %dx%dx%d -> CL %d", HS, WS, CS, CL);
-  const int kc = CS >= 64 ? 64 : CS;
-  const int bw = WS + 1, bn = 128 / bw;
-  TapGemmParams p;
-  memset(&p, 0, sizeof(p));
-  int rc;
-  if ((rc = encode_act_map(&p.tmA, S, batch, HS, WS, CS, kc, bw, 1, bn, 1))) return rc;
-  if ((rc = encode_mat_map(&p.tmB, Wp, 4LL * CL, 4LL * CS, kc, 4 * CL))) return rc;
-  p.num_taps = 4; p.chunks = CS / kc; p.a_scale = 1; p.BW = bw; p.BH = 1; p.BN = bn;
-  p.tiles_w = 1; p.tiles_h = HS + 1;
-  for (int t = 0; t < 4; ++t) { p.a_dh[0][t] = (short)(-(t >> 1)); p.a_dw[0][t] = (short)(-(t & 1)); }
-  p.b_tap_stride = CS;
-  p.KC = kc; p.swz = umma_swizzle_for(kc * 2);
-  p.N = 4 * CL; p.n_store = 4 * CL; p.n_slabs = 1;
-  p.rows_valid = bw * bn; p.blk_cl = CL;
-  p.out = L; p.mask = mask; p.bias = bias; p.bias_mod = CL; p.bias_n = CL;
-  p.act = act & ~GCCVAE_LAYOUT_FLAGS; p.out_f32 = 0;
-  p.out_s2d = (act & GCCVAE_OUT_S2D) ? 1 : 0; p.mask_s2d = (act & GCCVAE_MASK_S2D) ? 1 : 0;
-  p.OH = 2 * HS; p.OW = 2 * WS; p.OC = CL; p.oys = p.oxs = 1;
-  p.batch = batch;
-  const int groups = (batch + bn - 1) / bn;
-  return launch_tapgemm(p, groups, 1, (cudaStream_t)stream, "sl_blk");
-}
-
 // dW[(kh,kw,c<3), cs] (fp32, Keras layout) += sum_pix gather4(in2)[pix, (a,b,dy,dx,c4)] * S[pix, cs]
 // in2 = [B,33,33,16] bf16 x2 blocks of a 3-channel 64x64 tensor, S = [B,32,32,CS] bf16.
 // db (optional, blocks written by gccvae_prep_x2_bf16 only - element 15 of every block is 1.0): db[cs] += sum_pix S[pix, cs].
@@ -2787,20 +2376,14 @@ extern "C" int gccvae_tap4_wg_bf16(int batch, const void* in2, const void* S, in
   GCC_REQUIRE(CS % 32 == 0 && CS <= 256, "tap4_wg: CS=%d unsupported (multiple of 32, <= 256)", CS);
   WgParams p;
   memset(&p, 0, sizeof(p));
-  static int env_tma = -1;
-  if (env_tma < 0) { const char* e = getenv("GCCVAE_TAP4_WG_TMA"); env_tma = e ? atoi(e) : 0; }
-  if (!env_tma) {
-    // A tile built by the (otherwise idle) epilogue warps: one 128-byte row per pixel, SWIZZLE_128B, which is an
-    // MN-major operand with M = 64 (a,b,dy,dx,c4); the instruction's rows 64..127 come from the unused second slab
-    // Only ONE 16 KB slab per stage is built and reserved: the second slab the M = 128 instruction reads (LBO = 16 KB
-    // further on: the stage's B tile and the next stage, or the slack behind the last stage) feeds accumulator rows
-    // 64..127, which nobody reads.  24 KB stages instead of 40: four pipeline stages in the same 100 KB per CTA - the
-    // kernel is bound by the round trip of a stage (profiles/r02_timeline_wgrad.txt), so depth is what it needs.
-    p.in2 = (const uint4*)in2;
-    p.kcA = 64; p.blocks_per_tap = 1; p.blocks_per_mtile = 1; p.taps = 1; p.c4_rows = 2;
-  } else {
-    p.kcA = 16; p.blocks_per_tap = 1; p.blocks_per_mtile = 8; p.taps = 4; p.c4_rows = 2;
-  }
+  // A tile built by the (otherwise idle) epilogue warps: one 128-byte row per pixel, SWIZZLE_128B, which is an
+  // MN-major operand with M = 64 (a,b,dy,dx,c4); the instruction's rows 64..127 come from the unused second slab
+  // Only ONE 16 KB slab per stage is built and reserved: the second slab the M = 128 instruction reads (LBO = 16 KB
+  // further on: the stage's B tile and the next stage, or the slack behind the last stage) feeds accumulator rows
+  // 64..127, which nobody reads.  24 KB stages instead of 40: four pipeline stages in the same 100 KB per CTA - the
+  // kernel is bound by the round trip of a stage (profiles/r02_timeline_wgrad.txt), so depth is what it needs.
+  p.in2 = (const uint4*)in2;
+  p.kcA = 64; p.blocks_per_tap = 1; p.blocks_per_mtile = 1; p.taps = 1; p.c4_rows = 2;
   p.kcB = (CS % 64 == 0) ? 64 : 32;
   p.b_loads = CS / p.kcB;
   p.swzA = umma_swizzle_for(p.kcA * 2);
@@ -2809,35 +2392,28 @@ extern "C" int gccvae_tap4_wg_bf16(int batch, const void* in2, const void* S, in
   GCC_REQUIRE(pick_tile(32, 32, &bw, &bh, &bn) == 0, "tap4_wg: tile");
   p.a_scale = 1;
   for (int t = 0; t < 4; ++t) { p.a_dh[t] = (short)(t >> 1); p.a_dw[t] = (short)(t & 1); }
-  if ((rc = encode_act_map(&p.tmA, in2, batch, 33, 33, 16, 16, bw, bh, bn, 1))) return rc;   // unused in x2 mode
+  if ((rc = encode_act_map(&p.tmA, in2, batch, 33, 33, 16, 16, bw, bh, bn, 1))) return rc;   // prefetched, never loaded
   if ((rc = encode_act_map(&p.tmB, S, batch, 32, 32, CS, p.kcB, bw, bh, bn, 1))) return rc;
   p.BW = bw; p.BH = bh; p.BN = bn; p.tiles_w = 32 / bw; p.tiles_h = 32 / bh;
   p.N = CS;
   p.out.n_seg = 1; p.out.m_valid = 64;
   p.out.seg[0].col0 = 0; p.out.seg[0].ncols = CS; p.out.seg[0].ld = CS; p.out.seg[0].dst = dW;
   p.ones_db = db;
-  if (g_colsum != nullptr && g_colsum_mod < 0) {   // armed by gccvae_next_launch_colsum(ptr, n, -1): sums of S
-    p.colsum = g_colsum; p.colsum_n = g_colsum_n; p.colsum_side = -g_colsum_mod;
-    g_colsum = nullptr;
-    GCC_REQUIRE(p.colsum_side == 1 && p.colsum_n > 0 && p.colsum_n <= CS, "tap4_wg: fused bias gradient: S side only");
-    // in x2 mode the epilogue warps build the A tile; the column-sum path of wgrad_kernel assumes they are idle
-    GCC_REQUIRE(env_tma, "tap4_wg: the fused bias gradient is not supported with the thread-built A tile");
-  }
   const int groups = (batch + bn - 1) / bn;
   p.tiles_total = groups * p.tiles_w * p.tiles_h;
-  int splits = 148 * wg_per_sm();
+  int splits = 148 * WG_PER_SM;
   if (splits > p.tiles_total) splits = p.tiles_total;
   p.tiles_per_cta = (p.tiles_total + splits - 1) / splits;
   splits = (p.tiles_total + p.tiles_per_cta - 1) / p.tiles_per_cta;
   const int stage_bytes = 128 * 128 * p.blocks_per_mtile + 128 * CS * 2;
-  int stages = (wg_smem_kb() * 1024) / stage_bytes;   // default 100 KB: two CTAs per SM
+  int stages = (WG_SMEM_KB * 1024) / stage_bytes;   // two CTAs per SM
   if (stages > 8) stages = 8;
   if (stages > p.tiles_per_cta) stages = p.tiles_per_cta;
   if (stages < 1) stages = 1;
   p.stages = stages;
   size_t smem = (size_t)stages * stage_bytes + 1024 + 256 + 1024;
   // the unread second slab of the LAST stage's A tile must still lie inside the allocation (layout: [A stages][B stages])
-  if (!env_tma && smem < (size_t)(stages + 1) * 16384 + 1024) smem = (size_t)(stages + 1) * 16384 + 1024;
+  if (smem < (size_t)(stages + 1) * 16384 + 1024) smem = (size_t)(stages + 1) * 16384 + 1024;
   static bool attr_set = false;
   if (!attr_set) {
     GCC_CUDA(cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
@@ -2975,20 +2551,8 @@ extern "C" int gccvae_c3conv_bf16(int batch, const void* in2, const void* Wp, in
   GCC_REQUIRE(!(act & GCCVAE_MASK_S2D), "c3conv: s2d mask is not supported");
   p.total_tiles = batch * 8;
   p.timeline = g_timeline;
-  if (g_colsum != nullptr && g_colsum_mod >= 0) {   // armed by gccvae_next_launch_colsum
-    GCC_REQUIRE(g_colsum_n == CS, "c3conv: fused bias gradient needs n == CS");
-    p.colsum = g_colsum;
-    g_colsum = nullptr;
-  }
-  { const char* e = getenv("GCCVAE_C3_DBG"); p.dbg = e ? atoi(e) : 0; }
-  static int env_per_sm = -1;
-  if (env_per_sm < 0) {
-    const char* e = getenv("GCCVAE_C3_PER_SM");
-    env_per_sm = e ? atoi(e) : 0;
-  }
-  int per_sm = env_per_sm > 0 ? env_per_sm : 2;
-  if (per_sm > 2) per_sm = 2;   // __launch_bounds__(288, 2): no register spills in the epilogue
-  if (per_sm > 512 / (4 * (CS <= 32 ? 32 : 64))) per_sm = 512 / (4 * (CS <= 32 ? 32 : 64));   // TMEM: 4 accumulator stages
+  // __launch_bounds__(288, 2): no register spills in the epilogue.  TMEM: 2 CTAs x 4 accumulator stages x <= 64 columns
+  constexpr int per_sm = 2;
   int stages = (200 * 1024 / per_sm - 8192 - 3072) / (128 * 128);
   if (stages > 6) stages = 6;
   GCC_REQUIRE(stages >= 2, "c3conv: shared memory");
@@ -3037,21 +2601,16 @@ extern "C" int gccvae_wg_s2d_bf16(int batch, int HS, int WS, int CL, const void*
   p.N = CS;
   p.out.n_seg = 1; p.out.m_valid = 16 * CL;
   p.out.seg[0].col0 = 0; p.out.seg[0].ncols = CS; p.out.seg[0].ld = CS; p.out.seg[0].dst = dW;
-  if (g_colsum != nullptr && g_colsum_mod < 0) {
-    p.colsum = g_colsum; p.colsum_n = g_colsum_n; p.colsum_side = -g_colsum_mod;
-    g_colsum = nullptr;
-    GCC_REQUIRE(p.colsum_side == 1 && p.colsum_n > 0 && p.colsum_n <= CS, "wg_s2d: fused bias gradient: S side only");
-  }
   const int groups = (batch + bn - 1) / bn;
   p.tiles_total = groups * p.tiles_w * p.tiles_h;
   const int mtiles = (16 * CL) / 128;
-  int splits = (148 * wg_per_sm() + mtiles - 1) / mtiles;
+  int splits = (148 * WG_PER_SM + mtiles - 1) / mtiles;
   if (splits > p.tiles_total) splits = p.tiles_total;
   if (splits < 1) splits = 1;
   p.tiles_per_cta = (p.tiles_total + splits - 1) / splits;
   splits = (p.tiles_total + p.tiles_per_cta - 1) / p.tiles_per_cta;
   const int stage_bytes = 128 * 128 * 2 + 128 * CS * 2;
-  int stages = (wg_smem_kb() * 1024) / stage_bytes;   // default 100 KB: two CTAs per SM
+  int stages = (WG_SMEM_KB * 1024) / stage_bytes;   // two CTAs per SM
   if (stages > 4) stages = 4;
   if (stages > p.tiles_per_cta) stages = p.tiles_per_cta;
   if (stages < 1) stages = 1;
@@ -3111,10 +2670,10 @@ extern "C" int gccvae_pack_jobs_bf16(const gccvae_pack_job* jobs, int n_jobs, vo
   PackJobs pj;
   memset(&pj, 0, sizeof(pj));
   for (int i = 0; i < n_jobs; ++i) {
-    GCC_REQUIRE(jobs[i].W && jobs[i].out && jobs[i].kind >= 0 && jobs[i].kind <= 10, "pack_jobs: bad job %d", i);
+    GCC_REQUIRE(jobs[i].W && jobs[i].out && jobs[i].kind >= 0 && jobs[i].kind <= 9, "pack_jobs: bad job %d", i);
     pj.j[i] = jobs[i];
   }
-  GCC_CUDA(launch_pdl_k(pack_jobs_kernel, dim3(64, n_jobs, 1), dim3(256), 0, (cudaStream_t)stream, pj));
+  GCC_CUDA(launch_aux(pack_jobs_kernel, dim3(64, n_jobs, 1), dim3(256), 0, (cudaStream_t)stream, pj));
   GCC_CHECK_LAUNCH("pack_jobs");
   return GCCVAE_OK;
 }

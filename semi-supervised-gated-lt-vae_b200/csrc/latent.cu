@@ -963,8 +963,8 @@ extern "C" int gccvae_gate_fwd(const float* mu, const float* c_in, const float* 
   GCC_REQUIRE((mu || c_in) && Wcls && bcls && Wlt && Wlf && Wst && Wsf && gate_ws, "gate_fwd: null pointer");
   GCC_REQUIRE((U1 == nullptr) == (U2 == nullptr), "gate_fwd: U1 and U2 must both be given or both be NULL");
   GCC_REQUIRE(temperature > 0.0f || temperature_dev, "gate_fwd: temperature must be > 0");
-  GCC_CUDA(launch_pdl_k(gate_fwd_kernel, dim3(1), dim3(352), 0, (cudaStream_t)stream, mu, c_in, U1, U2, seed, offset,
-                        step_dev, temperature, temperature_dev, Wcls, bcls, Wlt, Wlf, Wst, Wsf, gate_ws, c_out));
+  GCC_CUDA(launch_aux(gate_fwd_kernel, dim3(1), dim3(352), 0, (cudaStream_t)stream, mu, c_in, U1, U2, seed, offset,
+                      step_dev, temperature, temperature_dev, Wcls, bcls, Wlt, Wlf, Wst, Wsf, gate_ws, c_out));
   GCC_CHECK_LAUNCH("gate_fwd");
   return GCCVAE_OK;
 }
@@ -987,9 +987,9 @@ extern "C" int gccvae_latent_fwd(const gccvae_latent_fwd_args* a, void* stream) 
   GCC_REQUIRE((uintptr_t)a->eps_k % 8 == 0, "latent_fwd: eps_k must be 8-byte aligned");
   const int grid = latent_grid(a->batch);
   if (a->supervised)
-    GCC_CUDA(launch_pdl_k(latent_fwd_kernel<true>, dim3(grid), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+    GCC_CUDA(launch_aux(latent_fwd_kernel<true>, dim3(grid), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   else
-    GCC_CUDA(launch_pdl_k(latent_fwd_kernel<false>, dim3(grid), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+    GCC_CUDA(launch_aux(latent_fwd_kernel<false>, dim3(grid), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   GCC_CHECK_LAUNCH("latent_fwd");
   return GCCVAE_OK;
 }
@@ -1007,7 +1007,7 @@ extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) 
                   (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y_tgt % 8 == 0 && (uintptr_t)a->y_src % 8 == 0 &&
                   (uintptr_t)a->y_src_out % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
               "gen_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
-  GCC_CUDA(launch_pdl_k(gen_latent_kernel, dim3(latent_grid(a->batch)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+  GCC_CUDA(launch_aux(gen_latent_kernel, dim3(latent_grid(a->batch)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   GCC_CHECK_LAUNCH("gen_latent");
   return GCCVAE_OK;
 }
@@ -1024,7 +1024,7 @@ extern "C" int gccvae_iw_latent(const gccvae_iw_latent_args* a, void* stream) {
                   (uintptr_t)a->lw_part % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
               "iw_latent: misaligned pointer (fp32: 4 bytes, int64: 8, z16: 16)");
   const int rows = a->batch * a->kc;
-  GCC_CUDA(launch_pdl_k(iw_latent_kernel, dim3(latent_grid(rows)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+  GCC_CUDA(launch_aux(iw_latent_kernel, dim3(latent_grid(rows)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
   GCC_CHECK_LAUNCH("iw_latent");
   return GCCVAE_OK;
 }
@@ -1035,8 +1035,8 @@ extern "C" int gccvae_iw_accumulate(int batch, int kc, int k0, int K, const floa
   GCC_REQUIRE(batch > 0 && kc >= 1 && k0 >= 0 && k0 + kc <= K, "iw_accumulate: bad sizes B=%d K=%d k0=%d kc=%d", batch,
               K, k0, kc);
   GCC_REQUIRE(lw_part && log_pxz && state && (!finalize || (est && ess)), "iw_accumulate: null pointer");
-  GCC_CUDA(launch_pdl_k(iw_accumulate_kernel, dim3((batch + 7) / 8), dim3(256), 0, (cudaStream_t)stream, batch, kc, k0,
-                        K, lw_part, log_pxz, state, log_w, first, finalize, est, ess));
+  GCC_CUDA(launch_aux(iw_accumulate_kernel, dim3((batch + 7) / 8), dim3(256), 0, (cudaStream_t)stream, batch, kc, k0,
+                      K, lw_part, log_pxz, state, log_w, first, finalize, est, ess));
   GCC_CHECK_LAUNCH("iw_accumulate");
   return GCCVAE_OK;
 }
@@ -1060,13 +1060,13 @@ extern "C" int gccvae_latent_bwd(const gccvae_latent_bwd_args* a, void* stream) 
       GCC_CUDA(cudaFuncSetAttribute(latent_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr_done[1] = true;
     }
-    GCC_CUDA(launch_pdl_k(latent_bwd_kernel<true>, dim3(grid), dim3(WARPS * 32), smem, (cudaStream_t)stream, *a));
+    GCC_CUDA(launch_aux(latent_bwd_kernel<true>, dim3(grid), dim3(WARPS * 32), smem, (cudaStream_t)stream, *a));
   } else {
     if (!attr_done[0]) {
       GCC_CUDA(cudaFuncSetAttribute(latent_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr_done[0] = true;
     }
-    GCC_CUDA(launch_pdl_k(latent_bwd_kernel<false>, dim3(grid), dim3(WARPS * 32), smem, (cudaStream_t)stream, *a));
+    GCC_CUDA(launch_aux(latent_bwd_kernel<false>, dim3(grid), dim3(WARPS * 32), smem, (cudaStream_t)stream, *a));
   }
   GCC_CHECK_LAUNCH("latent_bwd");
   return GCCVAE_OK;
@@ -1084,9 +1084,9 @@ extern "C" int gccvae_gate_bwd(float* partials, int n_partials, const float* mu,
   // block ticket of the merged kernel: a spare slot of the gate workspace (zeroed by every gate_fwd launch and by the
   // kernel itself) - the workspace is caller-owned device memory, const only from the caller's point of view
   unsigned int* ticket = reinterpret_cast<unsigned int*>(const_cast<float*>(gate_ws)) + GW_B + 31;
-  GCC_CUDA(launch_pdl_k(reduce_gate_bwd_kernel, dim3((PT_TOTAL + 351) / 352), dim3(352), 0, (cudaStream_t)stream,
-                        (const float*)partials, n_partials, reduced, ticket, mu, Wcls, Wlt, Wlf, Wst, Wsf, gate_ws,
-                        gating_reg, l1_scale, dWcls, dbcls, dWlt, dWlf, dWst, dWsf, dmu, loss_inout));
+  GCC_CUDA(launch_aux(reduce_gate_bwd_kernel, dim3((PT_TOTAL + 351) / 352), dim3(352), 0, (cudaStream_t)stream,
+                      (const float*)partials, n_partials, reduced, ticket, mu, Wcls, Wlt, Wlf, Wst, Wsf, gate_ws,
+                      gating_reg, l1_scale, dWcls, dbcls, dWlt, dWlf, dWst, dWsf, dmu, loss_inout));
   GCC_CHECK_LAUNCH("gate_bwd");
   return GCCVAE_OK;
 }

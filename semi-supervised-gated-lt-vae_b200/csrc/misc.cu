@@ -18,14 +18,6 @@ void set_error(const char* fmt, ...) {
   va_end(ap);
 }
 void count_launch(int n) { g_launches += n; }
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GCCVAE_PDL_AUX");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
 
 // ---------------------------------------------------------------------------------------------
 // utils.py:101-105: log p(x|z) = sum_{h,w,c} Laplace(xhat,1).log_prob(x) = -|x-xhat|_1 - n ln2.
@@ -265,11 +257,11 @@ extern "C" int gccvae_adam_f32(float* param, const float* grad, float* m, float*
   long long blocks = (n + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
   if (step_dev) {
-    GCC_CUDA(launch_pdl_k(bump_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, step_dev));
+    GCC_CUDA(launch_aux(bump_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, step_dev));
     GCC_CHECK_LAUNCH("adam_bump");
   }
-  GCC_CUDA(launch_pdl_k(adam_kernel, dim3((int)blocks), dim3(256), 0, (cudaStream_t)stream, param, grad, m, v, n, lr,
-                        beta1, beta2, eps, step, (const int*)step_dev));
+  GCC_CUDA(launch_aux(adam_kernel, dim3((int)blocks), dim3(256), 0, (cudaStream_t)stream, param, grad, m, v, n, lr,
+                      beta1, beta2, eps, step, (const int*)step_dev));
   GCC_CHECK_LAUNCH("adam");
   return GCCVAE_OK;
 }
@@ -282,9 +274,9 @@ extern "C" int gccvae_adam_fused_f32(float* param, float* grad, float* m, float*
   GCC_REQUIRE(result_ring == nullptr || (result_loss && result_c && ring_slots > 0), "adam_fused: bad result ring");
   long long blocks = (n_zero - i0 + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  GCC_CUDA(launch_pdl_k(adam_fused_kernel, dim3((int)blocks), dim3(256), 0, (cudaStream_t)stream, param, grad, m, v, i0,
-                        n, n_zero, lr, beta1, beta2, eps, step_state, publish, result_loss, result_c, result_ring,
-                        ring_slots));
+  GCC_CUDA(launch_aux(adam_fused_kernel, dim3((int)blocks), dim3(256), 0, (cudaStream_t)stream, param, grad, m, v, i0,
+                      n, n_zero, lr, beta1, beta2, eps, step_state, publish, result_loss, result_c, result_ring,
+                      ring_slots));
   GCC_CHECK_LAUNCH("adam_fused");
   return GCCVAE_OK;
 }

@@ -42,8 +42,8 @@ S2D_TENSORS = ["enc.conv1.out", "enc.conv2.out", "enc.conv3.out", "dec.conv4t.do
 class EngineTC(Engine):
     precision = "bf16"
 
-    def __init__(self, store, fused_chain=True, wgrad_streams=2, post_chain_stream="side", markers=0, tail_split=False,
-                 sl_block_form=False, wgrad_plan="201202", dec_wgrad_plan="00000", tap_halo=True):
+    def __init__(self, store, fused_chain=True, wgrad_streams=2, post_chain_stream="side", markers=0,
+                 wgrad_plan="201202", dec_wgrad_plan="00000"):
         super().__init__(store)
         # scheduling of the weight-gradient kernels (they feed only the optimiser): the encoder's alternate between
         # `wgrad_streams` side streams so that a layer's weight gradient starts when its operand is ready instead of
@@ -51,11 +51,6 @@ class EngineTC(Engine):
         # weight gradients, gate backward) go to `post_chain_stream` ("side" = the weight-gradient stream, "side2" =
         # the bias-gradient stream).  Same-box A/B, ms per sup+unsup pair (profiles/r02_ab_log.txt): 1 stream / side
         # 1.344, 2 streams / side 1.336, 2 streams / side2 1.351, 1 stream / side2 1.375
-        # the step ends with conv2's dgrad -> conv1's weight / bias gradient, a strict chain of two HBM-bound kernels.
-        # `tail_split`: both run on the two halves of the batch, so the second half's dgrad overlaps the first half's
-        # weight gradient (tensors are contiguous per image: a half is a pointer offset).  Measured +2 % per step on
-        # B200 (the half-batch launches are less efficient than the overlap gains): off by default.
-        self.tail_split = bool(tail_split)
         # which weight-gradient lane (0, 1, 2 = three side streams) takes: the post-chain launches, conv5, conv4, conv3,
         # conv2, conv1 of the encoder backward (decoder weight gradients: lane 0).  After the fused chain kernel the encoder's
         # backward is bound by the weight-gradient streams: with everything on two lanes ("001010") the three small
@@ -63,8 +58,9 @@ class EngineTC(Engine):
         # gradient and the chain conv5 -> conv3 -> conv1 ended 70 us after the last dgrad; on their own lane the step is
         # 3 % shorter (profiles/r02_ab_log.txt: 1.304 -> 1.263 ms per pair; "101010" 1.279, "201201" / "201002" 1.264)
         # L -> S layers over s2d blocks (conv2-4 forward, convT dgrads): two column-shifted boxes with one halo row instead
-        # of four shifted boxes where the geometry allows it (16x16 outputs: conv2 forward, conv4t dgrad)
-        self.tap_flag = TAP_HALO if tap_halo else 0
+        # of four shifted boxes where the geometry allows it (16x16 outputs: conv2 forward, conv4t dgrad).  Same-box A/B,
+        # ms per sup+unsup pair (profiles/r02_ab_log.txt): 1.2569 / 1.2503 against 1.2756 / 1.2752 with four boxes
+        self.tap_flag = TAP_HALO
         self.wgrad_plan = [int(c) for c in str(wgrad_plan).zfill(6)]
         self.dec_wgrad_plan = [int(c) for c in str(dec_wgrad_plan).zfill(5)]     # lanes of conv5t, conv4t, conv3t, conv2t, conv1t
         self.wg_lanes = [None, torch.cuda.Stream(device=store.device), torch.cuda.Stream(device=store.device)]
@@ -100,17 +96,6 @@ class EngineTC(Engine):
         for name in S2D_LAYERS:
             _, _, (HL, WL, CL), (HS, WS, CS), k, s_, p_, _ = (_ENC.get(name) or _DEC[name])
             self.wp[name + ".s2d"] = z16(((CS + 15) // 16 * 16) * 16 * CL)
-        # S -> L direction of the six k4/s2/p1 layers (convT forward, conv dgrad) in block form: rows = output blocks of
-        # 2x2 pixels, N = 4 C_L, 4 taps over S (gccvae_sl_blk_bf16).  Parity-tested, but its 128 / 256-column epilogue on 4
-        # warps is slower than the halo kernel's 8 epilogue warps (conv2 dgrad 65 vs 49 us, conv4t forward 43 vs 39 us in
-        # the eager per-op profile; +7 % per step): off by default, the halo / 4-phase kernels stay the product path.
-        self.blk = {}
-        if sl_block_form:
-            for name in S2D_LAYERS:
-                _, _, (HL, WL, CL), (HS, WS, CS), k, s_, p_, _ = (_ENC.get(name) or _DEC[name])
-                if lib.gccvae_sl_blk_supported(HS, WS, CS, CL):
-                    self.blk[name] = (HS, WS, CS, CL)
-                    self.wp[name + ".blk"] = z16(4 * CL * 4 * CS)
         # 45-wide dense layers, zero-padded to tensor-core widths (pad regions stay zero forever)
         self.wp["heads.ls"] = z16(96, 256)       # rows 0..44 = W_loc^T, 48..92 = W_std^T
         self.wp["heads.sl"] = z16(256, 96)
@@ -157,16 +142,11 @@ class EngineTC(Engine):
                 _, _, (HL, WL, CL), (HS, WS, CS), k, s_, p_, _ = lay
                 if name not in S2D_LAYERS:     # the s2d layers use the kind-9 operand instead
                     J(0, k * k, CL, CS, v(name + ".w"), self.wp[name + ".ls"])
-                if name not in self.blk:       # (the block-form layers use the kind-10 operand instead)
-                    J(2 if (HS == 1 and WS == 1) else 1, k * k, CL, CS, v(name + ".w"), self.wp[name + ".sl"])
+                J(2 if (HS == 1 and WS == 1) else 1, k * k, CL, CS, v(name + ".w"), self.wp[name + ".sl"])
             J(1, 16, 3, 32, v("dec.conv5t.w"), self.wp["dec.conv5t.sl"])
             for name in self.halo:
-                if name in self.blk:
-                    continue
                 _, _, (HL, WL, CL), (HS, WS, CS), k, s_, p_, _ = (_ENC.get(name) or _DEC[name])
                 J(6, 16, CL, CS, v(name + ".w"), self.wp[name + ".sl9"])
-            for name, (HS, WS, CS, CL) in self.blk.items():
-                J(10, 16, CL, CS, v(name + ".w"), self.wp[name + ".blk"])
             for name in S2D_LAYERS:
                 _, _, (HL, WL, CL), (HS, WS, CS), k, s_, p_, _ = (_ENC.get(name) or _DEC[name])
                 J(9, 16, CL, CS, v(name + ".w"), self.wp[name + ".s2d"])
@@ -285,12 +265,7 @@ class EngineTC(Engine):
         st = _stream()
         if mask_s2d:
             act = act | MASK_S2D
-        if name in self.blk and out_f32 == 0:
-            HS, WS, CS, CL = self.blk[name]
-            W = self.wp[name + ".blk"]
-            self._run(what, (S, mask, L), lambda: self.lib.gccvae_sl_blk_bf16(
-                geom.batch, HS, WS, CS, ptr(S), ptr(W), CL, ptr(bias), act, ptr(mask), ptr(L), st))
-        elif name in self.halo:
+        if name in self.halo:
             W = self.wp[name + ".sl9"]
             self._run(what, (S, mask, L), lambda: self.lib.gccvae_sl_halo_bf16(
                 C.byref(geom), ptr(S), ptr(W), ptr(bias), act, ptr(mask), ptr(L), out_f32, st))
@@ -346,10 +321,9 @@ class EngineTC(Engine):
         self._lanes_used.add(k)      # (only lanes that carry work of THIS step may be waited for inside a capture)
         return self.wg_lanes[k]
 
-    def _side(self, fn, small=False, lane=0):
-        """run fn (weight-gradient launches) on a side stream, after everything issued so far on the main one.
-        (`small=True` keeps a launch on the main stream; measured slower for every candidate, so it is unused.)"""
-        if self.side is None or small:
+    def _side(self, fn, lane=0):
+        """run fn (weight-gradient launches) on a side stream, after everything issued so far on the main one."""
+        if self.side is None:
             fn()
             self._flush_deferred_bias()
             return
@@ -609,9 +583,7 @@ class EngineTC(Engine):
             if hook is not None and self.side is not None:
                 ev = torch.cuda.Event()
                 ev.record(torch.cuda.current_stream())     # everything the main stream has produced so far
-            split = self.tail_split and name == "enc.conv2" and B % 2 == 0 and B >= 128 and self.side is not None
-            if not split:
-                self._sl(name, geom, dout, None, ACT_NONE, xin, dxin, 0, name + " dgrad", mask_s2d=s2d_l)
+            self._sl(name, geom, dout, None, ACT_NONE, xin, dxin, 0, name + " dgrad", mask_s2d=s2d_l)
             if hook is not None:
                 self.tail_hook = None
                 if ev is not None:     # under this dgrad: after all earlier weight / bias gradients, not after it
@@ -628,22 +600,6 @@ class EngineTC(Engine):
                 else:
                     hook()
         dh1 = b["enc.conv1.dout"]
-        if split:
-            # last layer pair in two halves of the batch: dgrad(h0), then dgrad(h1) on the main stream while conv1's
-            # weight / bias gradient of h0 runs on the side streams, then those of h1
-            h = B // 2
-            geom_h = make_geom(_ENC["enc.conv2"], h)
-            dout2, mask2, X2 = b["enc.conv2.dout"], b["enc.conv1.out"], b["X2"]
-            for i in (0, 1):
-                sl = slice(i * h, (i + 1) * h)
-                self._sl("enc.conv2", geom_h, dout2[sl], None, ACT_NONE, mask2[sl], dh1[sl], 0, "enc.conv2 dgrad", mask_s2d=True)
-                def wg1(sl=sl, i=i):     # (the image blocks of half i: the first B x 1089 x 16 elements of the X2 buffer)
-                    self._run("enc.conv1 wgrad", (dh1[sl],), lambda: lib.gccvae_tap4_wg_bf16(
-                        h, ptr(X2) + i * h * 1089 * 32, ptr(dh1[sl]), 32, ptr(g_("enc.conv1.w")), ptr(g_("enc.conv1.b")),
-                        _stream()))
-                self._side(wg1, lane=self.wgrad_plan[5])
-            self.join_side()
-            return
         def wg1():     # conv1's bias gradient comes out of the same launch (the ones slot of prep_x2's blocks)
             self._run("enc.conv1 wgrad", (b["X2"][:B * 1089 * 16], dh1), lambda: lib.gccvae_tap4_wg_bf16(
                 B, ptr(b["X2"]), ptr(dh1), 32, ptr(g_("enc.conv1.w")), ptr(g_("enc.conv1.b")), _stream()))
