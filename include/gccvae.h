@@ -314,6 +314,48 @@ typedef struct {
 } gccvae_gen_latent_args;
 int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
 
+/* ---- latent code of a label walk (no counterpart in the reference) ---------------------------------------------
+ * Frames of B images along n_labels labels at n_alpha values each: row r = (b * n_labels + l) * n_alpha + t walks
+ * label labels[l] to the real value alphas[t] and keeps the other 17 labels.  Notation as gccvae_gen_latent; the
+ * conditional prior at a walked label is the prior of networks.py:118-127 with y_l replaced by alpha.  Its term of
+ * label l is exactly the boolean term at alpha = 0 and alpha = 1 and fmaf(alpha, P_true - P_false, P_false) otherwise,
+ * summed in the order of the prior (j = 0..17), so frames at alpha in {0, 1} are bit-identical to gccvae_gen_latent
+ * with that label set.  Any finite alpha is valid (beyond [0, 1] the prior extrapolates).
+ *   GCCVAE_WALK_LABELS:  z_s = eps_s, z_c = loc_p(y(alpha),c) + scale_p(y(alpha),c) eps_c (GCCVAE_GEN_GENERATE);
+ *                        sample = 0: z_s = 0, z_c = loc_p(y(alpha),c).
+ *   GCCVAE_WALK_IMAGES:  z = the posterior mean (sample = 1: loc + scale eps), then the classify dims move from y_src to
+ *                        y_src with label l at alpha by the counterfactual of GCCVAE_GEN_INTERVENE; y_src = y, or
+ *                        (y = NULL) the classifier's decision on z_c.  The frame at alpha = y_src,l is the posterior z
+ *                        bit for bit; z_s is never touched.
+ * Noise is drawn once per image: eps (image b, dim d) as gccvae_gen_latent, shared by every frame of the image.  The
+ * rows row0 .. row0 + rows - 1 are written at z / z16 rows 0 .. rows - 1 (one chunk of the decoder); y_src_out rows
+ * are written by the chunk that holds the image's first row. */
+#define GCCVAE_WALK_LABELS 1
+#define GCCVAE_WALK_IMAGES 2
+typedef struct {
+  int batch;               /* B images */
+  int mode;                /* GCCVAE_WALK_* */
+  int sample;              /* 0: means, 1: draw with eps (see above) */
+  int n_labels;            /* labels walked, 1..18 */
+  int labels[18];          /* labels[0 .. n_labels-1]: distinct label indices in [0, 18), in row order */
+  int n_alpha;             /* values per label, >= 1 */
+  const float* alphas;     /* [n_alpha] device fp32, finite */
+  int row0, rows;          /* this chunk: rows row0 .. row0 + rows - 1 of the B * n_labels * n_alpha */
+  int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
+  const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu (IMAGES) */
+  const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip (IMAGES) */
+  const long long* y;      /* [B,18] int64 labels, nonzero = 1: the labels (LABELS), y_src or NULL (IMAGES) */
+  const float* eps;        /* [B,45] N(0,1) or NULL -> Philox */
+  uint64_t seed, offset;   /* Philox key / counter base */
+  const int* step_dev;     /* optional device int added to `offset` */
+  const float* gate_ws;    /* from gccvae_gate_fwd */
+  /* outputs (at least one of z, z16) */
+  float* z;                /* optional [rows,45] fp32 (operand of the fp32 decoder) */
+  void* z16;               /* optional bf16 [rows,64], columns 45..63 zero (operand of the tensor-core fc1) */
+  int* y_src_out;          /* optional [B,18] int32: the y_src used (IMAGES) */
+} gccvae_walk_latent_args;
+int gccvae_walk_latent(const gccvae_walk_latent_args* a, void* stream);
+
 /* ---- importance-weighted log-likelihood (no counterpart in the reference) -------------------------------------
  * log p(x [, y]) >= log p_hat = logsumexp_k log w_k - ln K over K samples per image, with proposal q(z|x) (labelled) or
  * q(z|x) q(y|z_c) (unlabelled) and the gate sample c of gate_ws:

@@ -176,11 +176,22 @@ class Engine:
             h = b[lay[0] + ".out"]
         return h
 
-    def image_fwd(self, z, b, batch, out_u8):
+    def image_fwd(self, z, b, batch, out_u8, out=None):
         """generation path: the decoder from the latent code z [B,45] -> a fresh [B,64,64,3] image, the fp32 sigmoid
-        values or (out_u8) uint8 min(255, rint(255 xhat)) with the product and the rounding in fp32."""
-        xhat = self.decoder_fwd(z, b)
-        return image_u8(xhat) if out_u8 else xhat.clone()
+        values or (out_u8) uint8 min(255, rint(255 xhat)) with the product and the rounding in fp32.  `out`: a contiguous
+        [batch,64,64,3] tensor of that dtype (e.g. a row slice of a larger image tensor) to write instead; z and the
+        buffer set b (`bufs` or `dec_bufs`) may then hold more rows than `batch`, and only the first `batch` are decoded."""
+        if out is None:
+            xhat = self.decoder_fwd(z, b)
+            return image_u8(xhat) if out_u8 else xhat.clone()
+        h = z[:batch]
+        for lay in DEC_LAYERS:
+            dst = out if lay is DEC_LAYERS[-1] and not out_u8 else b[lay[0] + ".out"]
+            self.layer_fwd(lay, batch, h, dst)
+            h = dst
+        if out_u8:
+            out.copy_(image_u8(h[:batch]))
+        return out
 
     def iw_decoder_ll(self, x, b, batch, kc, dec, log_pxz):
         """importance-weighted likelihood: log_pxz[r] = log p(x_(r / kc) | z_r) for the batch * kc rows of dec["z"]

@@ -476,11 +476,14 @@ class EngineTC(Engine):
         self._log_pxz_ready = False
         return xhat
 
-    def image_fwd(self, z, b, batch, out_u8):
+    def image_fwd(self, z, b, batch, out_u8, out=None):
         """generation path: the decoder from the z16 operand the latent kernel wrote, conv5t + sigmoid straight into a
-        fresh [B,64,64,3] image (gccvae_convt_image_bf16): fp32, or uint8 min(255, rint(255 xhat))."""
+        fresh [B,64,64,3] image (gccvae_convt_image_bf16): fp32, or uint8 min(255, rint(255 xhat)).  `out`: a contiguous
+        [batch,64,64,3] tensor of that dtype to write instead (a row slice of a larger image tensor: rows are 12 or 48 KB,
+        so every slice keeps the kernel's 16-byte alignment); b (`bufs` or `dec_bufs`) may hold more rows than `batch`."""
         self.decoder_fwd(None, b, z16_ready=True, fused_recon=True, batch=batch, head=True)
-        out = torch.empty(batch, 64, 64, 3, dtype=torch.uint8 if out_u8 else torch.float32, device=self.device)
+        if out is None:
+            out = torch.empty(batch, 64, 64, 3, dtype=torch.uint8 if out_u8 else torch.float32, device=self.device)
         g4 = b["dec.conv4t.out"]
         self._run("dec.conv5t fwd image", (g4, out), lambda: self.lib.gccvae_convt_image_bf16(
             batch, ptr(g4), ptr(self.wp["dec.conv5t.x2t"]), ptr(self.store.view("dec.conv5t.b")), ptr(out), int(out_u8),

@@ -38,7 +38,7 @@ import torch
 
 from . import _lib, dp
 from ._lib import (GATE_WS_FLOATS, LATENT_PARTIAL_FLOATS, RESULT_SLOT_FLOATS, ChainBwdArgs, ChainFwdArgs, DpArgs,
-                   GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
+                   GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, WalkLatentArgs, ptr)
 from .engine import Engine, _stream
 from .networks import Classifier, Conditional_Prior, Decoder, Encoder, _default_device, as_device_f32
 from .params import ParamStore, keras_default_init
@@ -777,29 +777,41 @@ class Learner:
                                                                 tuple(t.shape)))
         return (t.to(self.device, non_blocking=True) != 0).to(torch.int64).contiguous()
 
-    def _generation(self, mode, x, y_tgt, y_src, sample, c, noise, dtype):
+    @staticmethod
+    def _check_dtype(dtype):
         if dtype not in (torch.float32, torch.uint8):
             raise ValueError("dtype must be torch.float32 or torch.uint8, got {}".format(dtype))
-        if x is not None:
-            x, _ = self._prep_inputs(x, None)
-            B = x.shape[0]
-            if B == 0:
-                raise ValueError("x holds no image")
-        else:
-            B = None
-        if y_tgt is not None:
-            y_tgt = self._gen_labels(y_tgt, B, "y" if x is None else "y_new")
-            B = y_tgt.shape[0]
-        if y_src is not None:
-            y_src = self._gen_labels(y_src, B, "y")
-        n = self._noise(noise, B, False, 0)
-        for k, shape in (("eps", (B, self.z_dim)), ("U1", (18, 18)), ("U2", (18, 18))):
+
+    def _gen_images(self, x):
+        """images of the forward-only calls -> (device tensor, B)."""
+        x, _ = self._prep_inputs(x, None)
+        if x.shape[0] == 0:
+            raise ValueError("x holds no image")
+        return x, x.shape[0]
+
+    def _gen_noise_c(self, noise, c, shapes):
+        """explicit draws and gate of the forward-only calls, checked: shapes = {noise key: required shape}."""
+        n = self._noise(noise, None, False, 0)
+        for k, shape in list(shapes.items()) + [("U1", (18, 18)), ("U2", (18, 18))]:
             if n[k] is not None and tuple(n[k].shape) != shape:
                 raise ValueError("noise[{!r}] must be {}, got {}".format(k, list(shape), tuple(n[k].shape)))
         if c is not None:
             c = as_device_f32(c, self.device)
             if tuple(c.shape) != (18, 18):
                 raise ValueError("c must be [18,18], got {}".format(tuple(c.shape)))
+        return n, c
+
+    def _generation(self, mode, x, y_tgt, y_src, sample, c, noise, dtype):
+        self._check_dtype(dtype)
+        B = None
+        if x is not None:
+            x, B = self._gen_images(x)
+        if y_tgt is not None:
+            y_tgt = self._gen_labels(y_tgt, B, "y" if x is None else "y_new")
+            B = y_tgt.shape[0]
+        if y_src is not None:
+            y_src = self._gen_labels(y_src, B, "y")
+        n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
         b = self.engine.bufs(B)
         z = torch.empty(B, self.z_dim, dtype=torch.float32, device=self.device)
         y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if mode == _lib.GEN_INTERVENE else None
@@ -820,6 +832,128 @@ class Learner:
             img = self.engine.image_fwd(z, b, B, dtype == torch.uint8)
         self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
         return img
+
+    def walk(self, x=None, y=None, labels=None, alphas=None, sample=False, c=None, noise=None, dtype=torch.float32,
+             max_rows=8192):
+        """Frames along single labels: for every image, every label l of `labels` and every value a of `alphas`, the
+        image decoded with y_l replaced by the real number a and the other labels kept.  The conditional prior is affine
+        in y before its softplus (networks.py:118-127), so it is defined at any finite a: a = 0 and a = 1 are the prior's
+        own boolean terms, bit for bit, values beyond [0, 1] extrapolate.
+          From images (x [B,64,64,3] given), the counterpart of `intervene`: z as in `reconstruct`, then the classify dims
+            move from the labels y (default: the classifier's decision on z_c) to y with y_l = a, by the counterfactual of
+            `intervene`.  The frame at a = y_l is `reconstruct(x)`; a = 1 - y_l is `intervene` with label l flipped.
+          From labels (x=None, y [B,18] required), the counterpart of `generate`: z_s = eps_s, z_c = loc_p + scale_p eps_c
+            at the walked labels (`sample=False`: z_s = 0, z_c = loc_p).
+        labels: distinct label indices in [0, 18), in output order (default: all 18); alphas: a non-empty 1-D sequence of
+        finite floats, taken as fp32 (default: 8 points from 0 to 1, both ends exact).  The noise of an image is drawn
+        once and shared by all its frames; c, `noise={"eps": [B,45], "U1", "U2"}` and `dtype` are as in `generate`.
+        Returns a fresh [B, L, T, 64, 64, 3] device tensor (L labels, T alphas), decoded in chunks of at most `max_rows`
+        frames, which bounds the memory and changes no value.
+        `self.last` = {"z": [B,L,T,45] fp32, "c": [18,18], "y_src": [B,18] int32 labels walked from (images) or None}.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        self._check_dtype(dtype)
+        if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
+            raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
+        labels = self._walk_labels(labels)
+        alphas = self._walk_alphas(alphas)
+        B = None
+        if x is not None:
+            x, B = self._gen_images(x)
+        elif y is None:
+            raise ValueError("walk needs images x or labels y")
+        if y is not None:
+            y = self._gen_labels(y, B, "y")
+            B = y.shape[0]
+        n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
+        L, T = len(labels), alphas.numel()
+        rows = B * L * T
+        if rows >= 1 << 31:
+            raise ValueError("walk of {} frames: at most 2^31 - 1".format(rows))
+        chunk = min(int(max_rows), rows)
+        out = torch.empty(B, L, T, 64, 64, 3, dtype=dtype, device=self.device)
+        z = torch.empty(B, L, T, self.z_dim, dtype=torch.float32, device=self.device)
+        y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if x is not None else None
+        out_rows, z_rows = out.view(rows, 64, 64, 3), z.view(rows, self.z_dim)
+        dec = self.engine.dec_bufs(chunk)
+        a = WalkLatentArgs()
+        a.batch, a.sample, a.n_labels, a.n_alpha = B, int(bool(sample)), L, T
+        a.labels[:L] = labels
+        alphas = alphas.to(self.device)
+        with self._fresh_noise():
+            self._gate(n, c_in=c)
+            if x is None:
+                a.mode = _lib.WALK_LABELS
+                self.engine.pack_weights()
+            else:
+                a.mode = _lib.WALK_IMAGES
+                b = self.engine.bufs(B)
+                self.engine.encoder_fwd(x, b)
+                io = self.engine.latent_io(b)
+                a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
+            a.alphas, a.y, a.eps = ptr(alphas), ptr(y), ptr(n["eps"])
+            a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
+            a.gate_ws, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(dec.get("z16")), ptr(y_used)
+            for r0 in range(0, rows, chunk):
+                nr = min(chunk, rows - r0)
+                a.row0, a.rows, a.z = r0, nr, ptr(z_rows[r0:])
+                _lib.check(self.lib.gccvae_walk_latent(C.byref(a), _stream()), "walk_latent")
+                self.engine.image_fwd(z_rows[r0:r0 + nr], dec, nr, dtype == torch.uint8, out=out_rows[r0:r0 + nr])
+        self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
+        return out
+
+    def _walk_labels(self, labels):
+        if labels is None:
+            return list(range(self.y_dim))
+        v = np.asarray(labels.cpu() if torch.is_tensor(labels) else labels)
+        if v.ndim != 1 or v.size == 0 or v.dtype.kind not in "iu":
+            raise ValueError("labels must be a non-empty 1-D sequence of integers, got {!r}".format(labels))
+        out = [int(t) for t in v]
+        if min(out) < 0 or max(out) >= self.y_dim or len(set(out)) != len(out):
+            raise ValueError("labels must be distinct indices in [0, {}), got {}".format(self.y_dim, out))
+        return out
+
+    @staticmethod
+    def _walk_alphas(alphas):
+        if alphas is None:
+            return torch.arange(8, dtype=torch.float64).div(7).float()     # 0/7 .. 7/7: both ends exact
+        try:
+            v = torch.as_tensor(alphas.detach().cpu() if torch.is_tensor(alphas) else alphas, dtype=torch.float32)
+        except (TypeError, ValueError, RuntimeError) as e:
+            raise ValueError("alphas must be a 1-D sequence of floats, got {!r}".format(alphas)) from e
+        if v.dim() != 1 or v.numel() == 0 or not bool(torch.isfinite(v).all()):
+            raise ValueError("alphas must be a non-empty 1-D sequence of finite floats, got {!r}".format(alphas))
+        return v.contiguous()
+
+    def swap(self, x_style, x_char, dtype=torch.float32):
+        """Characteristic swap: images decoded from z = [z_s of x_style, z_c of x_char], both posterior means (the style
+        of one image with the label-linked latents of another).  x_style and x_char are [B,64,64,3] each (fp32 in [0,1]
+        or uint8) and go through one encoder pass over 2B images; no gate and no prior are involved, so swap(x, x) is
+        reconstruct(x).  Returns a fresh [B,64,64,3] image as `generate` does; `self.last` = {"z": [B,45]}."""
+        self._check_dtype(dtype)
+        xs, B = self._gen_images(x_style)
+        xc, Bc = self._gen_images(x_char)
+        if Bc != B:
+            raise ValueError("x_style and x_char must hold as many images, got {} and {}".format(B, Bc))
+        if xs.dtype != xc.dtype:     # one of each: both as fp32 in [0,1], the division the kernels do on uint8 images
+            xs, xc = (t.to(torch.float32) / 255.0 if t.dtype == torch.uint8 else t for t in (xs, xc))
+        x = torch.cat([xs, xc])
+        b = self.engine.bufs(2 * B)
+        z = torch.empty(2 * B, self.z_dim, dtype=torch.float32, device=self.device)
+        out = torch.empty(B, 64, 64, 3, dtype=dtype, device=self.device)
+        self.engine.encoder_fwd(x, b)
+        a, io = GenLatentArgs(), self.engine.latent_io(b)
+        a.batch, a.mode, a.sample = 2 * B, _lib.GEN_RECONSTRUCT, 0
+        a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
+        a.gate_ws, a.z, a.z16 = ptr(self._gate_ws), ptr(z), io["z16"]
+        _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
+        # rows 0..B-1 become the swapped codes; z16 = bf16(z) elementwise, so composing its columns is exact
+        zs = self.z_style
+        z[:B, zs:].copy_(z[B:, zs:])
+        if b.get("z16") is not None:
+            b["z16"][:B, zs:self.z_dim].copy_(b["z16"][B:, zs:self.z_dim])
+        self.engine.image_fwd(z[:B], b, B, dtype == torch.uint8, out=out)
+        self.last = dict(z=z[:B])
+        return out
 
     # ---- importance-weighted log-likelihood (an extension: the reference scores a model by accuracy only) ------------
     def log_likelihood(self, x, y=None, k=100, c=None, noise=None, max_rows=8192, keep_log_w=False):
@@ -843,21 +977,11 @@ class Learner:
         if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
             raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
         K = int(k)
-        x, _ = self._prep_inputs(x, None)
+        x, B = self._gen_images(x)
         x = x.contiguous()
-        B = x.shape[0]
-        if B == 0:
-            raise ValueError("x holds no image")
         if y is not None:
             y = self._gen_labels(y, B, "y")
-        n = self._noise(noise, B, False, 0)
-        for key, shape in (("eps", (K, B, self.z_dim)), ("U_y", (K, B, self.y_dim)), ("U1", (18, 18)), ("U2", (18, 18))):
-            if n[key] is not None and tuple(n[key].shape) != shape:
-                raise ValueError("noise[{!r}] must be {}, got {}".format(key, list(shape), tuple(n[key].shape)))
-        if c is not None:
-            c = as_device_f32(c, self.device)
-            if tuple(c.shape) != (18, 18):
-                raise ValueError("c must be [18,18], got {}".format(tuple(c.shape)))
+        n, c = self._gen_noise_c(noise, c, {"eps": (K, B, self.z_dim), "U_y": (K, B, self.y_dim)})
         kc = max(1, min(K, int(max_rows) // B))
         b, dec = self.engine.bufs(B), self.engine.dec_bufs(B * kc)
         e = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)
