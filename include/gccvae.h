@@ -275,86 +275,60 @@ typedef struct {
 int gccvae_latent_bwd_partials(int batch);
 int gccvae_latent_bwd(const gccvae_latent_bwd_args* a, void* stream);
 
-/* ---- latent code of the generation path (no counterpart in the reference) ------------------------------------
- * One warp per image writes the z the decoder turns into an image, in one of three modes.  Notation: c is the gate
- * sample of gate_ws (gccvae_gate_fwd); loc_p(y,c), scale_p(y,c) are the conditional prior of networks.py:118-127
- * (scale after softplus and the [1e-3, 1e3] clip); eps [B,45] is N(0,1) with the layout of gccvae_latent_fwd
- * (columns 0..26 style dims, 27..44 classify dims).  Labels are nonzero -> 1.
+/* ---- latent code of the forward-only image calls (no counterpart in the reference) -----------------------------
+ * One warp per frame writes the z the decoder turns into an image.  Every image has F frames: F = 1 (n_labels = 0), or
+ * for a label walk F = n_labels * n_alpha, frame (l, t) of image b being row r = (b * n_labels + l) * n_alpha + t, which
+ * walks label labels[l] to the real value alphas[t] in the target prior and keeps the other 17 labels.  Notation: c is
+ * the gate sample of gate_ws (gccvae_gate_fwd); loc_p(y,c), scale_p(y,c) are the conditional prior of
+ * networks.py:118-127 (scale after softplus and the [1e-3, 1e3] clip); eps [B,45] is N(0,1) with the layout of
+ * gccvae_latent_fwd (columns 0..26 style dims, 27..44 classify dims).  Labels are nonzero -> 1.
  *   GCCVAE_GEN_GENERATE:     z_s = eps_s, z_c = loc_p(y_tgt,c) + scale_p(y_tgt,c) eps_c;
  *                            sample = 0: z_s = 0, z_c = loc_p(y_tgt,c).
  *   GCCVAE_GEN_RECONSTRUCT:  z = loc (posterior mean: relu / clipped softplus of the heads, networks.py:17-18,33-34);
- *                            sample = 1: z = loc + scale eps.
+ *                            sample = 1: z = loc + scale eps.  No prior step; a walk is rejected.
  *   GCCVAE_GEN_INTERVENE:    z as for RECONSTRUCT, then the classify dims move from y_src to y_tgt by the Gaussian
  *                            counterfactual  e = (z_c - loc_p(y_src,c)) / scale_p(y_src,c),
  *                            z_c' = z_c + (loc_p(y_tgt,c) - loc_p(y_src,c)) + (scale_p(y_tgt,c) - scale_p(y_src,c)) e
  *                            (y_src == y_tgt leaves z_c bit-identical); z_s is never touched.  y_src = NULL: the
  *                            classifier's decision on z_c, sigmoid(logit) > 0.5 (as gccvae_accuracy_f32 decides).
+ *                            y_tgt = NULL: y_tgt = y_src, valid only in a walk.
+ * In a walk the target prior is the prior at y_tgt with y_tgt,l replaced by alpha.  Its term of label l is exactly the
+ * boolean term at alpha = 0 and alpha = 1 and fmaf(alpha, P_true - P_false, P_false) otherwise, summed in the order of
+ * the prior (j = 0..17).  So a frame at alpha in {0, 1} is bit for bit the one-frame call of the same mode whose y_tgt
+ * has y_tgt,l = alpha, and (INTERVENE, y_tgt = NULL) the frame at alpha = y_src,l is RECONSTRUCT's z.
+ * Any finite alpha is valid (beyond [0, 1] the prior extrapolates).
  * Only RECONSTRUCT and INTERVENE read loc_pre / scale_pre; only GENERATE and INTERVENE read y_tgt; eps is read only when
- * sampling (eps = NULL: the Philox stream of gccvae_latent_fwd, which gccvae_draw_noise_f32 kind 0 reproduces). */
+ * sampling (eps = NULL: the Philox stream of gccvae_latent_fwd, which gccvae_draw_noise_f32 kind 0 reproduces).  Noise
+ * is drawn once per image (image b, dim d) and shared by all its frames.  The rows row0 .. row0 + rows - 1 are written
+ * at z / z16 rows 0 .. rows - 1 (one chunk of the decoder; one-frame calls pass row0 = 0, rows = B); y_src_out rows are
+ * written by the chunk that holds the image's first frame. */
 #define GCCVAE_GEN_GENERATE 1
 #define GCCVAE_GEN_RECONSTRUCT 2
 #define GCCVAE_GEN_INTERVENE 3
 typedef struct {
-  int batch;
+  int batch;               /* B images */
   int mode;                /* GCCVAE_GEN_* */
   int sample;              /* 0: means, 1: draw with eps (see above) */
   int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
+  int n_labels;            /* labels walked, 0..18 (0: one frame per image) */
+  int labels[18];          /* labels[0 .. n_labels-1]: distinct label indices in [0, 18), in row order */
+  int n_alpha;             /* values per walked label, >= 1 (walk) */
+  const float* alphas;     /* [n_alpha] device fp32, finite (walk) */
+  int row0, rows;          /* this chunk: rows row0 .. row0 + rows - 1 of the B * F */
   const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu (RECONSTRUCT, INTERVENE) */
   const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip */
-  const long long* y_tgt;  /* [B,18] int64 target labels (GENERATE, INTERVENE) */
+  const long long* y_tgt;  /* [B,18] int64 target labels (GENERATE; INTERVENE, or NULL in a walk) */
   const long long* y_src;  /* [B,18] int64 source labels (INTERVENE) or NULL */
-  const float* eps;        /* [B,45] N(0,1) or NULL -> Philox */
-  uint64_t seed, offset;   /* Philox key / counter base */
-  const int* step_dev;     /* optional device int added to `offset` */
-  const float* gate_ws;    /* from gccvae_gate_fwd */
-  /* outputs */
-  float* z;                /* [B,45] fp32 */
-  void* z16;               /* optional bf16 [B,64] copy of z, columns 45..63 zero (operand of the tensor-core fc1) */
-  int* y_src_out;          /* optional [B,18] int32: the y_src used (INTERVENE) */
-} gccvae_gen_latent_args;
-int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
-
-/* ---- latent code of a label walk (no counterpart in the reference) ---------------------------------------------
- * Frames of B images along n_labels labels at n_alpha values each: row r = (b * n_labels + l) * n_alpha + t walks
- * label labels[l] to the real value alphas[t] and keeps the other 17 labels.  Notation as gccvae_gen_latent; the
- * conditional prior at a walked label is the prior of networks.py:118-127 with y_l replaced by alpha.  Its term of
- * label l is exactly the boolean term at alpha = 0 and alpha = 1 and fmaf(alpha, P_true - P_false, P_false) otherwise,
- * summed in the order of the prior (j = 0..17), so frames at alpha in {0, 1} are bit-identical to gccvae_gen_latent
- * with that label set.  Any finite alpha is valid (beyond [0, 1] the prior extrapolates).
- *   GCCVAE_WALK_LABELS:  z_s = eps_s, z_c = loc_p(y(alpha),c) + scale_p(y(alpha),c) eps_c (GCCVAE_GEN_GENERATE);
- *                        sample = 0: z_s = 0, z_c = loc_p(y(alpha),c).
- *   GCCVAE_WALK_IMAGES:  z = the posterior mean (sample = 1: loc + scale eps), then the classify dims move from y_src to
- *                        y_src with label l at alpha by the counterfactual of GCCVAE_GEN_INTERVENE; y_src = y, or
- *                        (y = NULL) the classifier's decision on z_c.  The frame at alpha = y_src,l is the posterior z
- *                        bit for bit; z_s is never touched.
- * Noise is drawn once per image: eps (image b, dim d) as gccvae_gen_latent, shared by every frame of the image.  The
- * rows row0 .. row0 + rows - 1 are written at z / z16 rows 0 .. rows - 1 (one chunk of the decoder); y_src_out rows
- * are written by the chunk that holds the image's first row. */
-#define GCCVAE_WALK_LABELS 1
-#define GCCVAE_WALK_IMAGES 2
-typedef struct {
-  int batch;               /* B images */
-  int mode;                /* GCCVAE_WALK_* */
-  int sample;              /* 0: means, 1: draw with eps (see above) */
-  int n_labels;            /* labels walked, 1..18 */
-  int labels[18];          /* labels[0 .. n_labels-1]: distinct label indices in [0, 18), in row order */
-  int n_alpha;             /* values per label, >= 1 */
-  const float* alphas;     /* [n_alpha] device fp32, finite */
-  int row0, rows;          /* this chunk: rows row0 .. row0 + rows - 1 of the B * n_labels * n_alpha */
-  int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
-  const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu (IMAGES) */
-  const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip (IMAGES) */
-  const long long* y;      /* [B,18] int64 labels, nonzero = 1: the labels (LABELS), y_src or NULL (IMAGES) */
   const float* eps;        /* [B,45] N(0,1) or NULL -> Philox */
   uint64_t seed, offset;   /* Philox key / counter base */
   const int* step_dev;     /* optional device int added to `offset` */
   const float* gate_ws;    /* from gccvae_gate_fwd */
   /* outputs (at least one of z, z16) */
   float* z;                /* optional [rows,45] fp32 (operand of the fp32 decoder) */
-  void* z16;               /* optional bf16 [rows,64], columns 45..63 zero (operand of the tensor-core fc1) */
-  int* y_src_out;          /* optional [B,18] int32: the y_src used (IMAGES) */
-} gccvae_walk_latent_args;
-int gccvae_walk_latent(const gccvae_walk_latent_args* a, void* stream);
+  void* z16;               /* optional bf16 [rows,64] copy of z, columns 45..63 zero (operand of the tensor-core fc1) */
+  int* y_src_out;          /* optional [B,18] int32: the y_src used (INTERVENE) */
+} gccvae_gen_latent_args;
+int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
 
 /* ---- importance-weighted log-likelihood (no counterpart in the reference) -------------------------------------
  * log p(x [, y]) >= log p_hat = logsumexp_k log w_k - ln K over K samples per image, with proposal q(z|x) (labelled) or

@@ -1,7 +1,7 @@
 """Throughput of the label walk on the bf16 engine: Learner.walk from images at B = 64 (uint8 images, the shipped
 checkpoint), all 18 labels, 8 values each (9216 decoded rows per call, two chunks at the default max_rows = 8192), for
 both output dtypes; event, host issue and device time per call, decoded rows/s, the peak device memory of a call, and
-the walk's latent kernel (gccvae_walk_latent) alone.
+the latent kernel of the walk (gccvae_gen_latent) alone.
 
     python scripts/walk_bench.py [--batch 64] [--out result.json]
 
@@ -73,14 +73,14 @@ def main():
     chunk = min(8192, rows)
     io, dec = eng.latent_io(eng.bufs(B)), eng.dec_bufs(chunk)
     al = torch.tensor(alphas, dtype=torch.float32, device="cuda")
-    w = L.WalkLatentArgs()
-    w.batch, w.mode, w.sample, w.n_labels, w.n_alpha = B, L.WALK_IMAGES, 0, 18, T
+    w = L.GenLatentArgs()
+    w.batch, w.mode, w.sample, w.n_labels, w.n_alpha = B, L.GEN_INTERVENE, 0, 18, T
     w.labels[:18] = list(range(18))
     w.alphas, w.row0, w.rows = L.ptr(al), 0, chunk
     w.loc_pre, w.scale_pre, w.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
     w.gate_ws, w.z16 = L.ptr(lrn._gate_ws), L.ptr(dec["z16"])
     st = torch.cuda.current_stream().cuda_stream
-    launch = lambda: L.check(eng.lib.gccvae_walk_latent(C.byref(w), st), "walk_latent")
+    launch = lambda: L.check(eng.lib.gccvae_gen_latent(C.byref(w), st), "gen_latent")
     for _ in range(8):
         launch()
     torch.cuda.synchronize()
@@ -92,8 +92,8 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     t = e0.elapsed_time(e1) / 1e3 / a.kernel_launches
-    res["walk_latent_kernel"] = dict(rows=chunk, us_per_launch=round(t * 1e3 * 1e3, 2),
-                                     rows_per_s=round(chunk / t))
+    res["gen_latent_kernel"] = dict(rows=chunk, us_per_launch=round(t * 1e3 * 1e3, 2),
+                                    rows_per_s=round(chunk / t))
     text = json.dumps(res, indent=1)
     print(text)
     if a.out:

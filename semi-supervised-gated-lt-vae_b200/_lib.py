@@ -40,7 +40,8 @@ GEN_GENERATE, GEN_RECONSTRUCT, GEN_INTERVENE = 1, 2, 3
 class GenLatentArgs(C.Structure):
     """gccvae_gen_latent_args (include/gccvae.h)."""
     _fields_ = [
-        ("batch", C.c_int), ("mode", C.c_int), ("sample", C.c_int), ("ld_pre", C.c_int),
+        ("batch", C.c_int), ("mode", C.c_int), ("sample", C.c_int), ("ld_pre", C.c_int), ("n_labels", C.c_int),
+        ("labels", C.c_int * 18), ("n_alpha", C.c_int), ("alphas", C.c_void_p), ("row0", C.c_int), ("rows", C.c_int),
         ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y_tgt", C.c_void_p), ("y_src", C.c_void_p),
         ("eps", C.c_void_p), ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p),
         ("gate_ws", C.c_void_p), ("z", C.c_void_p), ("z16", C.c_void_p), ("y_src_out", C.c_void_p),
@@ -54,20 +55,6 @@ class IwLatentArgs(C.Structure):
         ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y", C.c_void_p), ("eps", C.c_void_p), ("U_y", C.c_void_p),
         ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p), ("gate_ws", C.c_void_p),
         ("lw_part", C.c_void_p), ("z", C.c_void_p), ("z16", C.c_void_p),
-    ]
-
-
-WALK_LABELS, WALK_IMAGES = 1, 2
-
-
-class WalkLatentArgs(C.Structure):
-    """gccvae_walk_latent_args (include/gccvae.h)."""
-    _fields_ = [
-        ("batch", C.c_int), ("mode", C.c_int), ("sample", C.c_int), ("n_labels", C.c_int), ("labels", C.c_int * 18),
-        ("n_alpha", C.c_int), ("alphas", C.c_void_p), ("row0", C.c_int), ("rows", C.c_int), ("ld_pre", C.c_int),
-        ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y", C.c_void_p), ("eps", C.c_void_p),
-        ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p), ("gate_ws", C.c_void_p),
-        ("z", C.c_void_p), ("z16", C.c_void_p), ("y_src_out", C.c_void_p),
     ]
 
 
@@ -185,7 +172,6 @@ SIGNATURES = {
     "gccvae_latent_fwd": (_I, [C.POINTER(LatentFwdArgs), _P]),
     "gccvae_latent_bwd_partials": (_I, [_I]),
     "gccvae_gen_latent": (_I, [C.POINTER(GenLatentArgs), _P]),
-    "gccvae_walk_latent": (_I, [C.POINTER(WalkLatentArgs), _P]),
     "gccvae_iw_latent": (_I, [C.POINTER(IwLatentArgs), _P]),
     "gccvae_iw_accumulate": (_I, [_I, _I, _I, _I, _P, _P, _P, _P, _I, _I, _P, _P, _P]),
     "gccvae_latent_bwd": (_I, [C.POINTER(LatentBwdArgs), _P]),

@@ -692,21 +692,56 @@ __global__ void __launch_bounds__(256) accuracy_kernel(const float* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------
-// latent code of the generation path (gccvae_gen_latent, include/gccvae.h): one warp per image, as latent_fwd
+// latent code of the forward-only image calls (gccvae_gen_latent, include/gccvae.h): one warp per frame
 // ---------------------------------------------------------------------------------------------
+// prior_i with label l at the real value alpha: at alpha = 0 / 1 the term of l is the prior's own select (so the result is
+// prior_i's bit for bit), otherwise alpha P_true + (1 - alpha) P_false as one fmaf; the sum keeps prior_i's order.
+// l = Y, alpha = 0 walks no label: ymask has no bit Y, so every term is prior_i's select
+__device__ __forceinline__ void prior_walk_i(const GateSmem& g, uint32_t ymask, int l, float alpha, int i, float& mp,
+                                             float& spr) {
+  const bool between = !(alpha == 0.0f || alpha == 1.0f);
+  const uint32_t m = alpha == 1.0f ? (ymask | (1u << l)) : (ymask & ~(1u << l));
+  float a = 0.0f, s = 0.0f;
+#pragma unroll
+  for (int j = 0; j < Y; ++j) {
+    const int q = j * ZC + i;
+    const bool y1 = (m >> j) & 1u;
+    float ta = y1 ? g.Plt[q] : g.Plf[q], ts = y1 ? g.Pst[q] : g.Psf[q];
+    if (between && j == l) {
+      ta = fmaf(alpha, g.Plt[q] - g.Plf[q], g.Plf[q]);
+      ts = fmaf(alpha, g.Pst[q] - g.Psf[q], g.Psf[q]);
+    }
+    a += ta;
+    s += ts;
+  }
+  mp = a;
+  spr = s;
+}
+
 __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_latent_args a) {
   pdl_prologue();
   __shared__ __align__(16) GateSmem g;
   __shared__ float s_zc[WARPS][ZC];
   load_gate_smem(g, a.gate_ws);
   __syncthreads();
-  if (a.step_dev) a.offset += (uint64_t)(*a.step_dev);
+  // a local, not a.offset +=: a written parameter struct of this size loses its pointers' global address space
+  const uint64_t offset = a.offset + (a.step_dev ? (uint64_t)(*a.step_dev) : 0ull);
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int ldp = a.ld_pre > 0 ? a.ld_pre : Z;
   const bool from_image = a.mode != GCCVAE_GEN_GENERATE;
+  const int per_image = a.n_labels > 0 ? a.n_labels * a.n_alpha : 1;
   float* zcs = s_zc[wid];
 
-  for (int b = blockIdx.x * WARPS + wid; b < a.batch; b += gridDim.x * WARPS) {
+  for (int r = blockIdx.x * WARPS + wid; r < a.rows; r += gridDim.x * WARPS) {
+    const int gr = a.row0 + r, b = gr / per_image, f = gr - b * per_image;
+    int l = Y;          // one frame per image: no walked label
+    float alpha = 0.0f;
+    if (a.n_labels > 0) {
+      const int li = f / a.n_alpha;
+#pragma unroll
+      for (int k = 0; k < Y; ++k) l = k == li ? a.labels[k] : l;   // constant-bank reads: a dynamic index would copy the params to the stack
+      alpha = a.alphas[f - li * a.n_alpha];
+    }
     // --- posterior (Reconstruct / Intervene) or N(0,1) style dims (Generate) ------------------------------------
     float zv[2] = {0.0f, 0.0f};
 #pragma unroll
@@ -717,18 +752,17 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
       if (from_image) {
         float loc, sc;
         head_act(a.loc_pre[(size_t)b * ldp + d], a.scale_pre[(size_t)b * ldp + d], loc, sc);
-        z = a.sample ? fmaf(sc, draw_eps(a.eps, a.seed, a.offset, b, d), loc) : loc;
+        z = a.sample ? fmaf(sc, draw_eps(a.eps, a.seed, offset, b, d), loc) : loc;
       } else if (d < ZS && a.sample) {
-        z = draw_eps(a.eps, a.seed, a.offset, b, d);
+        z = draw_eps(a.eps, a.seed, offset, b, d);
       }
       zv[h] = z;
       if (d >= ZS) zcs[d - ZS] = z;
     }
     __syncwarp();
-    // --- labels: target, and (Intervene) source = given or the classifier's decision on z_c -------------------------
+    // --- labels: (Intervene) source = given or the classifier's decision on z_c; target = given or the source --------
     bool yt = false, ys = false;
     if (lane < Y) {
-      if (a.mode != GCCVAE_GEN_RECONSTRUCT) yt = a.y_tgt[(size_t)b * Y + lane] != 0;
       if (a.mode == GCCVAE_GEN_INTERVENE) {
         if (a.y_src != nullptr) {
           ys = a.y_src[(size_t)b * Y + lane] != 0;
@@ -738,18 +772,19 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
           for (int i = 0; i < ZC; ++i) acc = fmaf(zcs[i], g.M[i * Y + lane], acc);
           ys = sigmoid_f(acc) > 0.5f;
         }
-        if (a.y_src_out != nullptr) a.y_src_out[(size_t)b * Y + lane] = ys ? 1 : 0;
+        if (a.y_src_out != nullptr && f == 0) a.y_src_out[(size_t)b * Y + lane] = ys ? 1 : 0;
       }
+      if (a.mode != GCCVAE_GEN_RECONSTRUCT) yt = a.y_tgt != nullptr ? a.y_tgt[(size_t)b * Y + lane] != 0 : ys;
     }
     const uint32_t tmask = __ballot_sync(0xffffffffu, yt), smask = __ballot_sync(0xffffffffu, ys);
-    // --- classify dims through the conditional prior (lane i < ZC: classify dim i) -------------------------------------
+    // --- classify dims through the conditional prior at the target, label l at alpha (lane i < ZC: classify dim i) -----
     if (lane < ZC && a.mode != GCCVAE_GEN_RECONSTRUCT) {
       float mt, st;
-      prior_i(g, tmask, lane, mt, st);
+      prior_walk_i(g, tmask, l, alpha, lane, mt, st);
       const float spt = clip_f(softplus_f(st), 1e-3f, 1e3f);
       float zc;
       if (a.mode == GCCVAE_GEN_GENERATE) {
-        zc = a.sample ? fmaf(spt, draw_eps(a.eps, a.seed, a.offset, b, ZS + lane), mt) : mt;
+        zc = a.sample ? fmaf(spt, draw_eps(a.eps, a.seed, offset, b, ZS + lane), mt) : mt;
       } else {
         float ms, ss;
         prior_i(g, smask, lane, ms, ss);
@@ -766,10 +801,10 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
       const int d = lane + 32 * h;
       if (d < Z) {
         const float z = d >= ZS ? zcs[d - ZS] : zv[h];
-        a.z[(size_t)b * Z + d] = z;
-        if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)b * 64 + d] = __float2bfloat16(z);
+        if (a.z != nullptr) a.z[(size_t)r * Z + d] = z;
+        if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(z);
       } else if (d < 64 && a.z16 != nullptr) {
-        reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)b * 64 + d] = __float2bfloat16(0.0f);
+        reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(0.0f);
       }
     }
     __syncwarp();
@@ -920,118 +955,6 @@ __global__ void draw_iw_noise_kernel(int kind, uint64_t seed, uint64_t offset, i
   out[t] = kind == 4 ? draw_iw_eps(nullptr, seed, offset, B, b, k, d) : draw_iw_uy(nullptr, seed, offset, B, b, k, d);
 }
 
-// ---------------------------------------------------------------------------------------------
-// latent code of a label walk (gccvae_walk_latent, include/gccvae.h): one warp per decoded row
-// ---------------------------------------------------------------------------------------------
-// prior_i with label l at the real value alpha: at alpha = 0 / 1 the term of l is the prior's own select (so the result is
-// prior_i's bit for bit), otherwise alpha P_true + (1 - alpha) P_false as one fmaf; the sum keeps prior_i's order
-__device__ __forceinline__ void prior_walk_i(const GateSmem& g, uint32_t ymask, int l, float alpha, int i, float& mp,
-                                             float& spr) {
-  const bool between = !(alpha == 0.0f || alpha == 1.0f);
-  const uint32_t m = alpha == 1.0f ? (ymask | (1u << l)) : (ymask & ~(1u << l));
-  float a = 0.0f, s = 0.0f;
-#pragma unroll
-  for (int j = 0; j < Y; ++j) {
-    const int q = j * ZC + i;
-    const bool y1 = (m >> j) & 1u;
-    float ta = y1 ? g.Plt[q] : g.Plf[q], ts = y1 ? g.Pst[q] : g.Psf[q];
-    if (between && j == l) {
-      ta = fmaf(alpha, g.Plt[q] - g.Plf[q], g.Plf[q]);
-      ts = fmaf(alpha, g.Pst[q] - g.Psf[q], g.Psf[q]);
-    }
-    a += ta;
-    s += ts;
-  }
-  mp = a;
-  spr = s;
-}
-
-__global__ void __launch_bounds__(WARPS * 32) walk_latent_kernel(gccvae_walk_latent_args a) {
-  pdl_prologue();
-  __shared__ __align__(16) GateSmem g;
-  __shared__ float s_zc[WARPS][ZC];
-  load_gate_smem(g, a.gate_ws);
-  __syncthreads();
-  if (a.step_dev) a.offset += (uint64_t)(*a.step_dev);
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const int ldp = a.ld_pre > 0 ? a.ld_pre : Z;
-  const bool from_image = a.mode == GCCVAE_WALK_IMAGES;
-  const int per_image = a.n_labels * a.n_alpha;
-  float* zcs = s_zc[wid];
-
-  for (int r = blockIdx.x * WARPS + wid; r < a.rows; r += gridDim.x * WARPS) {
-    const int gr = a.row0 + r, b = gr / per_image, f = gr - b * per_image;
-    const int li = f / a.n_alpha;
-    int l = 0;
-#pragma unroll
-    for (int k = 0; k < Y; ++k) l = k == li ? a.labels[k] : l;   // constant-bank reads: a dynamic index would copy the params to the stack
-    const float alpha = a.alphas[f - li * a.n_alpha];
-    // --- the image's z before the walk: posterior (images) or N(0,1) style dims (labels), as gen_latent_kernel -----------
-    float zv[2] = {0.0f, 0.0f};
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int d = lane + 32 * h;
-      if (d >= Z) continue;
-      float z = 0.0f;
-      if (from_image) {
-        float loc, sc;
-        head_act(a.loc_pre[(size_t)b * ldp + d], a.scale_pre[(size_t)b * ldp + d], loc, sc);
-        z = a.sample ? fmaf(sc, draw_eps(a.eps, a.seed, a.offset, b, d), loc) : loc;
-      } else if (d < ZS && a.sample) {
-        z = draw_eps(a.eps, a.seed, a.offset, b, d);
-      }
-      zv[h] = z;
-      if (d >= ZS) zcs[d - ZS] = z;
-    }
-    __syncwarp();
-    // --- labels the walk starts from: given, or (images, y = NULL) the classifier's decision on z_c ---------------------
-    bool y1 = false;
-    if (lane < Y) {
-      if (a.y != nullptr) {
-        y1 = a.y[(size_t)b * Y + lane] != 0;
-      } else {
-        float acc = g.b[lane];
-#pragma unroll
-        for (int i = 0; i < ZC; ++i) acc = fmaf(zcs[i], g.M[i * Y + lane], acc);
-        y1 = sigmoid_f(acc) > 0.5f;
-      }
-      if (a.y_src_out != nullptr && f == 0) a.y_src_out[(size_t)b * Y + lane] = y1 ? 1 : 0;
-    }
-    const uint32_t ymask = __ballot_sync(0xffffffffu, y1);
-    // --- classify dims under the prior with label l at alpha (lane i < ZC: classify dim i) ------------------------------
-    if (lane < ZC) {
-      float mt, st;
-      prior_walk_i(g, ymask, l, alpha, lane, mt, st);
-      const float spt = clip_f(softplus_f(st), 1e-3f, 1e3f);
-      float zc;
-      if (!from_image) {
-        zc = a.sample ? fmaf(spt, draw_eps(a.eps, a.seed, a.offset, b, ZS + lane), mt) : mt;
-      } else {
-        float ms, ss;
-        prior_i(g, ymask, lane, ms, ss);
-        const float sps = clip_f(softplus_f(ss), 1e-3f, 1e3f);
-        const float z0 = zcs[lane];
-        const float e = (z0 - ms) / sps;
-        zc = fmaf(spt - sps, e, z0 + (mt - ms));   // the expression of gen_latent_kernel's intervention
-      }
-      zcs[lane] = zc;
-    }
-    __syncwarp();
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int d = lane + 32 * h;
-      if (d < Z) {
-        const float z = d >= ZS ? zcs[d - ZS] : zv[h];
-        if (a.z != nullptr) a.z[(size_t)r * Z + d] = z;
-        if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(z);
-      } else if (d < 64 && a.z16 != nullptr) {
-        reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(0.0f);
-      }
-    }
-    __syncwarp();
-  }
-}
-
 }  // namespace gccvae
 
 using namespace gccvae;
@@ -1108,48 +1031,33 @@ extern "C" int gccvae_latent_fwd(const gccvae_latent_fwd_args* a, void* stream) 
 
 extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) {
   GCC_REQUIRE(a, "gen_latent: null args");
-  GCC_REQUIRE(a->batch > 0, "gen_latent: bad batch %d", a->batch);
   GCC_REQUIRE(a->mode >= GCCVAE_GEN_GENERATE && a->mode <= GCCVAE_GEN_INTERVENE,
               "gen_latent: mode %d (1 generate, 2 reconstruct, 3 intervene)", a->mode);
-  GCC_REQUIRE(a->gate_ws && a->z, "gen_latent: null pointer");
-  GCC_REQUIRE(a->mode == GCCVAE_GEN_GENERATE || (a->loc_pre && a->scale_pre && a->ld_pre >= 0),
-              "gen_latent: reconstruct / intervene need loc_pre and scale_pre");
-  GCC_REQUIRE(a->mode == GCCVAE_GEN_RECONSTRUCT || a->y_tgt, "gen_latent: generate / intervene need y_tgt");
-  GCC_REQUIRE((uintptr_t)a->z % 4 == 0 && (uintptr_t)a->eps % 4 == 0 && (uintptr_t)a->loc_pre % 4 == 0 &&
-                  (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y_tgt % 8 == 0 && (uintptr_t)a->y_src % 8 == 0 &&
-                  (uintptr_t)a->y_src_out % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
-              "gen_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
-  GCC_CUDA(launch_aux(gen_latent_kernel, dim3(latent_grid(a->batch)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
-  GCC_CHECK_LAUNCH("gen_latent");
-  return GCCVAE_OK;
-}
-
-extern "C" int gccvae_walk_latent(const gccvae_walk_latent_args* a, void* stream) {
-  GCC_REQUIRE(a, "walk_latent: null args");
-  GCC_REQUIRE(a->mode == GCCVAE_WALK_LABELS || a->mode == GCCVAE_WALK_IMAGES, "walk_latent: mode %d (1 labels, 2 images)",
-              a->mode);
-  GCC_REQUIRE(a->batch > 0 && a->n_labels >= 1 && a->n_labels <= Y && a->n_alpha >= 1,
-              "walk_latent: bad sizes B=%d labels=%d alphas=%d", a->batch, a->n_labels, a->n_alpha);
-  const long long total = (long long)a->batch * a->n_labels * a->n_alpha;
-  GCC_REQUIRE(total < (1LL << 31), "walk_latent: too many rows");
+  GCC_REQUIRE(a->batch > 0 && a->n_labels >= 0 && a->n_labels <= Y && (a->n_labels == 0 || a->n_alpha >= 1),
+              "gen_latent: bad sizes B=%d labels=%d alphas=%d", a->batch, a->n_labels, a->n_alpha);
+  GCC_REQUIRE(a->n_labels == 0 || a->mode != GCCVAE_GEN_RECONSTRUCT, "gen_latent: reconstruct walks no label");
+  const long long total = (long long)a->batch * (a->n_labels > 0 ? (long long)a->n_labels * a->n_alpha : 1LL);
+  GCC_REQUIRE(total < (1LL << 31), "gen_latent: too many rows");
   GCC_REQUIRE(a->row0 >= 0 && a->rows >= 1 && (long long)a->row0 + a->rows <= total,
-              "walk_latent: chunk %d + %d outside the %lld rows", a->row0, a->rows, total);
+              "gen_latent: chunk %d + %d outside the %lld rows", a->row0, a->rows, total);
   unsigned seen = 0;
   for (int i = 0; i < a->n_labels; ++i) {
     GCC_REQUIRE(a->labels[i] >= 0 && a->labels[i] < Y && !((seen >> a->labels[i]) & 1u),
-                "walk_latent: labels must be distinct indices in [0, 18)");
+                "gen_latent: labels must be distinct indices in [0, 18)");
     seen |= 1u << a->labels[i];
   }
-  GCC_REQUIRE(a->alphas && a->gate_ws && (a->z || a->z16), "walk_latent: null pointer");
-  GCC_REQUIRE(a->mode == GCCVAE_WALK_LABELS || (a->loc_pre && a->scale_pre && a->ld_pre >= 0),
-              "walk_latent: images mode needs loc_pre and scale_pre");
-  GCC_REQUIRE(a->mode == GCCVAE_WALK_IMAGES || a->y, "walk_latent: labels mode needs y");
+  GCC_REQUIRE(a->gate_ws && (a->z || a->z16) && (a->n_labels == 0 || a->alphas), "gen_latent: null pointer");
+  GCC_REQUIRE(a->mode == GCCVAE_GEN_GENERATE || (a->loc_pre && a->scale_pre && a->ld_pre >= 0),
+              "gen_latent: reconstruct / intervene need loc_pre and scale_pre");
+  GCC_REQUIRE(a->mode != GCCVAE_GEN_GENERATE || a->y_tgt, "gen_latent: generate needs y_tgt");
+  GCC_REQUIRE(a->mode != GCCVAE_GEN_INTERVENE || a->y_tgt || a->n_labels > 0,
+              "gen_latent: intervene needs y_tgt unless it walks labels");
   GCC_REQUIRE((uintptr_t)a->z % 4 == 0 && (uintptr_t)a->eps % 4 == 0 && (uintptr_t)a->alphas % 4 == 0 &&
-                  (uintptr_t)a->loc_pre % 4 == 0 && (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y % 8 == 0 &&
-                  (uintptr_t)a->y_src_out % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
-              "walk_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
-  GCC_CUDA(launch_aux(walk_latent_kernel, dim3(latent_grid(a->rows)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
-  GCC_CHECK_LAUNCH("walk_latent");
+                  (uintptr_t)a->loc_pre % 4 == 0 && (uintptr_t)a->scale_pre % 4 == 0 && (uintptr_t)a->y_tgt % 8 == 0 &&
+                  (uintptr_t)a->y_src % 8 == 0 && (uintptr_t)a->y_src_out % 4 == 0 && (uintptr_t)a->z16 % 16 == 0,
+              "gen_latent: misaligned pointer (fp32 / int32: 4 bytes, int64: 8, z16: 16)");
+  GCC_CUDA(launch_aux(gen_latent_kernel, dim3(latent_grid(a->rows)), dim3(WARPS * 32), 0, (cudaStream_t)stream, *a));
+  GCC_CHECK_LAUNCH("gen_latent");
   return GCCVAE_OK;
 }
 

@@ -38,7 +38,7 @@ import torch
 
 from . import _lib, dp
 from ._lib import (GATE_WS_FLOATS, LATENT_PARTIAL_FLOATS, RESULT_SLOT_FLOATS, ChainBwdArgs, ChainFwdArgs, DpArgs,
-                   GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, WalkLatentArgs, ptr)
+                   GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
 from .engine import Engine, _stream
 from .networks import Classifier, Conditional_Prior, Decoder, Encoder, _default_device, as_device_f32
 from .params import ParamStore, keras_default_init
@@ -748,13 +748,13 @@ class Learner:
         conditional prior p(z_c|y,c) (networks.py:118-127); `sample=False`: z_s = 0, z_c = loc_p(y,c).
         Returns a fresh [B,64,64,3] NHWC device tensor: fp32 sigmoid values (`dtype=torch.float32`) or uint8
         min(255, rint(255 x)) (`dtype=torch.uint8`).  See `intervene` for c, noise and `last`."""
-        return self._generation(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype)
+        return self._image_call(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype)
 
     def reconstruct(self, x, sample=False, noise=None, dtype=torch.float32):
         """Decoded posterior of images x [B,64,64,3] (fp32 in [0,1] or uint8 0..255): z = the posterior mean (heads after
         relu / clipped softplus, networks.py:17-18,33-34); `sample=True`: z = loc + scale eps.  Returns the image as
         `generate` does."""
-        return self._generation(_lib.GEN_RECONSTRUCT, x, None, None, sample, None, noise, dtype)
+        return self._image_call(_lib.GEN_RECONSTRUCT, x, None, None, sample, None, noise, dtype)
 
     def intervene(self, x, y_new, y=None, sample=False, c=None, noise=None, dtype=torch.float32):
         """Counterfactual of images x: z as in `reconstruct`, then the classify dims move from the labels y to y_new
@@ -768,7 +768,7 @@ class Learner:
         explicit (eps layout: style dims 0..26, classify dims 27..44); without it every call draws new noise.
         `self.last` = {"z": [B,45], "c": [18,18], "y_src": [B,18] int32 labels moved from (intervene) or None}.
         In data-parallel runs every rank works on its own batch; there is no collective."""
-        return self._generation(_lib.GEN_INTERVENE, x, y_new, y, sample, c, noise, dtype)
+        return self._image_call(_lib.GEN_INTERVENE, x, y_new, y, sample, c, noise, dtype)
 
     def _gen_labels(self, y, B, what):
         t = torch.as_tensor(y) if not torch.is_tensor(y) else y
@@ -801,37 +801,71 @@ class Learner:
                 raise ValueError("c must be [18,18], got {}".format(tuple(c.shape)))
         return n, c
 
-    def _generation(self, mode, x, y_tgt, y_src, sample, c, noise, dtype):
+    @staticmethod
+    def _check_max_rows(max_rows):
+        if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
+            raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
+        return int(max_rows)
+
+    def _image_call(self, mode, x, y_tgt, y_src, sample, c, noise, dtype, walk=None):
+        """generate / reconstruct / intervene (one frame per image, decoded in `bufs(B)`) and, with walk = (labels,
+        alphas, max_rows), `walk` (frames decoded in chunks through `dec_bufs`): checks, gate, encoder or weight packing,
+        then per chunk gccvae_gen_latent and the decoder into the chunk's rows of the output."""
         self._check_dtype(dtype)
+        frames = ()
+        if walk is not None:
+            max_rows = self._check_max_rows(walk[2])
+            labels, alphas = self._walk_labels(walk[0]), self._walk_alphas(walk[1])
+            frames = (len(labels), alphas.numel())
         B = None
         if x is not None:
             x, B = self._gen_images(x)
+        elif walk is not None and y_tgt is None:
+            raise ValueError("walk needs images x or labels y")
         if y_tgt is not None:
             y_tgt = self._gen_labels(y_tgt, B, "y" if x is None else "y_new")
             B = y_tgt.shape[0]
         if y_src is not None:
             y_src = self._gen_labels(y_src, B, "y")
         n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
-        b = self.engine.bufs(B)
-        z = torch.empty(B, self.z_dim, dtype=torch.float32, device=self.device)
+        rows = B * math.prod(frames)
+        if rows >= 1 << 31:
+            raise ValueError("walk of {} frames: at most 2^31 - 1".format(rows))
+        out = torch.empty(B, *frames, 64, 64, 3, dtype=dtype, device=self.device)
+        z = torch.empty(B, *frames, self.z_dim, dtype=torch.float32, device=self.device)
         y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if mode == _lib.GEN_INTERVENE else None
+        a = GenLatentArgs()
+        a.batch, a.mode, a.sample = B, mode, int(bool(sample))
+        if walk is None:
+            dec, chunks = self.engine.bufs(B), [(0, B, z, out)]
+        else:
+            chunk = min(max_rows, rows)
+            dec = self.engine.dec_bufs(chunk)
+            z_rows, out_rows = z.view(rows, self.z_dim), out.view(rows, 64, 64, 3)
+            chunks = [(r0, min(chunk, rows - r0), z_rows[r0:r0 + chunk], out_rows[r0:r0 + chunk])
+                      for r0 in range(0, rows, chunk)]
+            a.n_labels, a.n_alpha = frames
+            a.labels[:len(labels)] = labels
+            alphas = alphas.to(self.device)
+            a.alphas = ptr(alphas)
         with self._fresh_noise():
             self._gate(n, c_in=c)
             if x is None:
                 self.engine.pack_weights()
             else:
+                b = self.engine.bufs(B)
                 self.engine.encoder_fwd(x, b)
-            a, io = GenLatentArgs(), self.engine.latent_io(b)
-            a.batch, a.mode, a.sample = B, mode, int(bool(sample))
-            if x is not None:
+                io = self.engine.latent_io(b)
                 a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
             a.y_tgt, a.y_src, a.eps = ptr(y_tgt), ptr(y_src), ptr(n["eps"])
             a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
-            a.gate_ws, a.z, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(z), io["z16"], ptr(y_used)
-            _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
-            img = self.engine.image_fwd(z, b, B, dtype == torch.uint8)
+            a.gate_ws, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(dec.get("z16")), ptr(y_used)
+            for r0, nr, z_chunk, out_chunk in chunks:
+                a.row0, a.rows, a.z = r0, nr, ptr(z_chunk)
+                _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
+                self.engine.image_fwd(z_chunk, dec, nr, dtype == torch.uint8, out=out_chunk)
         self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
-        return img
+        return out
 
     def walk(self, x=None, y=None, labels=None, alphas=None, sample=False, c=None, noise=None, dtype=torch.float32,
              max_rows=8192):
@@ -851,55 +885,9 @@ class Learner:
         frames, which bounds the memory and changes no value.
         `self.last` = {"z": [B,L,T,45] fp32, "c": [18,18], "y_src": [B,18] int32 labels walked from (images) or None}.
         In data-parallel runs every rank works on its own batch; there is no collective."""
-        self._check_dtype(dtype)
-        if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
-            raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
-        labels = self._walk_labels(labels)
-        alphas = self._walk_alphas(alphas)
-        B = None
-        if x is not None:
-            x, B = self._gen_images(x)
-        elif y is None:
-            raise ValueError("walk needs images x or labels y")
-        if y is not None:
-            y = self._gen_labels(y, B, "y")
-            B = y.shape[0]
-        n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
-        L, T = len(labels), alphas.numel()
-        rows = B * L * T
-        if rows >= 1 << 31:
-            raise ValueError("walk of {} frames: at most 2^31 - 1".format(rows))
-        chunk = min(int(max_rows), rows)
-        out = torch.empty(B, L, T, 64, 64, 3, dtype=dtype, device=self.device)
-        z = torch.empty(B, L, T, self.z_dim, dtype=torch.float32, device=self.device)
-        y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if x is not None else None
-        out_rows, z_rows = out.view(rows, 64, 64, 3), z.view(rows, self.z_dim)
-        dec = self.engine.dec_bufs(chunk)
-        a = WalkLatentArgs()
-        a.batch, a.sample, a.n_labels, a.n_alpha = B, int(bool(sample)), L, T
-        a.labels[:L] = labels
-        alphas = alphas.to(self.device)
-        with self._fresh_noise():
-            self._gate(n, c_in=c)
-            if x is None:
-                a.mode = _lib.WALK_LABELS
-                self.engine.pack_weights()
-            else:
-                a.mode = _lib.WALK_IMAGES
-                b = self.engine.bufs(B)
-                self.engine.encoder_fwd(x, b)
-                io = self.engine.latent_io(b)
-                a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
-            a.alphas, a.y, a.eps = ptr(alphas), ptr(y), ptr(n["eps"])
-            a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
-            a.gate_ws, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(dec.get("z16")), ptr(y_used)
-            for r0 in range(0, rows, chunk):
-                nr = min(chunk, rows - r0)
-                a.row0, a.rows, a.z = r0, nr, ptr(z_rows[r0:])
-                _lib.check(self.lib.gccvae_walk_latent(C.byref(a), _stream()), "walk_latent")
-                self.engine.image_fwd(z_rows[r0:r0 + nr], dec, nr, dtype == torch.uint8, out=out_rows[r0:r0 + nr])
-        self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
-        return out
+        if x is None:
+            return self._image_call(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype, (labels, alphas, max_rows))
+        return self._image_call(_lib.GEN_INTERVENE, x, None, y, sample, c, noise, dtype, (labels, alphas, max_rows))
 
     def _walk_labels(self, labels):
         if labels is None:
@@ -942,7 +930,7 @@ class Learner:
         out = torch.empty(B, 64, 64, 3, dtype=dtype, device=self.device)
         self.engine.encoder_fwd(x, b)
         a, io = GenLatentArgs(), self.engine.latent_io(b)
-        a.batch, a.mode, a.sample = 2 * B, _lib.GEN_RECONSTRUCT, 0
+        a.batch, a.mode, a.sample, a.rows = 2 * B, _lib.GEN_RECONSTRUCT, 0, 2 * B
         a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
         a.gate_ws, a.z, a.z16 = ptr(self._gate_ws), ptr(z), io["z16"]
         _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
@@ -974,15 +962,14 @@ class Learner:
         In data-parallel runs every rank works on its own batch; there is no collective."""
         if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
             raise ValueError("k must be an integer >= 1, got {!r}".format(k))
-        if isinstance(max_rows, bool) or not isinstance(max_rows, (int, np.integer)) or max_rows < 1:
-            raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
+        max_rows = self._check_max_rows(max_rows)
         K = int(k)
         x, B = self._gen_images(x)
         x = x.contiguous()
         if y is not None:
             y = self._gen_labels(y, B, "y")
         n, c = self._gen_noise_c(noise, c, {"eps": (K, B, self.z_dim), "U_y": (K, B, self.y_dim)})
-        kc = max(1, min(K, int(max_rows) // B))
+        kc = max(1, min(K, max_rows // B))
         b, dec = self.engine.bufs(B), self.engine.dec_bufs(B * kc)
         e = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)
         lw_part, log_pxz, state, est, ess = e(B * kc), e(B * kc), e(B, 3), e(B), e(B)

@@ -1,4 +1,4 @@
-"""GPU: the label walk and the characteristic swap - Learner.walk / swap (gccvae_walk_latent + the chunked forward-only
+"""GPU: the label walk and the characteristic swap - Learner.walk / swap (gccvae_gen_latent + the chunked forward-only
 decoder, on the bf16 engine gccvae_convt_image_bf16 into each chunk's slice of the output) - against the fp64
 restatement of tests/walk_oracle.py, their exact known answers against generate / reconstruct / intervene on both
 engines, chunking, sizes and argument checks."""
