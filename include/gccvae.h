@@ -276,9 +276,15 @@ int gccvae_latent_bwd_partials(int batch);
 int gccvae_latent_bwd(const gccvae_latent_bwd_args* a, void* stream);
 
 /* ---- latent code of the forward-only image calls (no counterpart in the reference) -----------------------------
- * One warp per frame writes the z the decoder turns into an image.  Every image has F frames: F = 1 (n_labels = 0), or
- * for a label walk F = n_labels * n_alpha, frame (l, t) of image b being row r = (b * n_labels + l) * n_alpha + t, which
- * walks label labels[l] to the real value alphas[t] in the target prior and keeps the other 17 labels.  Notation: c is
+ * One warp per frame writes the z the decoder turns into an image.  Every image has F frames, of at most one kind:
+ *   one frame (n_labels = n_dims = pair = 0): F = 1;
+ *   label walk: F = n_labels * n_alpha, frame (l, t) of image b being row r = (b * n_labels + l) * n_alpha + t, which
+ *     walks label labels[l] to the real value alphas[t] in the target prior and keeps the other 17 labels;
+ *   latent traversal: F = n_dims * n_alpha, frame (d, t) of image b being row r = (b * n_dims + d) * n_alpha + t: the
+ *     mode's z with z_{dims[d]} set to alphas[t] (an absolute value); every other dim keeps the one-frame call's bits;
+ *   pair interpolation (RECONSTRUCT, sample = 0 only): B pairs, F = n_alpha, frame t of pair b being row r = b * n_alpha
+ *     + t: with z_a, z_b the posterior means of rows b and B + b of loc_pre, z = z_a outside [mix_lo, mix_hi) and inside
+ *     it z_a at t = 0, z_b at t = 1, fmaf(t, z_b - z_a, z_a) otherwise (t = alphas[t], any finite value).  Notation: c is
  * the gate sample of gate_ws (gccvae_gate_fwd); loc_p(y,c), scale_p(y,c) are the conditional prior of
  * networks.py:118-127 (scale after softplus and the [1e-3, 1e3] clip); eps [B,45] is N(0,1) with the layout of
  * gccvae_latent_fwd (columns 0..26 style dims, 27..44 classify dims).  Labels are nonzero -> 1.
@@ -312,8 +318,8 @@ typedef struct {
   int ld_pre;              /* row stride (floats) of loc_pre / scale_pre; 0 = 45 */
   int n_labels;            /* labels walked, 0..18 (0: one frame per image) */
   int labels[18];          /* labels[0 .. n_labels-1]: distinct label indices in [0, 18), in row order */
-  int n_alpha;             /* values per walked label, >= 1 (walk) */
-  const float* alphas;     /* [n_alpha] device fp32, finite (walk) */
+  int n_alpha;             /* values per walked label / traversed dim / pair, >= 1 (walk, traversal, pair) */
+  const float* alphas;     /* [n_alpha] device fp32, finite (walk, traversal, pair) */
   int row0, rows;          /* this chunk: rows row0 .. row0 + rows - 1 of the B * F */
   const float* loc_pre;    /* [B,45] encoder locs head BEFORE relu (RECONSTRUCT, INTERVENE) */
   const float* scale_pre;  /* [B,45] encoder std head BEFORE softplus/clip */
@@ -327,6 +333,12 @@ typedef struct {
   float* z;                /* optional [rows,45] fp32 (operand of the fp32 decoder) */
   void* z16;               /* optional bf16 [rows,64] copy of z, columns 45..63 zero (operand of the tensor-core fc1) */
   int* y_src_out;          /* optional [B,18] int32: the y_src used (INTERVENE) */
+  /* latent traversal (any mode) */
+  int n_dims;              /* latent dims traversed, 0..45 (0: no traversal) */
+  int dims[45];            /* dims[0 .. n_dims-1]: distinct indices in [0, 45), in row order */
+  /* pair interpolation (RECONSTRUCT, sample = 0) */
+  int pair;                /* 1: loc_pre / scale_pre hold 2B rows, image b's partner at row B + b */
+  int mix_lo, mix_hi;      /* the dims [mix_lo, mix_hi) that move; 0 <= mix_lo < mix_hi <= 45 */
 } gccvae_gen_latent_args;
 int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream);
 

@@ -45,6 +45,7 @@ class GenLatentArgs(C.Structure):
         ("loc_pre", C.c_void_p), ("scale_pre", C.c_void_p), ("y_tgt", C.c_void_p), ("y_src", C.c_void_p),
         ("eps", C.c_void_p), ("seed", C.c_uint64), ("offset", C.c_uint64), ("step_dev", C.c_void_p),
         ("gate_ws", C.c_void_p), ("z", C.c_void_p), ("z16", C.c_void_p), ("y_src_out", C.c_void_p),
+        ("n_dims", C.c_int), ("dims", C.c_int * 45), ("pair", C.c_int), ("mix_lo", C.c_int), ("mix_hi", C.c_int),
     ]
 
 

@@ -729,18 +729,28 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int ldp = a.ld_pre > 0 ? a.ld_pre : Z;
   const bool from_image = a.mode != GCCVAE_GEN_GENERATE;
-  const int per_image = a.n_labels > 0 ? a.n_labels * a.n_alpha : 1;
+  const int n_sel = a.n_labels > 0 ? a.n_labels : a.n_dims;    // walked labels or traversed dims (at most one is > 0)
+  const int per_image = n_sel > 0 ? n_sel * a.n_alpha : (a.pair ? a.n_alpha : 1);
   float* zcs = s_zc[wid];
 
   for (int r = blockIdx.x * WARPS + wid; r < a.rows; r += gridDim.x * WARPS) {
     const int gr = a.row0 + r, b = gr / per_image, f = gr - b * per_image;
-    int l = Y;          // one frame per image: no walked label
-    float alpha = 0.0f;
-    if (a.n_labels > 0) {
-      const int li = f / a.n_alpha;
+    int l = Y;          // walked label; Y: none, and then prior_walk_i ignores alpha
+    int dt = Z;         // traversed dim; Z: none
+    float alpha = 0.0f; // the frame's value: of label l, of dim dt, or the pair's t
+    if (n_sel > 0) {
+      const int si = f / a.n_alpha;
+      alpha = a.alphas[f - si * a.n_alpha];
+      // constant-bank reads: a dynamic index would copy the params to the stack
+      if (a.n_labels > 0) {
 #pragma unroll
-      for (int k = 0; k < Y; ++k) l = k == li ? a.labels[k] : l;   // constant-bank reads: a dynamic index would copy the params to the stack
-      alpha = a.alphas[f - li * a.n_alpha];
+        for (int k = 0; k < Y; ++k) l = k == si ? a.labels[k] : l;
+      } else {
+#pragma unroll
+        for (int k = 0; k < Z; ++k) dt = k == si ? a.dims[k] : dt;
+      }
+    } else if (a.pair) {
+      alpha = a.alphas[f];
     }
     // --- posterior (Reconstruct / Intervene) or N(0,1) style dims (Generate) ------------------------------------
     float zv[2] = {0.0f, 0.0f};
@@ -753,6 +763,11 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
         float loc, sc;
         head_act(a.loc_pre[(size_t)b * ldp + d], a.scale_pre[(size_t)b * ldp + d], loc, sc);
         z = a.sample ? fmaf(sc, draw_eps(a.eps, a.seed, offset, b, d), loc) : loc;
+        if (a.pair && d >= a.mix_lo && d < a.mix_hi) {   // z_a -> z_b, both ends exact (as prior_walk_i)
+          float loc_b, sc_b;
+          head_act(a.loc_pre[(size_t)(a.batch + b) * ldp + d], a.scale_pre[(size_t)(a.batch + b) * ldp + d], loc_b, sc_b);
+          z = alpha == 0.0f ? z : (alpha == 1.0f ? loc_b : fmaf(alpha, loc_b - z, z));
+        }
       } else if (d < ZS && a.sample) {
         z = draw_eps(a.eps, a.seed, offset, b, d);
       }
@@ -800,7 +815,7 @@ __global__ void __launch_bounds__(WARPS * 32) gen_latent_kernel(gccvae_gen_laten
     for (int h = 0; h < 2; ++h) {
       const int d = lane + 32 * h;
       if (d < Z) {
-        const float z = d >= ZS ? zcs[d - ZS] : zv[h];
+        const float z = d == dt ? alpha : (d >= ZS ? zcs[d - ZS] : zv[h]);
         if (a.z != nullptr) a.z[(size_t)r * Z + d] = z;
         if (a.z16 != nullptr) reinterpret_cast<__nv_bfloat16*>(a.z16)[(size_t)r * 64 + d] = __float2bfloat16(z);
       } else if (d < 64 && a.z16 != nullptr) {
@@ -1033,10 +1048,22 @@ extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) 
   GCC_REQUIRE(a, "gen_latent: null args");
   GCC_REQUIRE(a->mode >= GCCVAE_GEN_GENERATE && a->mode <= GCCVAE_GEN_INTERVENE,
               "gen_latent: mode %d (1 generate, 2 reconstruct, 3 intervene)", a->mode);
-  GCC_REQUIRE(a->batch > 0 && a->n_labels >= 0 && a->n_labels <= Y && (a->n_labels == 0 || a->n_alpha >= 1),
-              "gen_latent: bad sizes B=%d labels=%d alphas=%d", a->batch, a->n_labels, a->n_alpha);
+  const int kinds = (a->n_labels != 0) + (a->n_dims != 0) + (a->pair != 0);
+  GCC_REQUIRE(kinds <= 1, "gen_latent: a row is at most one of a label walk, a traversal and a pair");
+  GCC_REQUIRE(a->batch > 0 && a->n_labels >= 0 && a->n_labels <= Y && a->n_dims >= 0 && a->n_dims <= Z &&
+                  (a->pair == 0 || a->pair == 1) && (kinds == 0 || a->n_alpha >= 1),
+              "gen_latent: bad sizes B=%d labels=%d dims=%d pair=%d alphas=%d", a->batch, a->n_labels, a->n_dims, a->pair,
+              a->n_alpha);
   GCC_REQUIRE(a->n_labels == 0 || a->mode != GCCVAE_GEN_RECONSTRUCT, "gen_latent: reconstruct walks no label");
-  const long long total = (long long)a->batch * (a->n_labels > 0 ? (long long)a->n_labels * a->n_alpha : 1LL);
+  GCC_REQUIRE(!a->pair || (a->mode == GCCVAE_GEN_RECONSTRUCT && a->sample == 0 && a->mix_lo >= 0 &&
+                           a->mix_lo < a->mix_hi && a->mix_hi <= Z),
+              "gen_latent: a pair needs reconstruct without sampling and 0 <= mix_lo < mix_hi <= 45 (got mode %d, "
+              "sample %d, [%d, %d))", a->mode, a->sample, a->mix_lo, a->mix_hi);
+  const long long per_image = a->n_labels > 0 ? (long long)a->n_labels * a->n_alpha
+                              : a->n_dims > 0 ? (long long)a->n_dims * a->n_alpha
+                              : a->pair       ? (long long)a->n_alpha
+                                              : 1LL;
+  const long long total = (long long)a->batch * per_image;
   GCC_REQUIRE(total < (1LL << 31), "gen_latent: too many rows");
   GCC_REQUIRE(a->row0 >= 0 && a->rows >= 1 && (long long)a->row0 + a->rows <= total,
               "gen_latent: chunk %d + %d outside the %lld rows", a->row0, a->rows, total);
@@ -1046,7 +1073,13 @@ extern "C" int gccvae_gen_latent(const gccvae_gen_latent_args* a, void* stream) 
                 "gen_latent: labels must be distinct indices in [0, 18)");
     seen |= 1u << a->labels[i];
   }
-  GCC_REQUIRE(a->gate_ws && (a->z || a->z16) && (a->n_labels == 0 || a->alphas), "gen_latent: null pointer");
+  unsigned long long seen_d = 0;
+  for (int i = 0; i < a->n_dims; ++i) {
+    GCC_REQUIRE(a->dims[i] >= 0 && a->dims[i] < Z && !((seen_d >> a->dims[i]) & 1ull),
+                "gen_latent: dims must be distinct indices in [0, 45)");
+    seen_d |= 1ull << a->dims[i];
+  }
+  GCC_REQUIRE(a->gate_ws && (a->z || a->z16) && (kinds == 0 || a->alphas), "gen_latent: null pointer");
   GCC_REQUIRE(a->mode == GCCVAE_GEN_GENERATE || (a->loc_pre && a->scale_pre && a->ld_pre >= 0),
               "gen_latent: reconstruct / intervene need loc_pre and scale_pre");
   GCC_REQUIRE(a->mode != GCCVAE_GEN_GENERATE || a->y_tgt, "gen_latent: generate needs y_tgt");

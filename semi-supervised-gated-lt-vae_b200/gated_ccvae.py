@@ -21,6 +21,7 @@ Extensions the reference lacks (for parity testing, data parallelism, image gene
   * a forward-only generation path with no counterpart in the reference: `generate(y)` decodes target labels through
     the conditional prior, `reconstruct(x)` decodes an image's posterior, `intervene(x, y_new)` moves an image's classify
     dims to new labels by a Gaussian counterfactual; each returns a [B,64,64,3] fp32 or uint8 image on the device;
+    `walk`, `swap`, `traverse` and `interpolate` decode frames along one label, between images or along one latent dim;
   * the importance-weighted (IWAE) log-likelihood with K samples: `log_likelihood(x)` bounds log p(x) and
     `log_likelihood(x, y)` bounds log p(x, y) per image (nats, tighter as K grows); `test_log_likelihood(loader)` is its
     `accuracy(loader)` counterpart.
@@ -807,36 +808,51 @@ class Learner:
             raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
         return int(max_rows)
 
-    def _image_call(self, mode, x, y_tgt, y_src, sample, c, noise, dtype, walk=None):
-        """generate / reconstruct / intervene (one frame per image, decoded in `bufs(B)`) and, with walk = (labels,
-        alphas, max_rows), `walk` (frames decoded in chunks through `dec_bufs`): checks, gate, encoder or weight packing,
-        then per chunk gccvae_gen_latent and the decoder into the chunk's rows of the output."""
+    def _image_call(self, mode, x, y_tgt, y_src, sample, c, noise, dtype, frames=None):
+        """generate / reconstruct / intervene (one frame per image, decoded in `bufs(B)`) and, with frames = (kind, items,
+        values, max_rows), the calls with several frames per image (decoded in chunks through `dec_bufs`): "walk" (items:
+        labels), "traverse" (items: latent dims) and "pair" (items: the mixed range (lo, hi); x = (x_a, x_b)).  Checks,
+        gate, encoder or weight packing, then per chunk gccvae_gen_latent and the decoder into the chunk's rows of the
+        output."""
         self._check_dtype(dtype)
-        frames = ()
-        if walk is not None:
-            max_rows = self._check_max_rows(walk[2])
-            labels, alphas = self._walk_labels(walk[0]), self._walk_alphas(walk[1])
-            frames = (len(labels), alphas.numel())
+        kind, shape = None, ()
+        if frames is not None:
+            kind, items, values, max_rows = frames
+            max_rows = self._check_max_rows(max_rows)
+            values = self._walk_alphas(values, "alphas" if kind == "walk" else "values" if kind == "traverse" else "ts")
+            if kind == "walk":
+                items = self._walk_labels(items)
+            elif kind == "traverse":
+                items = self._traverse_dims(items)
+            shape = (values.numel(),) if kind == "pair" else (len(items), values.numel())
         B = None
-        if x is not None:
+        if kind == "pair":
+            xa, B = self._gen_images(x[0])
+            xb, Bb = self._gen_images(x[1])
+            if Bb != B:
+                raise ValueError("the two image sets must hold as many images, got {} and {}".format(B, Bb))
+            if xa.dtype != xb.dtype:     # one of each: both as fp32 in [0,1], the division the kernels do on uint8 images
+                xa, xb = (t.to(torch.float32) / 255.0 if t.dtype == torch.uint8 else t for t in (xa, xb))
+            x = torch.cat([xa, xb])
+        elif x is not None:
             x, B = self._gen_images(x)
-        elif walk is not None and y_tgt is None:
-            raise ValueError("walk needs images x or labels y")
+        elif frames is not None and y_tgt is None:
+            raise ValueError("{} needs images x or labels y".format(kind))
         if y_tgt is not None:
             y_tgt = self._gen_labels(y_tgt, B, "y" if x is None else "y_new")
             B = y_tgt.shape[0]
         if y_src is not None:
             y_src = self._gen_labels(y_src, B, "y")
         n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
-        rows = B * math.prod(frames)
+        rows = B * math.prod(shape)
         if rows >= 1 << 31:
-            raise ValueError("walk of {} frames: at most 2^31 - 1".format(rows))
-        out = torch.empty(B, *frames, 64, 64, 3, dtype=dtype, device=self.device)
-        z = torch.empty(B, *frames, self.z_dim, dtype=torch.float32, device=self.device)
+            raise ValueError("{} of {} frames: at most 2^31 - 1".format(kind, rows))
+        out = torch.empty(B, *shape, 64, 64, 3, dtype=dtype, device=self.device)
+        z = torch.empty(B, *shape, self.z_dim, dtype=torch.float32, device=self.device)
         y_used = torch.empty(B, self.y_dim, dtype=torch.int32, device=self.device) if mode == _lib.GEN_INTERVENE else None
         a = GenLatentArgs()
         a.batch, a.mode, a.sample = B, mode, int(bool(sample))
-        if walk is None:
+        if frames is None:
             dec, chunks = self.engine.bufs(B), [(0, B, z, out)]
         else:
             chunk = min(max_rows, rows)
@@ -844,16 +860,25 @@ class Learner:
             z_rows, out_rows = z.view(rows, self.z_dim), out.view(rows, 64, 64, 3)
             chunks = [(r0, min(chunk, rows - r0), z_rows[r0:r0 + chunk], out_rows[r0:r0 + chunk])
                       for r0 in range(0, rows, chunk)]
-            a.n_labels, a.n_alpha = frames
-            a.labels[:len(labels)] = labels
-            alphas = alphas.to(self.device)
-            a.alphas = ptr(alphas)
-        with self._fresh_noise():
-            self._gate(n, c_in=c)
+            if kind == "walk":
+                a.n_labels = len(items)
+                a.labels[:len(items)] = items
+            elif kind == "traverse":
+                a.n_dims = len(items)
+                a.dims[:len(items)] = items
+            else:
+                a.pair, (a.mix_lo, a.mix_hi) = 1, items
+            a.n_alpha = values.numel()
+            values = values.to(self.device)
+            a.alphas = ptr(values)
+        # a pair reads no gate, prior or noise: it leaves c and the noise stream of the other calls as they were
+        with contextlib.nullcontext() if kind == "pair" else self._fresh_noise():
+            if kind != "pair":
+                self._gate(n, c_in=c)
             if x is None:
                 self.engine.pack_weights()
             else:
-                b = self.engine.bufs(B)
+                b = self.engine.bufs(x.shape[0])
                 self.engine.encoder_fwd(x, b)
                 io = self.engine.latent_io(b)
                 a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
@@ -864,7 +889,12 @@ class Learner:
                 a.row0, a.rows, a.z = r0, nr, ptr(z_chunk)
                 _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
                 self.engine.image_fwd(z_chunk, dec, nr, dtype == torch.uint8, out=out_chunk)
-        self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
+        if kind == "pair":
+            self.last = dict(z=z)
+        elif kind == "traverse":
+            self.last = dict(z=z, c=self._c.clone())
+        else:
+            self.last = dict(z=z, c=self._c.clone(), y_src=y_used)
         return out
 
     def walk(self, x=None, y=None, labels=None, alphas=None, sample=False, c=None, noise=None, dtype=torch.float32,
@@ -885,9 +915,10 @@ class Learner:
         frames, which bounds the memory and changes no value.
         `self.last` = {"z": [B,L,T,45] fp32, "c": [18,18], "y_src": [B,18] int32 labels walked from (images) or None}.
         In data-parallel runs every rank works on its own batch; there is no collective."""
+        frames = ("walk", labels, alphas, max_rows)
         if x is None:
-            return self._image_call(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype, (labels, alphas, max_rows))
-        return self._image_call(_lib.GEN_INTERVENE, x, None, y, sample, c, noise, dtype, (labels, alphas, max_rows))
+            return self._image_call(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype, frames)
+        return self._image_call(_lib.GEN_INTERVENE, x, None, y, sample, c, noise, dtype, frames)
 
     def _walk_labels(self, labels):
         if labels is None:
@@ -901,47 +932,81 @@ class Learner:
         return out
 
     @staticmethod
-    def _walk_alphas(alphas):
+    def _walk_alphas(alphas, name="alphas"):
+        """alphas of `walk`, values of `traverse`, ts of `interpolate`; None: 8 points from 0 to 1, both ends exact."""
         if alphas is None:
             return torch.arange(8, dtype=torch.float64).div(7).float()     # 0/7 .. 7/7: both ends exact
         try:
             v = torch.as_tensor(alphas.detach().cpu() if torch.is_tensor(alphas) else alphas, dtype=torch.float32)
         except (TypeError, ValueError, RuntimeError) as e:
-            raise ValueError("alphas must be a 1-D sequence of floats, got {!r}".format(alphas)) from e
+            raise ValueError("{} must be a 1-D sequence of floats, got {!r}".format(name, alphas)) from e
         if v.dim() != 1 or v.numel() == 0 or not bool(torch.isfinite(v).all()):
-            raise ValueError("alphas must be a non-empty 1-D sequence of finite floats, got {!r}".format(alphas))
+            raise ValueError("{} must be a non-empty 1-D sequence of finite floats, got {!r}".format(name, alphas))
         return v.contiguous()
+
+    def traverse(self, x=None, y=None, dims=None, values=None, sample=False, c=None, noise=None, dtype=torch.float32,
+                 max_rows=8192):
+        """Frames along single latent dims: for every image, every dim d of `dims` and every value v of `values`, the
+        image decoded from the base code with z_d set to v; every other dim keeps the base code's bits.  This shows what
+        one latent encodes, also a style dim (0..26) that no label reaches or a classify dim (27..44) that a learned gate
+        wires to several labels or to none.
+          From images (x [B,64,64,3] given): the base code is `reconstruct(x, sample)`'s z.
+          From labels (x=None, y [B,18] required): the base code is `generate(y, sample)`'s z.
+        dims: distinct latent indices in [0, 45), in output order (default: all 45); values: a non-empty 1-D sequence of
+        finite floats, taken as fp32, the absolute value given to z_d (default: the integers -3 .. 3).  The frame whose
+        value is the base's own z_d is the base image, bit for bit.  The noise of an image is drawn once and shared by
+        all its frames; c, `noise={"eps": [B,45], "U1", "U2"}` and `dtype` are as in `generate`.
+        Returns a fresh [B, D, T, 64, 64, 3] device tensor (D dims, T values), decoded in chunks of at most `max_rows`
+        frames, which bounds the memory and changes no value.  `self.last` = {"z": [B,D,T,45] fp32, "c": [18,18]}.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        if values is None:
+            values = torch.arange(-3, 4, dtype=torch.float32)
+        frames = ("traverse", dims, values, max_rows)
+        if x is None:
+            if y is None:
+                raise ValueError("traverse needs images x or labels y")
+            return self._image_call(_lib.GEN_GENERATE, None, y, None, sample, c, noise, dtype, frames)
+        if y is not None:
+            raise ValueError("traverse takes images x or labels y, not both")
+        return self._image_call(_lib.GEN_RECONSTRUCT, x, None, None, sample, c, noise, dtype, frames)
+
+    def _traverse_dims(self, dims):
+        if dims is None:
+            return list(range(self.z_dim))
+        v = np.asarray(dims.cpu() if torch.is_tensor(dims) else dims)
+        if v.ndim != 1 or v.size == 0 or v.dtype.kind not in "iu":
+            raise ValueError("dims must be a non-empty 1-D sequence of integers, got {!r}".format(dims))
+        out = [int(t) for t in v]
+        if min(out) < 0 or max(out) >= self.z_dim or len(set(out)) != len(out):
+            raise ValueError("dims must be distinct indices in [0, {}), got {}".format(self.z_dim, out))
+        return out
+
+    def interpolate(self, x_a, x_b, ts=None, part="all", dtype=torch.float32, max_rows=8192):
+        """Frames on the straight line between the posterior means z_a of x_a and z_b of x_b: for every pair and every t
+        of `ts`, the image decoded from z with z = z_a outside the mixed dims and, inside them, z_a + t (z_b - z_a) -
+        exactly z_a at t = 0 and exactly z_b at t = 1; values beyond [0, 1] extrapolate.  part: the mixed dims, "all"
+        (0..44), "style" (0..26) or "classify" (27..44).  So part "classify" at t = 1 is `swap(x_a, x_b)` and part "all"
+        at t = 1 is `reconstruct(x_b)`, bit for bit.  No gate, prior or noise is involved.
+        x_a, x_b: [B,64,64,3] each (fp32 in [0,1] or uint8), one encoder pass over the 2B images; ts: a non-empty 1-D
+        sequence of finite floats, taken as fp32 (default: 8 points from 0 to 1, both ends exact).  Returns a fresh
+        [B, T, 64, 64, 3] device tensor, decoded in chunks of at most `max_rows` frames (this changes no value), as
+        `generate` does for `dtype`.  `self.last` = {"z": [B,T,45] fp32}.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        ranges = {"all": (0, self.z_dim), "style": (0, self.z_style), "classify": (self.z_style, self.z_dim)}
+        if not isinstance(part, str) or part not in ranges:
+            raise ValueError("part must be one of 'all', 'style', 'classify', got {!r}".format(part))
+        return self._image_call(_lib.GEN_RECONSTRUCT, (x_a, x_b), None, None, False, None, None, dtype,
+                                ("pair", ranges[part], ts, max_rows))
 
     def swap(self, x_style, x_char, dtype=torch.float32):
         """Characteristic swap: images decoded from z = [z_s of x_style, z_c of x_char], both posterior means (the style
         of one image with the label-linked latents of another).  x_style and x_char are [B,64,64,3] each (fp32 in [0,1]
         or uint8) and go through one encoder pass over 2B images; no gate and no prior are involved, so swap(x, x) is
-        reconstruct(x).  Returns a fresh [B,64,64,3] image as `generate` does; `self.last` = {"z": [B,45]}."""
-        self._check_dtype(dtype)
-        xs, B = self._gen_images(x_style)
-        xc, Bc = self._gen_images(x_char)
-        if Bc != B:
-            raise ValueError("x_style and x_char must hold as many images, got {} and {}".format(B, Bc))
-        if xs.dtype != xc.dtype:     # one of each: both as fp32 in [0,1], the division the kernels do on uint8 images
-            xs, xc = (t.to(torch.float32) / 255.0 if t.dtype == torch.uint8 else t for t in (xs, xc))
-        x = torch.cat([xs, xc])
-        b = self.engine.bufs(2 * B)
-        z = torch.empty(2 * B, self.z_dim, dtype=torch.float32, device=self.device)
-        out = torch.empty(B, 64, 64, 3, dtype=dtype, device=self.device)
-        self.engine.encoder_fwd(x, b)
-        a, io = GenLatentArgs(), self.engine.latent_io(b)
-        a.batch, a.mode, a.sample, a.rows = 2 * B, _lib.GEN_RECONSTRUCT, 0, 2 * B
-        a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
-        a.gate_ws, a.z, a.z16 = ptr(self._gate_ws), ptr(z), io["z16"]
-        _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
-        # rows 0..B-1 become the swapped codes; z16 = bf16(z) elementwise, so composing its columns is exact
-        zs = self.z_style
-        z[:B, zs:].copy_(z[B:, zs:])
-        if b.get("z16") is not None:
-            b["z16"][:B, zs:self.z_dim].copy_(b["z16"][B:, zs:self.z_dim])
-        self.engine.image_fwd(z[:B], b, B, dtype == torch.uint8, out=out)
-        self.last = dict(z=z[:B])
-        return out
+        reconstruct(x).  It is `interpolate(x_style, x_char, ts=[1.0], part="classify")`.  Returns a fresh [B,64,64,3]
+        image as `generate` does; `self.last` = {"z": [B,45]}."""
+        out = self.interpolate(x_style, x_char, ts=[1.0], part="classify", dtype=dtype)
+        self.last = dict(z=self.last["z"][:, 0])
+        return out[:, 0]
 
     # ---- importance-weighted log-likelihood (an extension: the reference scores a model by accuracy only) ------------
     def log_likelihood(self, x, y=None, k=100, c=None, noise=None, max_rows=8192, keep_log_w=False):
