@@ -176,6 +176,19 @@ int gccvae_fill_f32(float* p, long long n, float v, void* stream);
  *   The uint8 output is the fp32 output of the same call converted by that rule, bit for bit. */
 int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp8, const float* bias, void* out, int out_u8,
                             void* stream);
+/* One iteration of image completion (no counterpart in the reference: gated_ccvae.py's Learner.complete): conv5t forward
+ * + sigmoid as gccvae_convt_image_bf16 computes it, written straight into the encoder's input blocks for the next
+ * iteration instead of into an image.
+ *   g4, Wp8, bias: as gccvae_convt_image_bf16.
+ *   mask_blocks: [B,33,33] uint8, the pixel mask in x2 block form: bit dy * 2 + dx of block (i, j) is set when pixel
+ *     (2i-1+dy, 2j-1+dx) is observed.  Bits of pixels outside the image are ignored.
+ *   X2: [B,33,33,16] bf16 x2 blocks as gccvae_prep_x2_bf16 writes them (16-byte aligned), updated IN PLACE: every
+ *     unobserved pixel gets bf16(xhat) in its three channel lanes (the bits gccvae_prep_x2_bf16 makes of the fp32 image
+ *     that gccvae_convt_image_bf16 writes), and its pad lane is written with the value it already holds (0, or 1.0 in
+ *     element 15).  Observed pixels are not written, and a block with no unobserved pixel is not stored at all, so
+ *     nothing beyond the B x 1089 blocks - such as the raw-byte blocks XB that may follow them - is touched. */
+int gccvae_convt_complete_bf16(int batch, const void* g4, const void* Wp8, const float* bias, const void* mask_blocks,
+                               void* X2, void* stream);
 /* Likelihood of K decoded rows per source image (no counterpart in the reference: the importance-weighted estimate of
  * gated_ccvae.py's Learner.log_likelihood): conv5t forward + sigmoid + the Laplace log-likelihood of utils.py:101-105,
  * with no gradient, no reconstruction and no bias gradient.

@@ -167,6 +167,7 @@ SIGNATURES = {
     "gccvae_tap4_wg_bf16": (_I, [_I, _P, _P, _I, _P, _P, _P]),
     "gccvae_convt_recon_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _I, _P]),
     "gccvae_convt_image_bf16": (_I, [_I, _P, _P, _P, _P, _I, _P]),
+    "gccvae_convt_complete_bf16": (_I, [_I, _P, _P, _P, _P, _P, _P]),
     "gccvae_convt_ll_bf16": (_I, [_I, _I, _P, _P, _P, _P, _I, _P, _P]),
     "gccvae_fill_f32": (_I, [_P, _LL, _F, _P]),
     "gccvae_gate_fwd": (_I, [_P, _P, _P, _P, _U64, _U64, _P, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -1208,6 +1208,8 @@ __global__ void __launch_bounds__(256) prep_x2_u8_staged_kernel(const uint8_t* _
 //   LL         Laplace log-likelihood of decoded row n against source image n / kc - the importance-weighted likelihood
 //   IMAGE_F32  the sigmoid into the [B,64,64,3] fp32 image - the generation path
 //   IMAGE_U8   the same as uint8 min(255, rint(255 x))
+//   COMPLETE   the sigmoid, bf16-rounded, into the unobserved pixel slots of the encoder's input blocks X2 in place - the
+//              composite of one iteration of image completion (gccvae_convt_complete_bf16)
 // Output block (i, j) of an image = sum over the 2x2 taps (a, b) of g4[i - a, j - b, :] . W_ab  (K = 32 per tap, N = 16).
 // Tile = 128 CONSECUTIVE blocks f = 33 i + j of one image (9 tiles per image, the last one holds 65).  The operand of
 // all four taps is ONE TMA box of the decoder activation g4 [B,32,32,32]: 6 image rows x 33 columns starting at column
@@ -1216,7 +1218,7 @@ __global__ void __launch_bounds__(256) prep_x2_u8_staged_kernel(const uint8_t* _
 // 33): a start-address offset of the A descriptor.  The swizzle XOR is taken from the absolute shared-memory address, so
 // a K-major operand may start at ANY row of a swizzled buffer (scripts/microbench/desc_offset.cu,
 // profiles/r02_microbench_desc_offset.txt) - 198 box rows per tile instead of the 4 x 121 of one box per tap.
-enum ConvtOut { RECON, LL, IMAGE_F32, IMAGE_U8 };
+enum ConvtOut { RECON, LL, IMAGE_F32, IMAGE_U8, COMPLETE };
 
 struct alignas(64) CtParams {
   CUtensorMap tmA, tmB;
@@ -1230,8 +1232,9 @@ struct alignas(64) CtParams {
   float* db;           // RECON: optional [3] += sum of dlogit (bias gradient of conv5t)
   int batch, total_tiles, stages;
   long long* timeline;
-  void* out;           // IMAGE_*: [B,64,64,3] fp32 or uint8
+  void* out;           // IMAGE_*: [B,64,64,3] fp32 or uint8; COMPLETE: the x2 blocks [B,33,33,16] bf16, rewritten in place
   int kc;              // LL: decoded rows per source image
+  const uint8_t* mask; // COMPLETE: [B,33,33], bit dy * 2 + dx of block (i, j) set = pixel (2i-1+dy, 2j-1+dx) observed
 };
 
 constexpr int CTR_BOX_ROWS = 6 * 33;          // rows of the A box (64 bytes each)
@@ -1249,7 +1252,7 @@ __device__ __forceinline__ float rcp_approx(float v) {
 }
 
 // XM = form of the image operand of RECON / LL: 0 fp32 NHWC, 1 uint8 NHWC, 2 uint8 raw-byte blocks XB [B,33,33,16]
-// (prep_x2).  The IMAGE kinds read no image and are instantiated with XM = 0.
+// (prep_x2).  The IMAGE kinds and COMPLETE read no image and are instantiated with XM = 0.
 // XM = 2: the 2 KB of raw bytes of a tile's 128 blocks travel with the tile's operand box (one bulk copy into the same
 // pipeline stage, same barrier); the stage is free again when the MMAs have read the box AND the four epilogue warps have
 // taken their bytes.  A register prefetch one tile ahead (XM = 0 / 1) is too short: a tile's epilogue is ~0.3 us of work,
@@ -1258,7 +1261,7 @@ constexpr int CTR_X_BYTES = 128 * 16;
 template <int OUT, int XM>
 __global__ void __launch_bounds__(TG_THREADS, 4) convt_kernel(const __grid_constant__ CtParams p) {
   constexpr bool HAS_X = OUT == RECON || OUT == LL;   // reads an image operand
-  static_assert(HAS_X || XM == 0, "the IMAGE kinds are instantiated with XM = 0");
+  static_assert(HAS_X || XM == 0, "the IMAGE kinds and COMPLETE are instantiated with XM = 0");
   constexpr bool RAW_X = HAS_X && XM == 2;            // the raw image bytes travel with the pipeline stage
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -1413,6 +1416,9 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_kernel(const __grid_const
       const int f = k * 128 + m, i = f / 33, j = f - i * 33;
       const bool row_ok = f < 33 * 33;
       const int n_cur = n;
+      uint32_t mbits = 0xfu;   // COMPLETE: the block's mask byte, loaded here so that its latency hides behind the wait below
+      if constexpr (OUT == COMPLETE)
+        if (row_ok) mbits = __ldg(p.mask + (size_t)n_cur * 1089 + f);
       // (consumed at the very end of the tile: an L2 access that needs no prefetch)
       const float cb = OUT == RECON && p.coef != nullptr ? __ldg(p.coef + n_cur) : 0.0f;
       float xv[12];
@@ -1495,6 +1501,15 @@ __global__ void __launch_bounds__(TG_THREADS, 4) convt_kernel(const __grid_const
       } else if constexpr (OUT == LL) {
 #pragma unroll
         for (int k2 = 0; k2 < 12; ++k2) l1 = fmaf(okf[k2 / 3], fabsf(xv[k2] - xh[k2]), l1);
+      } else if constexpr (OUT == COMPLETE) {
+        // an unobserved pixel's 8 bytes are rewritten as prep_x2 writes them: its three channels, then the pad lane (0, or
+        // the block's constant 1.0 in element 15); observed and out-of-image pixels keep their bytes, and a block without
+        // an unobserved pixel is not stored at all
+        uint2* dst = static_cast<uint2*>(p.out) + ((size_t)n_cur * 1089 + f) * 4;
+#pragma unroll
+        for (int qq = 0; qq < 4; ++qq)
+          if (ok[qq] && !((mbits >> qq) & 1u))
+            dst[qq] = make_uint2(pack_bf16x2(xh[3 * qq], xh[3 * qq + 1]), pack_bf16x2(xh[3 * qq + 2], qq == 3 ? 1.0f : 0.0f));
       } else {
 #pragma unroll
         for (int qq = 0; qq < 4; ++qq)
@@ -2442,7 +2457,7 @@ static_assert(CT_PER_SM * (convt_smem(true) + 1024) <= 227 * 1024, "conv5t: CT_P
 // The common launch of conv5t over `rows` decoded rows of g4 [rows,32,32,32] bf16 (Wp8 = pack kind 8): the tensor maps,
 // the launch shape, and the (out, x_form) instantiation; the caller fills the rest of p.
 static int launch_convt(int out, int rows, const void* g4, const void* Wp8, CtParams& p, int x_form, cudaStream_t st) {
-  static const char* const name[4] = {"convt_recon", "convt_ll", "convt_image", "convt_image"};
+  static const char* const name[5] = {"convt_recon", "convt_ll", "convt_image", "convt_image", "convt_complete"};
   EncodeTiledFn enc = get_encode();
   GCC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable");
   {
@@ -2462,11 +2477,12 @@ static int launch_convt(int out, int rows, const void* g4, const void* Wp8, CtPa
   p.stages = CT_STAGES;
   const size_t smem = convt_smem((out == RECON || out == LL) && x_form == 2);
   using Kernel = void (*)(const CtParams);
-  static const Kernel kernels[4][3] = {{convt_kernel<RECON, 0>, convt_kernel<RECON, 1>, convt_kernel<RECON, 2>},
+  static const Kernel kernels[5][3] = {{convt_kernel<RECON, 0>, convt_kernel<RECON, 1>, convt_kernel<RECON, 2>},
                                        {convt_kernel<LL, 0>, convt_kernel<LL, 1>, convt_kernel<LL, 2>},
                                        {convt_kernel<IMAGE_F32, 0>, nullptr, nullptr},
-                                       {convt_kernel<IMAGE_U8, 0>, nullptr, nullptr}};
-  static bool attr_set[4][3] = {};
+                                       {convt_kernel<IMAGE_U8, 0>, nullptr, nullptr},
+                                       {convt_kernel<COMPLETE, 0>, nullptr, nullptr}};
+  static bool attr_set[5][3] = {};
   const Kernel kernel = kernels[out][x_form];
   if (!attr_set[out][x_form]) {
     GCC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -2517,6 +2533,19 @@ extern "C" int gccvae_convt_image_bf16(int batch, const void* g4, const void* Wp
   memset(&p, 0, sizeof(p));
   p.bias = bias; p.out = out; p.batch = batch;
   return launch_convt(out_u8 ? IMAGE_U8 : IMAGE_F32, batch, g4, Wp8, p, 0, (cudaStream_t)stream);
+}
+
+// conv5t forward + sigmoid written into the unobserved pixels of the x2 blocks X2 [B,33,33,16] bf16, in place (one
+// iteration of image completion): mask_blocks [B,33,33] uint8, bit dy * 2 + dx set = pixel (2i-1+dy, 2j-1+dx) observed.
+extern "C" int gccvae_convt_complete_bf16(int batch, const void* g4, const void* Wp8, const float* bias,
+                                          const void* mask_blocks, void* X2, void* stream) {
+  GCC_REQUIRE(g4 && Wp8 && bias && mask_blocks && X2, "convt_complete: null pointer");
+  GCC_REQUIRE(batch > 0 && batch <= (1 << 26), "convt_complete: bad batch %d", batch);
+  GCC_REQUIRE((uintptr_t)X2 % 16 == 0 && (uintptr_t)g4 % 16 == 0, "convt_complete: X2 and g4 must be 16-byte aligned");
+  CtParams p;
+  memset(&p, 0, sizeof(p));
+  p.bias = bias; p.out = X2; p.mask = (const uint8_t*)mask_blocks; p.batch = batch;
+  return launch_convt(COMPLETE, batch, g4, Wp8, p, 0, (cudaStream_t)stream);
 }
 
 // conv5t forward + sigmoid + Laplace log-likelihood of `rows` decoded rows, row r against source image r / kc

@@ -193,6 +193,17 @@ class Engine:
             out.copy_(image_u8(h[:batch]))
         return out
 
+    def complete_begin(self, x, mask):
+        """per-call state of image completion: the pixel mask [B,64,64] bool (True = observed) and the composite image
+        the encoder reads from the second iteration on."""
+        return {"mask": mask.unsqueeze(-1), "img": torch.empty_like(x)}
+
+    def complete_fwd(self, z, b, batch, state, x):
+        """one iteration of image completion (the parity path): decode z, then the composite where(mask, x, xhat) of the
+        fp32 image x into the image the next encoder pass reads, which is returned."""
+        xhat = self.decoder_fwd(z[:batch], b)
+        return torch.where(state["mask"], x, xhat, out=state["img"])
+
     def iw_decoder_ll(self, x, b, batch, kc, dec, log_pxz):
         """importance-weighted likelihood: log_pxz[r] = log p(x_(r / kc) | z_r) for the batch * kc rows of dec["z"]
         (the parity path: the generic decoder, then the reconstruction likelihood against the repeated images)."""

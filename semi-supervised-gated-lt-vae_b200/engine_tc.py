@@ -391,7 +391,9 @@ class EngineTC(Engine):
         B, u8 = x.shape[0], int(x.dtype == torch.uint8)
         return self.lib.gccvae_prep_x2_bf16(ptr(x), u8, B, ptr(x2), self.xb_ptr(x2, B) if u8 else None, stream)
 
-    def encoder_fwd(self, x, b, heads=True):
+    def encoder_fwd(self, x, b, heads=True, blocks_ready=False):
+        """`blocks_ready`: b["X2"] already holds the image blocks (image completion writes them in place), x only gives
+        the batch size: no prep_x2."""
         B = x.shape[0]
         lib, st, v = self.lib, _stream(), self.store.view
         begun, self._begun = getattr(self, "_begun", False), False
@@ -402,8 +404,7 @@ class EngineTC(Engine):
         else:
             self._log_pxz_ready = False
             self.pack_weights()
-            u8 = int(x.dtype == torch.uint8)
-            if not self.x2_ready:
+            if not (self.x2_ready or blocks_ready):
                 self._run("prep_x2", (x, b["X2"]), lambda: self.prep_x2(x, b["X2"], st))
         self._run("enc.conv1 fwd", (b["X2"][:B * 1089 * 16], b["enc.conv1.out"]), lambda: lib.gccvae_c3conv_bf16(
             B, ptr(b["X2"]), ptr(self.wp["enc.conv1.x2"]), 32, ptr(v("enc.conv1.b")), ACT_RELU | OUT_S2D, None,
@@ -489,6 +490,27 @@ class EngineTC(Engine):
             batch, ptr(g4), ptr(self.wp["dec.conv5t.x2t"]), ptr(self.store.view("dec.conv5t.b")), ptr(out), int(out_u8),
             _stream()))
         return out
+
+    def complete_begin(self, x, mask):
+        """per-call state of image completion: the pixel mask [B,64,64] bool (True = observed) in x2 block form,
+        [B,33,33] uint8 with bit dy * 2 + dx of block (i, j) set when pixel (2i-1+dy, 2j-1+dx) is observed; pixels outside
+        the image count as observed."""
+        B = mask.shape[0]
+        m = torch.nn.functional.pad(mask.to(torch.uint8), (1, 1, 1, 1), value=1)        # [B,66,66]
+        m = m.view(B, 33, 2, 33, 2).permute(0, 1, 3, 2, 4)                               # [B,33,33,dy,dx]
+        bit = torch.tensor([[1, 2], [4, 8]], dtype=torch.uint8, device=self.device)
+        return {"mask_blocks": (m * bit).sum((-2, -1), dtype=torch.uint8).contiguous()}
+
+    def complete_fwd(self, z, b, batch, state, x):
+        """one iteration of image completion: the decoder from the z16 operand the latent kernel wrote, then conv5t +
+        sigmoid straight into the unobserved pixels of the encoder's input blocks b["X2"], in place
+        (gccvae_convt_complete_bf16).  Returns x: the next encoder pass reads the blocks as they are (blocks_ready)."""
+        self.decoder_fwd(None, b, z16_ready=True, fused_recon=True, batch=batch, head=True)
+        g4, mb = b["dec.conv4t.out"], state["mask_blocks"]
+        self._run("dec.conv5t fwd complete", (g4, mb), lambda: self.lib.gccvae_convt_complete_bf16(
+            batch, ptr(g4), ptr(self.wp["dec.conv5t.x2t"]), ptr(self.store.view("dec.conv5t.b")), ptr(mb), ptr(b["X2"]),
+            _stream()))
+        return x
 
     def iw_decoder_ll(self, x, b, batch, kc, dec, log_pxz):
         """importance-weighted likelihood: the decoder over the batch * kc rows of dec["z16"], then conv5t + sigmoid +

@@ -22,6 +22,7 @@ Extensions the reference lacks (for parity testing, data parallelism, image gene
     the conditional prior, `reconstruct(x)` decodes an image's posterior, `intervene(x, y_new)` moves an image's classify
     dims to new labels by a Gaussian counterfactual; each returns a [B,64,64,3] fp32 or uint8 image on the device;
     `walk`, `swap`, `traverse` and `interpolate` decode frames along one label, between images or along one latent dim;
+    `complete(x, mask, y_new)` fills in the unobserved pixels of images, optionally steered to target labels;
   * the importance-weighted (IWAE) log-likelihood with K samples: `log_likelihood(x)` bounds log p(x) and
     `log_likelihood(x, y)` bounds log p(x, y) per image (nats, tighter as K grows); `test_log_likelihood(loader)` is its
     `accuracy(loader)` counterpart.
@@ -40,7 +41,7 @@ import torch
 from . import _lib, dp
 from ._lib import (GATE_WS_FLOATS, LATENT_PARTIAL_FLOATS, RESULT_SLOT_FLOATS, ChainBwdArgs, ChainFwdArgs, DpArgs,
                    GenLatentArgs, IwLatentArgs, LatentBwdArgs, LatentFwdArgs, ptr)
-from .engine import Engine, _stream
+from .engine import Engine, _stream, image_u8
 from .networks import Classifier, Conditional_Prior, Decoder, Encoder, _default_device, as_device_f32
 from .params import ParamStore, keras_default_init
 from .utils_data import gating_matrix_csv, load_learned_gating_matrix
@@ -808,12 +809,13 @@ class Learner:
             raise ValueError("max_rows must be an integer >= 1, got {!r}".format(max_rows))
         return int(max_rows)
 
-    def _image_call(self, mode, x, y_tgt, y_src, sample, c, noise, dtype, frames=None):
+    def _image_call(self, mode, x, y_tgt, y_src, sample, c, noise, dtype, frames=None, complete=None):
         """generate / reconstruct / intervene (one frame per image, decoded in `bufs(B)`) and, with frames = (kind, items,
         values, max_rows), the calls with several frames per image (decoded in chunks through `dec_bufs`): "walk" (items:
         labels), "traverse" (items: latent dims) and "pair" (items: the mixed range (lo, hi); x = (x_a, x_b)).  Checks,
         gate, encoder or weight packing, then per chunk gccvae_gen_latent and the decoder into the chunk's rows of the
-        output."""
+        output.  complete = (mask, iters): that body `iters` times, each time on the composite of x's observed pixels and
+        the previous decode (`complete`), with the gate of the first."""
         self._check_dtype(dtype)
         kind, shape = None, ()
         if frames is not None:
@@ -843,7 +845,10 @@ class Learner:
             B = y_tgt.shape[0]
         if y_src is not None:
             y_src = self._gen_labels(y_src, B, "y")
-        n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim)})
+        iters = 1
+        if complete is not None:
+            mask, iters = self._complete_mask(complete[0], B), complete[1]
+        n, c = self._gen_noise_c(noise, c, {"eps": (B, self.z_dim) if complete is None else (iters, B, self.z_dim)})
         rows = B * math.prod(shape)
         if rows >= 1 << 31:
             raise ValueError("{} of {} frames: at most 2^31 - 1".format(kind, rows))
@@ -871,24 +876,41 @@ class Learner:
             a.n_alpha = values.numel()
             values = values.to(self.device)
             a.alphas = ptr(values)
-        # a pair reads no gate, prior or noise: it leaves c and the noise stream of the other calls as they were
-        with contextlib.nullcontext() if kind == "pair" else self._fresh_noise():
-            if kind != "pair":
-                self._gate(n, c_in=c)
-            if x is None:
-                self.engine.pack_weights()
-            else:
-                b = self.engine.bufs(x.shape[0])
-                self.engine.encoder_fwd(x, b)
-                io = self.engine.latent_io(b)
-                a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
-            a.y_tgt, a.y_src, a.eps = ptr(y_tgt), ptr(y_src), ptr(n["eps"])
-            a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
-            a.gate_ws, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(dec.get("z16")), ptr(y_used)
-            for r0, nr, z_chunk, out_chunk in chunks:
-                a.row0, a.rows, a.z = r0, nr, ptr(z_chunk)
-                _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
-                self.engine.image_fwd(z_chunk, dec, nr, dtype == torch.uint8, out=out_chunk)
+        # (one iteration decodes straight into the output: no composite, no mask blocks)
+        state = self.engine.complete_begin(x, mask) if iters > 1 else None
+        x_in = x
+        for t in range(iters):
+            # a pair reads no gate, prior or noise: it leaves c and the noise stream of the other calls as they were
+            with contextlib.nullcontext() if kind == "pair" else self._fresh_noise():
+                if kind != "pair" and t == 0:
+                    self._gate(n, c_in=c)
+                if x is None:
+                    self.engine.pack_weights()
+                else:
+                    b = self.engine.bufs(x.shape[0])
+                    if t > 0 and getattr(self.engine, "x2", False):   # the composite is already in b["X2"]
+                        self.engine.encoder_fwd(x_in, b, blocks_ready=True)
+                    else:
+                        self.engine.encoder_fwd(x_in, b)
+                    io = self.engine.latent_io(b)
+                    a.loc_pre, a.scale_pre, a.ld_pre = io["loc_pre"], io["scale_pre"], io["ld_pre"]
+                eps = n["eps"] if complete is None or n["eps"] is None else n["eps"][t]
+                a.y_tgt, a.y_src, a.eps = ptr(y_tgt), ptr(y_src), ptr(eps)
+                a.seed, a.offset, a.step_dev = dp.data_seed(self.seed, self.rank), self._noise_offset, ptr(self.optimiser.step_dev)
+                a.gate_ws, a.z16, a.y_src_out = ptr(self._gate_ws), ptr(dec.get("z16")), ptr(y_used)
+                for r0, nr, z_chunk, out_chunk in chunks:
+                    a.row0, a.rows, a.z = r0, nr, ptr(z_chunk)
+                    _lib.check(self.lib.gccvae_gen_latent(C.byref(a), _stream()), "gen_latent")
+                    if t + 1 < iters:
+                        x_in = self.engine.complete_fwd(z_chunk, dec, nr, state, x)
+                    else:
+                        self.engine.image_fwd(z_chunk, dec, nr, dtype == torch.uint8, out=out_chunk)
+        if complete is not None:    # the observed pixels are x's, converted to dtype as the image calls convert
+            if dtype == torch.uint8 and x.dtype != torch.uint8:
+                x = image_u8(x)
+            elif dtype == torch.float32 and x.dtype == torch.uint8:
+                x = torch.div(x, 255.0)     # fp32 u / 255, as x.to(torch.float32) / 255.0 in one pass
+            out = torch.where(mask.unsqueeze(-1), x, out)
         if kind == "pair":
             self.last = dict(z=z)
         elif kind == "traverse":
@@ -1007,6 +1029,41 @@ class Learner:
         out = self.interpolate(x_style, x_char, ts=[1.0], part="classify", dtype=dtype)
         self.last = dict(z=self.last["z"][:, 0])
         return out[:, 0]
+
+    def complete(self, x, mask, y_new=None, y=None, iters=10, sample=False, c=None, noise=None, dtype=torch.float32):
+        """Completion of partially observed images x [B,64,64,3] (fp32 in [0,1] or uint8): mask [B,64,64] or [64,64]
+        (broadcast over the batch), bool or integer, nonzero = the pixel (all three channels) is observed.  The pixels
+        that are not observed start from whatever x holds there (the caller's initial fill, e.g. grey or noise).  Each of
+        the `iters` iterations (pseudo-Gibbs / iterative reconstruction) encodes the current composite, takes z as
+        `reconstruct` does (`sample=False`: the posterior mean, `sample=True`: loc + scale eps) and - with target labels
+        y_new [B,18] - moves the classify dims from y (default: the classifier's decision on that iteration's z_c) to
+        y_new as `intervene` does; the decoder's mean (the sigmoid every image call returns) then replaces the unobserved
+        pixels of the composite.  Observed pixels never change.  So one iteration is `reconstruct` / `intervene` of the
+        composite, bit for bit, followed by torch.where(mask, x, image) in fp32.
+        c [18,18]: one gate sample per call unless given, shared by every iteration; iteration t draws its noise as the
+        t-th of `iters` consecutive calls would; `noise={"eps": [iters,B,45], "U1": [18,18], "U2": [18,18]}` makes the
+        draws explicit.  Returns a fresh [B,64,64,3] device tensor of `dtype`: the observed pixels are x (uint8 -> fp32
+        as u / 255, fp32 -> uint8 as min(255, rint(255 x))), the others the last iteration's decode, as `generate`
+        returns it.  `self.last` = {"z": [B,45] of the last iteration, "c": [18,18], "y_src": [B,18] int32 labels the last
+        iteration moved from (with y_new) or None}.
+        On the bf16 engine the decode of every iteration but the last goes straight into the unobserved pixels of the
+        encoder's input blocks (gccvae_convt_complete_bf16): no image, mask pass or block transform in between.
+        In data-parallel runs every rank works on its own batch; there is no collective."""
+        if y is not None and y_new is None:
+            raise ValueError("complete: source labels y need target labels y_new")
+        if isinstance(iters, bool) or not isinstance(iters, (int, np.integer)) or iters < 1:
+            raise ValueError("iters must be an integer >= 1, got {!r}".format(iters))
+        mode = _lib.GEN_RECONSTRUCT if y_new is None else _lib.GEN_INTERVENE
+        return self._image_call(mode, x, y_new, y, sample, c, noise, dtype, complete=(mask, int(iters)))
+
+    def _complete_mask(self, mask, B):
+        """mask of `complete` -> [B,64,64] bool device tensor (True = observed)."""
+        m = torch.as_tensor(mask) if not torch.is_tensor(mask) else mask
+        if (m.dtype.is_floating_point or m.dtype.is_complex or m.dim() not in (2, 3) or tuple(m.shape[-2:]) != (64, 64)
+                or (m.dim() == 3 and m.shape[0] != B)):
+            raise ValueError("mask must be [B,64,64] or [64,64] bool or integer with B={}, got {} {}".format(
+                B, tuple(m.shape), m.dtype))
+        return (m.to(self.device, non_blocking=True) != 0).expand(B, 64, 64).contiguous()
 
     # ---- importance-weighted log-likelihood (an extension: the reference scores a model by accuracy only) ------------
     def log_likelihood(self, x, y=None, k=100, c=None, noise=None, max_rows=8192, keep_log_w=False):
