@@ -271,10 +271,14 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
     const int q = warp & 3;
     const int m = q * 32 + lane;
     const int dx = m % p.BW, dy = (m / p.BW) % p.BH, dn = m / (p.BW * p.BH);
-    // bias -> shared memory once per CTA (a global load per item would sit on the epilogue's critical path)
+    // bias -> shared memory once per CTA (a global load per item would sit on the epilogue's critical path), repeated
+    // with period bias_mod: a slab wider than bias_mod (bias_mod dividing 256) then reads it without a modulo
     {
       const int nb = p.bias == nullptr ? 0 : (p.bias_mod < p.bias_n ? p.bias_mod : p.bias_n);
-      for (int i = threadIdx.x - 64; i < 256; i += 128) s_bias[i] = i < nb ? p.bias[i] : 0.0f;
+      for (int i = threadIdx.x - 64; i < 256; i += 128) {
+        const int j = i % p.bias_mod;
+        s_bias[i] = j < nb ? p.bias[j] : 0.0f;
+      }
       asm volatile("bar.sync 1, 128;" ::: "memory");
     }
     for (int item = item_beg; item < item_end; ++item) {
@@ -304,13 +308,14 @@ __global__ void __launch_bounds__(TG_THREADS) tapgemm_kernel(const __grid_consta
       mbar_wait(&tfull[as], (uint32_t)(li >> 1) & 1u);
       tc_fence_after();
       if (threadIdx.x == 64) TL(li, 4);
-      // bias index of this slab's first channel: host guarantees bias_mod % N == 0 or bias_mod >= n_store,
-      // so no per-element modulo is needed
+      // bias index of this slab's first channel: host guarantees bias_mod % N == 0, 256 % bias_mod == 0 or
+      // bias_mod >= n_store, so no per-element modulo is needed
       const int bias_base = slab0 % p.bias_mod;
       const uint32_t s_bias_u32 = smem_u32(s_bias);
       for (int c0 = 0; c0 < p.N; c0 += 16) {
         const int cg = slab0 + c0;  // global output channel of this chunk
-        // bias_base + c0 + i < 256 always: bias_mod <= 256 wraps it, otherwise n_store <= 256
+        // (bias_base + c0 + i) & 255 is the bias index: bias_mod <= 256 divides 256 or the slab stays below bias_mod,
+        // otherwise n_store <= 256
         const uint32_t bsrc = s_bias_u32 + (uint32_t)(((bias_base + c0) & 255) * 4);
         uint32_t r[16];
         tmem_ld16(tacc + (uint32_t)c0, r);
@@ -1979,8 +1984,8 @@ static int launch_tapgemm(TapGemmParams& p, int groups, int phases, cudaStream_t
   if (p.n_slabs < 1) p.n_slabs = 1;
   if (p.bias_mod < 1 || p.bias == nullptr) p.bias_mod = 1 << 30;
   if (p.bias_n < 1) p.bias_n = p.n_store;
-  GCC_REQUIRE(p.bias_mod >= p.n_store || p.bias_mod % p.N == 0, "%s: bias_mod %d incompatible with N slab %d", name,
-              p.bias_mod, p.N);
+  GCC_REQUIRE(p.bias_mod >= p.n_store || p.bias_mod % p.N == 0 || 256 % p.bias_mod == 0,
+              "%s: bias_mod %d incompatible with N slab %d", name, p.bias_mod, p.N);
   GCC_REQUIRE(p.bias == nullptr || ((uintptr_t)p.bias % 16) == 0, "%s: bias must be 16-byte aligned", name);
   p.phases = phases;
   p.total_items = groups * p.tiles_w * p.tiles_h * p.n_slabs * phases;

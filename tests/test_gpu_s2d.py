@@ -7,6 +7,7 @@ import pytest
 import torch
 
 import gccvae_oracle as O
+from launch_reference import s2d_blocks
 
 pytestmark = pytest.mark.gpu
 
@@ -22,14 +23,6 @@ def _stream():
 
 def bf(t):
     return t.to(torch.bfloat16).to(torch.float32)
-
-
-def s2d_blocks(t):
-    """[B,H,W,C] -> [B,H/2+1,W/2+1,4C]: block (i,j) slot dy*2+dx = pixel (2i-1+dy, 2j-1+dx), zero outside."""
-    B, H, W, Cc = t.shape
-    pad = torch.zeros(B, H + 2, W + 2, Cc, dtype=t.dtype)
-    pad[:, 1:H + 1, 1:W + 1] = t
-    return pad.view(B, H // 2 + 1, 2, W // 2 + 1, 2, Cc).permute(0, 1, 3, 2, 4, 5).reshape(B, H // 2 + 1, W // 2 + 1, 4 * Cc)
 
 
 def pack9(lib, L, W, CL, CS):

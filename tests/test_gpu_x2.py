@@ -9,6 +9,7 @@ import pytest
 import torch
 
 import gccvae_oracle as O
+from launch_reference import _raw_byte_blocks, x2_blocks
 
 pytestmark = pytest.mark.gpu
 
@@ -24,20 +25,6 @@ def _stream():
 
 def bf(t):
     return t.to(torch.bfloat16).to(torch.float32)
-
-
-def x2_blocks(img, ones=False):
-    """[B,64,64,3] -> [B,33,33,16] with X2[n,i,j,(dy,dx,c4)] = img[n,2i-1+dy,2j-1+dx,c] (zero outside / pad).
-    ones=True: as gccvae_prep_x2_bf16 writes the blocks - element 15 (pad channel of the last pixel slot) is 1.0, the
-    constant row that turns conv1's weight gradient into its bias gradient as well."""
-    B = img.shape[0]
-    pad = torch.zeros(B, 66, 66, 4, dtype=img.dtype)
-    pad[:, 1:65, 1:65, :3] = img
-    blk = pad.view(B, 33, 2, 33, 2, 4).permute(0, 1, 3, 2, 4, 5).reshape(B, 33, 33, 16)
-    if ones:
-        blk = blk.clone()
-        blk[..., 15] = 1
-    return blk
 
 
 def pack(lib, L, kind, W, n_out):
@@ -81,19 +68,6 @@ def test_prep_x2(u8):
             assert torch.equal(X2.cpu().view(torch.int16), want.view(torch.int16))
     else:
         assert lib.gccvae_prep_x2_bf16(L.ptr(xin), 0, B, L.ptr(X2), L.ptr(X2), _stream()) != 0   # fp32 images have no raw bytes
-
-
-def _raw_byte_blocks(xi):
-    """[B,64,64,3] uint8 -> [B,33,33,16] uint8: block (i, j) = pixels (2i-1+dy, 2j-1+dx) x 3 channels, 4 zero bytes."""
-    B = xi.shape[0]
-    pad = torch.zeros(B, 66, 66, 3, dtype=torch.uint8)
-    pad[:, 1:65, 1:65] = xi
-    out = torch.zeros(B, 33, 33, 16, dtype=torch.uint8)
-    for dy in range(2):
-        for dx in range(2):
-            q = dy * 2 + dx
-            out[..., 3 * q:3 * q + 3] = pad[:, dy:dy + 65:2, dx:dx + 65:2][:, :33, :33]
-    return out
 
 
 def test_u8_normalisation_is_bit_exact_for_all_256_values():
